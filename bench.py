@@ -2,7 +2,7 @@
 """bench.py -- RNA-MSM MSA-transformer forward throughput on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload cfg2|cfg1|cfg4|cfg5] [--precision fp16|bf16|fp32]
+                    [--workload cfg2|cfg1|cfg4|cfg5] [--precision fp16|bf16|fp32] [--dump-outputs DIR]
 
 A "step" is one full forward of the hot path over one synthetic MSA: int64 token grid ->
 emb (L,768) + 120 tied-row attention maps, with random-init weights of the real architecture
@@ -21,6 +21,9 @@ Printed JSON (rank 0, one line):
   cpu_baseline the oracle (port of the reference's fp32 CPU forward) timed on this box's cores on
                a bounded sample: ONE of the 10 AxialTransformerLayers at the full shape, x10
   --impl reference : the CPU arm alone, same metric/config, one sample per step.
+
+--dump-outputs DIR writes what the last device-timed step returned (see dump_outputs) as DIR/<name>.npy.  Weights
+(torch seed 42) and tokens (seeded per rank) are the same in every run, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -308,6 +311,28 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, out):
+    """Write the arrays ``MSATransformer.forward`` returned to its caller as float32 ``out_dir/<name>.npy``:
+    ``row_attentions`` [1, layers, heads, C, C] and ``representations_<layers>`` [1, R, C, D].  Each array gets half of
+    DUMP_BYTES; a larger one is cut to a fixed, seeded sample of its query positions (maps) or MSA rows
+    (representations), always including index 0 and kept in ascending order."""
+    import numpy as np
+    import torch
+    arrays = {"row_attentions": (out["row_attentions"], 3), f"representations_{NL}": (out["representations"][NL], 1)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (t, axis) in arrays.items():
+        n = t.shape[axis]
+        keep = max(1, (DUMP_BYTES // len(arrays) - 1024) // (t.numel() // n * 4))    # 1 KB: room for the .npy header
+        if keep < n:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.cat([torch.zeros(1, dtype=torch.int64), 1 + torch.randperm(n - 1, generator=g)[:keep - 1]])
+            t = t.index_select(axis, idx.sort().values.to(t.device))
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def _rel_err(a, b):
     """max|a - b| / max|b| (the norm-relative gate of SURVEY.md 8d)."""
     return float((a.double() - b.double()).abs().max() / b.double().abs().max().clamp_min(1e-30))
@@ -680,11 +705,15 @@ def run_ours(args):
     barrier()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
-    for _ in range(args.steps):
+    for _ in range(args.steps - 1):
         step_device()
+    last = step_device()
     ev1.record()
     barrier()
     ms_total = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     launches = _lib.lib.rnamsm_launch_count() - launches0
     # per-kernel-class CUDA events over a second, identical region of K steps: two event records around each of the
     # ~132 launches per forward cost ~0.5 ms, which would be charged to `value` if they sat in the region above
@@ -820,7 +849,14 @@ def main():
     ap.add_argument("--fused", action="store_true",
                     help="with --shard: the peer-memory schedule (softmax pulling/pushing logits over NVLink, LayerNorm "
                          "pushing rows to the column owners, out-projection reducing into the row owners' residual)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all; "
+                         "single-MSA workloads, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "cfg3" or args.shard):
+        ap.error("--dump-outputs needs --impl ours, a single-MSA workload (not cfg3) and no --shard")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -59,12 +59,9 @@ def test_read_msa_cleaning_rules(pkg, tmp_path):
     assert np.array_equal(v.encode(seqs[:1]), otok.numpy())
 
 
-def test_tokenize_matches_golden_2drb(pkg, golden_dir):
-    ref = "/root/reference/results/2DRB_1.a2m_msa2"
-    if not os.path.exists(ref):
-        pytest.skip("reference checkout not present")
+def test_tokenize_matches_golden_2drb(pkg, golden_dir, msa_2drb_file):
     v = pkg.Vocab(pkg.Alphabet())
-    tok = pkg.tokenize_msa(ref, v, 512, 1024)
+    tok = pkg.tokenize_msa(msa_2drb_file, v, 512, 1024)
     g = np.load(os.path.join(golden_dir, "2DRB_1.npz"))
     assert np.array_equal(tok.numpy(), g["tokens"][0].astype(np.int64))
 
@@ -104,17 +101,19 @@ def test_extract_features_format(pkg):
     assert np.array_equal(o_emb, emb) and np.array_equal(o_atp, atp)
 
 
-def test_shipped_fixture_format():
-    """Format pin against the reference's shipped outputs (values need the unpublished checkpoint)."""
-    p = "/root/reference/results/2DRB_1_atp.npy"
-    if not os.path.exists(p):
-        pytest.skip("reference checkout not present")
-    atp = np.load(p)
-    emb = np.load("/root/reference/results/2DRB_1_emb.npy")
-    assert atp.shape == (120, 35, 35) and atp.dtype == np.float32
-    assert emb.shape == (35, 768) and emb.dtype == np.float32
-    ss = np.load("/root/reference/_downstream_tasks/SS/inputs/attention_map/6XJQ_A.npy")
-    assert ss.shape == (120, 58, 58) and ss.dtype == np.float32
+def test_shipped_fixture_format(pkg, golden_dir):
+    """Format pin against the reference's shipped outputs results/2DRB_1_{atp,emb}.npy (values need the unpublished
+    checkpoint): their shapes are stored in tests/golden/2DRB_1.npz, and extract_features on forward outputs shaped
+    for the 512 x 36 token grid must produce arrays of those shapes in float32."""
+    g = np.load(os.path.join(golden_dir, "2DRB_1.npz"))
+    atp_shape, emb_shape = tuple(g["shipped_atp_shape"]), tuple(g["shipped_emb_shape"])
+    assert atp_shape == (120, 35, 35) and emb_shape == (35, 768)
+    assert g["atp"].dtype == g["emb"].dtype == np.float32
+    R, Cc = g["tokens"].shape[1:]
+    out = {"row_attentions": torch.rand(1, 10, 12, Cc, Cc), "representations": {10: torch.randn(1, R, Cc, 768)}}
+    emb, atp = pkg.extract_features(out, pkg.Vocab(pkg.Alphabet()), 10)
+    assert atp.shape == atp_shape and atp.dtype == np.float32
+    assert emb.shape == emb_shape and emb.dtype == np.float32
 
 
 def test_plan_batches_covers_every_msa_once_within_budget():
