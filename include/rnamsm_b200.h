@@ -177,6 +177,16 @@ int rnamsm_row_attn_av(const void* probs, int ldp, const void* qkv, int R, int C
 int rnamsm_col_attn(const void* qkv, int R, int C, int H, int dtype, int qkv_col_major, const uint8_t* pad, void* ctx,
                     void* stream);
 
+/* Column-attention probabilities of K7 on request (the reference's [H, C, B, R, R] for one MSA, modules.py:907-918):
+ * from the same q|k and pad as rnamsm_col_attn (either q|k layout; the column-major one in the 16-bit path only),
+ *   probs_out fp32 [H, C, R, R]: P[h,c,i,j] = softmax_j(q[i,c,h,:].k[j,c,h,:]), logit -10000 where pad[j*C+c] != 0;
+ *   mean_out  fp32 [H, R, R]:    (1/C) sum_c P[h,c,i,j] over every column, computed without the full tensor.
+ * Either output may be NULL.  R == 1 gives all ones (modules.py:882-894; q|k and scratch are not read).
+ * scratch: rnamsm_col_probs_scratch_bytes(R, C, H) device bytes (per-row max and log-sum).  dtype RNAMSM_F32 runs FFMA
+ * kernels (expf), the 16-bit dtypes tcgen05 (ex2.approx).  Deterministic: no atomics, columns summed in order. */
+int rnamsm_col_attn_probs(const void* qkv, int R, int C, int H, int dtype, int qkv_col_major, const uint8_t* pad,
+                          float* probs_out, float* mean_out, void* scratch, void* stream);
+
 /* K9b -- tied LM-head projection logits[m, v] = h[m,:] . E[v,:] + bias[v] (modules.py:318), fp32. */
 int rnamsm_vocab_proj(const float* h, const float* E, const float* bias, long long M, int V, int D, float* out,
                       void* stream);
@@ -270,6 +280,9 @@ typedef struct rnamsm_model_weights {
 
 /* Bytes of scratch rnamsm_layer_forward / rnamsm_msa_forward need for an R x C MSA. */
 size_t rnamsm_workspace_bytes(int R, int C, int D, int H, int F, int dtype);
+/* Scratch of rnamsm_col_attn_probs, and what rnamsm_layer_forward_col_probs / rnamsm_msa_forward_col_probs need on top
+ * of their usual workspace when they export column probabilities: two fp32 [H, C, R], 256 B aligned; 0 for an empty shape. */
+size_t rnamsm_col_probs_scratch_bytes(int R, int C, int H);
 
 /* Range diagnostics for the 16-bit path.  rnamsm_range_scan: counters[0] += number of elements of buf (16-bit, n
  * elements) that are non-finite or sit at the largest finite value of the type (where the kernels' cvt.rn.satfinite
@@ -295,6 +308,14 @@ int rnamsm_layer_forward(const rnamsm_layer_weights* w, int D, int H, int F, flo
                          const uint8_t* pad, int dtype, float* row_probs_out, void* workspace,
                          size_t workspace_bytes, int xn_ready, const float* next_ln_w, const float* next_ln_b,
                          int next_ln_dtype, void* stream);
+/* rnamsm_layer_forward that also exports the column attention's probabilities: col_probs_out fp32 [H, C, R, R] and / or
+ * col_mean_out fp32 [H, R, R] (as rnamsm_col_attn_probs; NULL = not wanted).  With either set, workspace_bytes must
+ * cover rnamsm_workspace_bytes(...) + rnamsm_col_probs_scratch_bytes(R, C, H).  Both NULL: same launches, same
+ * results as rnamsm_layer_forward. */
+int rnamsm_layer_forward_col_probs(const rnamsm_layer_weights* w, int D, int H, int F, float ln_eps, float* x, int R, int C,
+                                   const uint8_t* pad, int dtype, float* row_probs_out, float* col_probs_out,
+                                   float* col_mean_out, void* workspace, size_t workspace_bytes, int xn_ready,
+                                   const float* next_ln_w, const float* next_ln_b, int next_ln_dtype, void* stream);
 
 /* MSATransformer.forward (model.py:338-416) for one MSA.
  *   tokens [R,C] int64 -> x (caller-provided fp32 [R*C, D] buffer; holds the final
@@ -306,6 +327,14 @@ int rnamsm_layer_forward(const rnamsm_layer_weights* w, int D, int H, int F, flo
 int rnamsm_msa_forward(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad, int dtype,
                        float* x, float* row_attn_out, float* const* rep_out, float* logits_out, void* workspace,
                        size_t workspace_bytes, void* stream);
+/* rnamsm_msa_forward that also exports every layer's column-attention probabilities: col_probs_out fp32
+ * [N, H, C, R, R] and / or col_mean_out fp32 [N, H, R, R] (NULL = not wanted).  With either set, workspace_bytes must
+ * cover what rnamsm_msa_forward needs plus rnamsm_col_probs_scratch_bytes(R, C, H).  Both NULL: same launches, same
+ * results as rnamsm_msa_forward. */
+int rnamsm_msa_forward_col_probs(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad,
+                                 int dtype, float* x, float* row_attn_out, float* col_probs_out, float* col_mean_out,
+                                 float* const* rep_out, float* logits_out, void* workspace, size_t workspace_bytes,
+                                 void* stream);
 
 /* Several short MSAs in one pass (SURVEY.md 8f row 4).  tokens: the int64 grids back to back
  * ([R[0]*C[0]] then [R[1]*C[1]] ...); R, C, has_pad: HOST arrays of n_msa entries (has_pad may be NULL);

@@ -63,6 +63,8 @@ SIGNATURES = {
     "rnamsm_row_softmax": (_i, [_vp, _i, _i, _i, _vp, _f, _vp, _vp, _i, _i, _vp]),
     "rnamsm_row_attn_av": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp]),
     "rnamsm_col_attn": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "rnamsm_col_attn_probs": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "rnamsm_col_probs_scratch_bytes": (_sz, [_i, _i, _i]),
     "rnamsm_vocab_proj": (_i, [_vp, _vp, _vp, _ll, _i, _i, _vp, _vp]),
     "rnamsm_msa_clean": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp]),
     "rnamsm_msa_greedy_workspace": (_sz, [_i, _i]),
@@ -76,6 +78,8 @@ SIGNATURES = {
     "rnamsm_debug_range_watch": (_i, [_vp]),
     "rnamsm_layer_forward": (_i, [C.POINTER(LayerWeights), _i, _i, _i, _f, _vp, _i, _i, _vp, _i, _vp, _vp, _sz,
                                   _i, _vp, _vp, _i, _vp]),
+    "rnamsm_layer_forward_col_probs": (_i, [C.POINTER(LayerWeights), _i, _i, _i, _f, _vp, _i, _i, _vp, _i, _vp, _vp, _vp,
+                                            _vp, _sz, _i, _vp, _vp, _i, _vp]),
     "rnamsm_peer_alloc": (_i, [_sz, C.POINTER(_vp)]),
     "rnamsm_peer_free": (_i, [_vp]),
     "rnamsm_ipc_export": (_i, [_vp, _vp]),
@@ -91,6 +95,8 @@ SIGNATURES = {
     "rnamsm_add_layernorm": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _i, _ll, _i, _f, _vp]),
     "rnamsm_msa_forward": (_i, [C.POINTER(ModelWeights), _vp, _i, _i, _i, _i, _vp, _vp, C.POINTER(_vp), _vp, _vp,
                                 _sz, _vp]),
+    "rnamsm_msa_forward_col_probs": (_i, [C.POINTER(ModelWeights), _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp,
+                                          C.POINTER(_vp), _vp, _vp, _sz, _vp]),
     "rnamsm_batch_workspace_bytes": (_sz, [_i, C.POINTER(_i), C.POINTER(_i), _i, _i, _i, _i]),
     "rnamsm_msa_forward_batch": (_i, [C.POINTER(ModelWeights), _i, _vp, C.POINTER(_i), C.POINTER(_i), C.c_char_p, _i, _vp,
                                       C.POINTER(_vp), _vp, _sz, _vp]),

@@ -231,10 +231,15 @@ static int range_watch(const void* p, long long n, int dtype, cudaStream_t st) {
 // LayerNorm of the NEXT layer's row block, produced by this layer's fc2 epilogue (16-bit path)
 struct NextLn { const float* w; const float* b; int dtype; };
 
+// Column-attention probabilities a caller asked for (col_attn_probs.cu): P [H, C, R, R] and / or the column mean
+// [H, R, R] (either NULL), lse: col_probs_scratch_bytes(R, C, H) bytes of scratch.
+struct ColProbsOut { float* probs; float* mean; void* lse; };
+
 // xn_ready: the workspace's xn region already holds LayerNorm_row(x) (written by the previous layer's fc2 epilogue).
 static int layer_forward(const rnamsm_layer_weights* w, int D, int H, int F, float eps, float* x, int R, int C,
                          const uint8_t* pad, int dtype, float* row_probs_out, uint8_t* ws, const Plan& p,
-                         cudaStream_t st, bool xn_ready = false, const NextLn* next = nullptr, bool f32_tensor = false) {
+                         cudaStream_t st, bool xn_ready = false, const NextLn* next = nullptr, bool f32_tensor = false,
+                         const ColProbsOut* colp = nullptr) {
   const long long T = (long long)R * C;
   void* xn = ws + p.off_xn;
   uint8_t* qkv = ws + p.off_qkvh;
@@ -316,6 +321,9 @@ static int layer_forward(const rnamsm_layer_weights* w, int D, int H, int F, flo
       if ((rc = launch_col_attn_f32((const float*)qkv, R, C, H, pad, (float*)ctx, st))) return rc;
     }
   }
+  // q|k of the column block are still in place (the flash kernel wrote ctx next to them)
+  if (colp && (rc = launch_col_probs(qkv, R, C, H, col_dt, col_major, pad, colp->probs, colp->mean, colp->lse, st)))
+    return rc;
   {
     LinearEpilogue e{RNAMSM_EPI_BIAS_RESIDUAL, w->col.b_out, 1.f, 0, nullptr};
     const LnFuse ln{w->ffn_ln_w, w->ffn_ln_b, eps, xn, dtype == RNAMSM_F16, 0, 0, cnt};
@@ -617,6 +625,11 @@ int rnamsm_col_attn(const void* qkv, int R, int C, int H, int dtype, int qkv_col
   return launch_col_attn_f32((const float*)qkv, R, C, H, pad, (float*)ctx, (cudaStream_t)stream);
 }
 
+int rnamsm_col_attn_probs(const void* qkv, int R, int C, int H, int dtype, int qkv_col_major, const uint8_t* pad,
+                          float* probs_out, float* mean_out, void* scratch, void* stream) {
+  return launch_col_probs(qkv, R, C, H, dtype, qkv_col_major, pad, probs_out, mean_out, scratch, (cudaStream_t)stream);
+}
+
 int rnamsm_vocab_proj(const float* h, const float* E, const float* bias, long long M, int V, int D, float* out,
                       void* stream) {
   return launch_vocab_proj(h, E, bias, M, V, D, out, (cudaStream_t)stream);
@@ -626,6 +639,8 @@ size_t rnamsm_workspace_bytes(int R, int C, int D, int H, int F, int dtype) {
   if (R <= 0 || C <= 0) return 0;
   return make_plan(R, C, D, H, F, dtype & 0xff, (dtype & RNAMSM_F32_TENSOR) != 0).total;
 }
+
+size_t rnamsm_col_probs_scratch_bytes(int R, int C, int H) { return col_probs_scratch_bytes(R, C, H); }
 
 int rnamsm_range_scan(const void* buf, long long n, int dtype, unsigned long long* counters, void* stream) {
   RNAMSM_REQUIRE(counters != nullptr, "range_scan: counters required");
@@ -638,25 +653,35 @@ int rnamsm_debug_range_watch(unsigned long long* counters) {
 
 int rnamsm_fused_layernorm(int dtype) { return (is16(dtype) && fuse_ln_enabled()) ? 1 : 0; }
 
-int rnamsm_layer_forward(const rnamsm_layer_weights* w, int D, int H, int F, float ln_eps, float* x, int R, int C,
-                         const uint8_t* pad, int dtype, float* row_probs_out, void* workspace, size_t workspace_bytes,
-                         int xn_ready, const float* next_ln_w, const float* next_ln_b, int next_ln_dtype, void* stream) {
+}  // extern "C"
+
+// col_probs_out / col_mean_out both NULL: exactly the launch sequence of rnamsm_layer_forward.  Otherwise the column
+// probabilities' scratch sits right after the layer's own workspace.
+static int layer_forward_entry(const rnamsm_layer_weights* w, int D, int H, int F, float ln_eps, float* x, int R, int C,
+                               const uint8_t* pad, int dtype, float* row_probs_out, float* col_probs_out,
+                               float* col_mean_out, void* workspace, size_t workspace_bytes, int xn_ready,
+                               const float* next_ln_w, const float* next_ln_b, int next_ln_dtype, void* stream) {
   RNAMSM_REQUIRE(D == H * 64, "layer_forward: head_dim must be 64 (D=%d H=%d)", D, H);
   const bool f32_tensor = (dtype & RNAMSM_F32_TENSOR) != 0;
   dtype &= 0xff;
   RNAMSM_REQUIRE(dtype == RNAMSM_F32 || (is16(dtype) && !f32_tensor), "layer_forward: unknown dtype %d", dtype);
   const Plan p = make_plan(R, C, D, H, F, dtype, f32_tensor);
-  RNAMSM_REQUIRE(workspace_bytes >= p.total, "layer_forward: workspace %zu < required %zu", workspace_bytes, p.total);
+  const bool want_col = col_probs_out || col_mean_out;
+  const size_t need = p.total + (want_col ? col_probs_scratch_bytes(R, C, H) : 0);
+  RNAMSM_REQUIRE(workspace_bytes >= need, "layer_forward: workspace %zu < required %zu", workspace_bytes, need);
   RNAMSM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "layer_forward: workspace must be 256 B aligned");
   RNAMSM_REQUIRE((next_ln_w == nullptr) == (next_ln_b == nullptr), "layer_forward: next_ln_w and next_ln_b go together");
   const NextLn next{next_ln_w, next_ln_b, block_dtype(next_ln_dtype, dtype)};
+  const ColProbsOut colp{col_probs_out, col_mean_out, (uint8_t*)workspace + p.total};
   return layer_forward(w, D, H, F, ln_eps, x, R, C, pad, dtype, row_probs_out, (uint8_t*)workspace, p,
-                       (cudaStream_t)stream, xn_ready != 0, next_ln_w ? &next : nullptr, f32_tensor);
+                       (cudaStream_t)stream, xn_ready != 0, next_ln_w ? &next : nullptr, f32_tensor,
+                       want_col ? &colp : nullptr);
 }
 
-int rnamsm_msa_forward(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad, int dtype,
-                       float* x, float* row_attn_out, float* const* rep_out, float* logits_out, void* workspace,
-                       size_t workspace_bytes, void* stream) {
+static int msa_forward_entry(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad, int dtype,
+                             float* x, float* row_attn_out, float* col_probs_out, float* col_mean_out,
+                             float* const* rep_out, float* logits_out, void* workspace, size_t workspace_bytes,
+                             void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   const int D = m->embed_dim, H = m->num_heads, F = m->ffn_dim, N = m->num_layers;
   RNAMSM_REQUIRE(D == H * 64, "msa_forward: head_dim must be 64 (D=%d H=%d)", D, H);
@@ -667,8 +692,9 @@ int rnamsm_msa_forward(const rnamsm_model_weights* m, const int64_t* tokens, int
   const Plan p = make_plan(R, C, D, H, F, dtype, f32_tensor);
   const size_t T = (size_t)R * C;
   const size_t pad_bytes = (T + 255) & ~(size_t)255;
-  RNAMSM_REQUIRE(workspace_bytes >= p.total + pad_bytes, "msa_forward: workspace %zu < required %zu", workspace_bytes,
-                 p.total + pad_bytes);
+  const bool want_col = col_probs_out || col_mean_out;
+  const size_t need = p.total + pad_bytes + (want_col ? col_probs_scratch_bytes(R, C, H) : 0);
+  RNAMSM_REQUIRE(workspace_bytes >= need, "msa_forward: workspace %zu < required %zu", workspace_bytes, need);
   RNAMSM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "msa_forward: workspace must be 256 B aligned");
   uint8_t* ws = (uint8_t*)workspace;
   uint8_t* pad = ws + p.total;
@@ -680,13 +706,15 @@ int rnamsm_msa_forward(const rnamsm_model_weights* m, const int64_t* tokens, int
   for (int l = 0; l < N; ++l) {
     if (rep_out && rep_out[l]) RNAMSM_CHECK_CUDA(cudaMemcpyAsync(rep_out[l], x, T * D * 4, cudaMemcpyDeviceToDevice, st));
     float* map = row_attn_out ? row_attn_out + (size_t)l * H * C * C : nullptr;
+    const ColProbsOut colp{col_probs_out ? col_probs_out + (size_t)l * H * C * R * R : nullptr,
+                           col_mean_out ? col_mean_out + (size_t)l * H * R * R : nullptr, pad + pad_bytes};
     // layer l's fc2 epilogue also writes layer l+1's row-block LayerNorm (16-bit path)
     const bool fuse = is16(dtype) && fuse_ln_enabled();
     NextLn next{nullptr, nullptr, dtype};
     if (fuse && l + 1 < N)
       next = NextLn{m->layers[l + 1].row.ln_w, m->layers[l + 1].row.ln_b, block_dtype(m->layers[l + 1].row.dtype, dtype)};
     if ((rc = layer_forward(&m->layers[l], D, H, F, m->ln_eps, x, R, C, pad_arg, dtype, map, ws, p, st, fuse && l > 0,
-                            next.w ? &next : nullptr, f32_tensor)))
+                            next.w ? &next : nullptr, f32_tensor, want_col ? &colp : nullptr)))
       return rc;
   }
   // 16-bit path with logits wanted: the LM head's dense GEMM runs on the tensor cores, so it needs the final
@@ -719,6 +747,38 @@ int rnamsm_msa_forward(const rnamsm_model_weights* m, const int64_t* tokens, int
     if ((rc = launch_vocab_proj(h32, m->tok_emb, m->lm_bias, (long long)T, m->vocab, D, logits_out, st))) return rc;
   }
   return 0;
+}
+
+extern "C" {
+
+int rnamsm_layer_forward(const rnamsm_layer_weights* w, int D, int H, int F, float ln_eps, float* x, int R, int C,
+                         const uint8_t* pad, int dtype, float* row_probs_out, void* workspace, size_t workspace_bytes,
+                         int xn_ready, const float* next_ln_w, const float* next_ln_b, int next_ln_dtype, void* stream) {
+  return layer_forward_entry(w, D, H, F, ln_eps, x, R, C, pad, dtype, row_probs_out, nullptr, nullptr, workspace,
+                             workspace_bytes, xn_ready, next_ln_w, next_ln_b, next_ln_dtype, stream);
+}
+
+int rnamsm_layer_forward_col_probs(const rnamsm_layer_weights* w, int D, int H, int F, float ln_eps, float* x, int R, int C,
+                                   const uint8_t* pad, int dtype, float* row_probs_out, float* col_probs_out,
+                                   float* col_mean_out, void* workspace, size_t workspace_bytes, int xn_ready,
+                                   const float* next_ln_w, const float* next_ln_b, int next_ln_dtype, void* stream) {
+  return layer_forward_entry(w, D, H, F, ln_eps, x, R, C, pad, dtype, row_probs_out, col_probs_out, col_mean_out,
+                             workspace, workspace_bytes, xn_ready, next_ln_w, next_ln_b, next_ln_dtype, stream);
+}
+
+int rnamsm_msa_forward(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad, int dtype,
+                       float* x, float* row_attn_out, float* const* rep_out, float* logits_out, void* workspace,
+                       size_t workspace_bytes, void* stream) {
+  return msa_forward_entry(m, tokens, R, C, has_pad, dtype, x, row_attn_out, nullptr, nullptr, rep_out, logits_out,
+                           workspace, workspace_bytes, stream);
+}
+
+int rnamsm_msa_forward_col_probs(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad,
+                                 int dtype, float* x, float* row_attn_out, float* col_probs_out, float* col_mean_out,
+                                 float* const* rep_out, float* logits_out, void* workspace, size_t workspace_bytes,
+                                 void* stream) {
+  return msa_forward_entry(m, tokens, R, C, has_pad, dtype, x, row_attn_out, col_probs_out, col_mean_out, rep_out,
+                           logits_out, workspace, workspace_bytes, stream);
 }
 
 size_t rnamsm_batch_workspace_bytes(int n_msa, const int* R, const int* C, int D, int H, int F, int dtype) {

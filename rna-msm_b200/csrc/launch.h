@@ -104,4 +104,10 @@ int launch_row_attn_short_16(const void* qkv, int R, int C, int H, int fp16, flo
 int launch_col_attn_16(const void* qkv, int R, int C, int H, int fp16, int col_major, const uint8_t* pad, void* ctx,
                        cudaStream_t st);
 
+// col_attn_probs.cu -- column-attention probabilities P [H, C, R, R] and / or their column mean [H, R, R] (either may
+// be NULL); dtype RNAMSM_F32 / BF16 / F16; scratch: col_probs_scratch_bytes(R, C, H) bytes (per-row max and log-sum)
+size_t col_probs_scratch_bytes(int R, int C, int H);
+int launch_col_probs(const void* qkv, int R, int C, int H, int dtype, int col_major, const uint8_t* pad, float* probs,
+                     float* mean, void* scratch, cudaStream_t st);
+
 }  // namespace rnamsm

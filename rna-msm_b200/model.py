@@ -198,9 +198,16 @@ class MSATransformer(nn.Module, _PrecisionMixin):
     # -- forward -------------------------------------------------------------------------------
     @torch.no_grad()
     def forward(self, tokens, repr_layers: Iterable[int] = (), need_head_weights: bool = False,
-                return_contacts: bool = False, want_logits: bool = True) -> Dict[str, object]:
+                return_contacts: bool = False, want_logits: bool = True, need_col_weights: bool = False,
+                need_col_weights_mean: bool = False) -> Dict[str, object]:
         """model.py:338-416.  ``want_logits=False`` (extension) skips the LM head, which the
-        inference script never reads."""
+        inference script never reads.
+
+        Column-attention probabilities (extensions, off by default; either works with or without
+        ``need_head_weights``): ``need_col_weights`` adds ``col_attentions`` ``[B, N, H, C, R, R]`` fp32
+        (the key and layout of the reference's ``msm/`` model); ``need_col_weights_mean`` adds
+        ``col_attentions_mean`` ``[B, N, H, R, R]``, their mean over the C columns, computed without
+        the full tensor (which outgrows the GPU at R x C = 1024 x 1024)."""
         if return_contacts:
             need_head_weights = True
         _infer_only(self)
@@ -219,16 +226,30 @@ class MSATransformer(nn.Module, _PrecisionMixin):
         x = torch.empty((B, R, Cc, D), dtype=torch.float32, device=dev)
         row_att = torch.empty((B, N, H, Cc, Cc), dtype=torch.float32, device=dev) if need_head_weights else None
         logits = torch.empty((B, R, Cc, len(self.vocab)), dtype=torch.float32, device=dev) if want_logits else None
+        # allocated before the first launch, so a size that does not fit fails before any kernel runs
+        col_att = torch.empty((B, N, H, Cc, R, R), dtype=torch.float32, device=dev) if need_col_weights else None
+        col_mean = torch.empty((B, N, H, R, R), dtype=torch.float32, device=dev) if need_col_weights_mean else None
+        want_col = need_col_weights or need_col_weights_mean
         reps: Dict[int, torch.Tensor] = {
             l: torch.empty((B, R, Cc, D), dtype=torch.float32, device=dev) for l in sorted(repr_layers) if 0 <= l < N}
         with torch.cuda.device(dev):
             m = self.c_weights(code)
             fcode = self._fwd_code
             nbytes = L.lib.rnamsm_workspace_bytes(R, Cc, D, H, 4 * D, fcode) + ((R * Cc + 255) // 256) * 256
+            if want_col:
+                nbytes += L.lib.rnamsm_col_probs_scratch_bytes(R, Cc, H)
             ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
             st = L.stream_ptr()
             for b in range(B):
                 rep_ptrs = (C.c_void_p * (N + 1))(*[reps[l][b].data_ptr() if l in reps else None for l in range(N + 1)])
+                if want_col:
+                    L.check(L.lib.rnamsm_msa_forward_col_probs(
+                        C.byref(m), L.ptr(tokens[b]), R, Cc, int(has_pad), fcode, L.ptr(x[b]),
+                        L.ptr(row_att[b]) if row_att is not None else None,
+                        L.ptr(col_att[b]) if col_att is not None else None,
+                        L.ptr(col_mean[b]) if col_mean is not None else None, rep_ptrs,
+                        L.ptr(logits[b]) if logits is not None else None, L.ptr(ws), nbytes, st), "msa_forward_col_probs")
+                    continue
                 L.check(L.lib.rnamsm_msa_forward(
                     C.byref(m), L.ptr(tokens[b]), R, Cc, int(has_pad), fcode, L.ptr(x[b]),
                     L.ptr(row_att[b]) if row_att is not None else None, rep_ptrs,
@@ -240,6 +261,10 @@ class MSATransformer(nn.Module, _PrecisionMixin):
             result["row_attentions"] = row_att                             # B x N x H x C x C
             if return_contacts:
                 result["contacts"] = self.contact_head(tokens, row_att)
+        if need_col_weights:
+            result["col_attentions"] = col_att                             # B x N x H x C x R x R
+        if need_col_weights_mean:
+            result["col_attentions_mean"] = col_mean                       # B x N x H x R x R
         return result
 
     @torch.no_grad()

@@ -181,13 +181,14 @@ class RowSelfAttention(_AxialAttentionBase):
 class ColumnSelfAttention(_AxialAttentionBase):
     """Column attention over the MSA depth (modules.py:824-945): K3 -> K7 (flash) -> out_proj.
 
-    Deliberate deviation: the reference returns the ``[H, C, B, R, R]`` probabilities; the fused
-    kernel never materialises them and the shipped model discards them (model.py:406-410), so the
-    second return value is ``None`` (except R == 1, where the reference's all-ones tensor is cheap).
+    The flash kernel never materialises the probabilities, so by default the second return value is
+    ``None`` (except R == 1, where the reference's all-ones tensor is cheap).  ``need_weights=True``
+    returns the reference's ``[H, C, B, R, R]`` fp32 probabilities, computed by a separate pair of
+    kernels from the same q|k (``rnamsm_col_attn_probs``); ``out`` is the same either way.
     """
 
     @torch.no_grad()
-    def forward(self, x, self_attn_mask=None, self_attn_padding_mask=None):
+    def forward(self, x, self_attn_mask=None, self_attn_padding_mask=None, need_weights: bool = False):
         self._check_input(x, self_attn_mask)
         R, Cc, B, D = x.shape
         H = self.num_heads
@@ -195,6 +196,11 @@ class ColumnSelfAttention(_AxialAttentionBase):
         dt = L.torch_dtype(code)
         w_qkv, b_qkv, w_out, b_out = self._pack(code)
         out = torch.empty((R, Cc, B, D), dtype=torch.float32, device=x.device)
+        want = need_weights and R > 1
+        if want:
+            attn = torch.empty((H, Cc, B, R, R), dtype=torch.float32, device=x.device)
+            probs = attn[:, :, 0] if B == 1 else torch.empty((H, Cc, R, R), dtype=torch.float32, device=x.device)
+            scratch = torch.empty(L.lib.rnamsm_col_probs_scratch_bytes(R, Cc, H), dtype=torch.uint8, device=x.device)
         with torch.cuda.device(x.device):
             st = L.stream_ptr()
             for b in range(B):
@@ -207,9 +213,15 @@ class ColumnSelfAttention(_AxialAttentionBase):
                     qkv = _linear(xb, w_qkv, b_qkv, code, L.EPI_BIAS, self.scaling, D, None)
                     ctx = torch.empty((R * Cc, D), dtype=dt, device=x.device)
                     L.check(L.lib.rnamsm_col_attn(L.ptr(qkv), R, Cc, H, code, 0, L.ptr(pad), L.ptr(ctx), st), "col_attn")
+                    if want:
+                        L.check(L.lib.rnamsm_col_attn_probs(L.ptr(qkv), R, Cc, H, code, 0, L.ptr(pad), L.ptr(probs), None,
+                                                            L.ptr(scratch), st), "col_attn_probs")
+                        if B > 1:
+                            attn[:, :, b] = probs
                     ob = _linear(ctx, w_out, b_out, code)
                 out[:, :, b, :] = ob.view(R, Cc, D).float()
-        attn = torch.ones(H, Cc, B, 1, 1, device=x.device, dtype=x.dtype) if R == 1 else None
+        if not want:
+            attn = torch.ones(H, Cc, B, 1, 1, device=x.device, dtype=x.dtype) if R == 1 else None
         return out, attn
 
 
@@ -342,7 +354,12 @@ class AxialTransformerLayer(nn.Module, _PrecisionMixin):
 
     @torch.no_grad()
     def forward(self, x: torch.Tensor, self_attn_mask: Optional[torch.Tensor] = None,
-                self_attn_padding_mask: Optional[torch.Tensor] = None, need_head_weights: bool = False):
+                self_attn_padding_mask: Optional[torch.Tensor] = None, need_head_weights: bool = False,
+                need_col_weights: bool = False):
+        """``need_col_weights=True`` (implies ``need_head_weights``) also returns the column attention's
+        probabilities ``[H, C, B, R, R]`` as the middle element, where it is ``None`` otherwise."""
+        if need_col_weights:
+            need_head_weights = True
         _infer_only(self)
         if self_attn_mask is not None:
             raise NotImplementedError
@@ -354,10 +371,14 @@ class AxialTransformerLayer(nn.Module, _PrecisionMixin):
         eps = float(self.row_self_attention.layer_norm.eps)
         y = torch.empty((R, Cc, B, D), dtype=torch.float32, device=x.device)
         row_attn = torch.empty((H, B, Cc, Cc), dtype=torch.float32, device=x.device) if need_head_weights else None
+        col_attn = torch.empty((H, Cc, B, R, R), dtype=torch.float32, device=x.device) if need_col_weights else None
         with torch.cuda.device(x.device):
             w = self.c_weights(code)
             fcode = self._fwd_code
             nbytes = L.lib.rnamsm_workspace_bytes(R, Cc, D, H, F, fcode)
+            if need_col_weights:
+                nbytes += L.lib.rnamsm_col_probs_scratch_bytes(R, Cc, H)
+                cp = col_attn[:, :, 0] if B == 1 else torch.empty((H, Cc, R, R), dtype=torch.float32, device=x.device)
             ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
             for b in range(B):
                 # fresh fp32 copy (never a view of the caller's x): the kernels update it in place
@@ -365,15 +386,22 @@ class AxialTransformerLayer(nn.Module, _PrecisionMixin):
                 xb.copy_(x[:, :, b, :])
                 pad = _pad_u8(self_attn_padding_mask, b)
                 pm = torch.empty((H, Cc, Cc), dtype=torch.float32, device=x.device) if need_head_weights else None
-                L.check(L.lib.rnamsm_layer_forward(C.byref(w), D, H, F, eps, L.ptr(xb), R, Cc, L.ptr(pad), fcode,
-                                                   L.ptr(pm), L.ptr(ws), nbytes, 0, None, None, 0, L.stream_ptr()),
-                        "layer_forward")
+                if need_col_weights:
+                    L.check(L.lib.rnamsm_layer_forward_col_probs(C.byref(w), D, H, F, eps, L.ptr(xb), R, Cc, L.ptr(pad),
+                                                                 fcode, L.ptr(pm), L.ptr(cp), None, L.ptr(ws), nbytes, 0,
+                                                                 None, None, 0, L.stream_ptr()), "layer_forward_col_probs")
+                    if B > 1:
+                        col_attn[:, :, b] = cp
+                else:
+                    L.check(L.lib.rnamsm_layer_forward(C.byref(w), D, H, F, eps, L.ptr(xb), R, Cc, L.ptr(pad), fcode,
+                                                       L.ptr(pm), L.ptr(ws), nbytes, 0, None, None, 0, L.stream_ptr()),
+                            "layer_forward")
                 y[:, :, b, :] = xb
                 if need_head_weights:
                     row_attn[:, b] = pm
         if need_head_weights:
-            # column probabilities are never materialised (see ColumnSelfAttention); keep the arity
-            return y, None, row_attn
+            # without need_col_weights the column probabilities are not computed (see ColumnSelfAttention)
+            return y, col_attn, row_attn
         return y
 
 
