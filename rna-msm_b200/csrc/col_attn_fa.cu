@@ -1,9 +1,10 @@
-// K7, 16-bit path, round-2 kernel: column attention with 128-key steps and P in tensor memory
+// K7, 16-bit path, MSAs deeper than 128 rows: column attention with 128-key steps and P in tensor memory
 // (modules.py:896-923).  For every alignment column c and head h the MSA depth R is the sequence axis:
 //   ctx[i,c,h,:] = sum_j softmax_j(q[i,c,h,:] . k[j,c,h,:]) v[j,c,h,:]     (q pre-scaled by 64^-1/2)
 //
 // Why this shape (tools/micro/mma_chain_bench.cu, tools/micro/tmem_umma_bench.cu on a B200; DESIGN.md 4.2): the
-// four-tile / 64-key kernel (col_attn_ws.cu) is held at ~3000 cycles per step by three resources at once --
+// round-1 kernel, four query tiles with 64-key steps and P through shared memory, was held at ~3000 cycles per step
+// by three resources at once --
 //   shared-memory port: an M128 N64 K16 MMA with both operands in shared memory reads 6 KiB for 32 cycles of math =
 //     48 cycles (measured: 4 issuing threads, 1536 cycles per 32 instructions), + 64 KiB of P stores per step
 //     = ~2200 cycles;  XU: 64 ex2 x 16 warps at 16/clk/SM = 2048 cycles;  issue slots of the softmax warps: ~2400
@@ -13,7 +14,7 @@
 //   P goes registers -> TENSOR MEMORY (tcgen05.st) and P V takes its A operand from there ([a_tmem]): only V is read
 //   from shared memory (2 KiB per 32-cycle instruction), no P stores, no generic->async proxy fence per step,
 //   one thread = one query row with 128 logits per step, so the per-step barrier / fence / wait overhead is paid
-//   once per 128 exponentials instead of once per 64, with 8 softmax warps of 168 registers instead of 16 of 96.
+//   once per 128 exponentials instead of once per 64, with 8 softmax warps of 216 registers instead of 16 of 96.
 // That leaves the XU as the only resource near its limit (shared memory ~1000, issue ~1100 of ~2200 cycles per step).
 //
 // TMEM (512 columns): tile t owns columns [256 t, 256 t + 256):  S 128 | P 64 (128 keys, two per column) | O 64.
@@ -24,16 +25,10 @@
 //   warps 1, 2        S issuer of tile 0 / 1 (lane 0); warp 1 owns the TMEM allocation
 //   warps 4, 5        PV issuer of tile 0 / 1 (lane 0); warps 3, 6, 7 idle (roles come in whole warpgroups for setmaxnreg)
 //   warps 8..15       softmax, one warpgroup per tile (thread = query row = TMEM lane): lazy rescaling (threshold 2^8),
-//                     packed fp32 pair arithmetic, optional polynomial 2^x on the FMA pipe for a share of the pairs
-#include <stdlib.h>
-
+//                     packed fp32 pair arithmetic
 #include "../../include/rnamsm_b200.h"
 #include "common.cuh"
 #include "launch.h"
-
-#ifndef RNAMSM_COL_WG
-#define RNAMSM_COL_WG 1
-#endif
 
 namespace rnamsm {
 
@@ -43,19 +38,15 @@ constexpr int NT = 2, BQ = 128, BKV = 128, HD = 64;
 constexpr int Q_BYTES = BQ * HD * 2;        // 16 KiB per tile
 constexpr int KV_BYTES = BKV * HD * 2;      // 16 KiB each for K and V
 constexpr int STG_BYTES = BQ * HD * 2;      // 16 KiB per tile: O rows staged for the TMA store
-constexpr int kKvStages = RNAMSM_COL_WG == 2 ? 3 : 4;   // (two warpgroups per tile: 2 KiB of row sums take the room of the 4th stage)
+constexpr int kKvStages = 4;
 constexpr int OFF_Q = 0;                                     // [2 item buffers][NT tiles]
 constexpr int OFF_KV = OFF_Q + 2 * NT * Q_BYTES;             // [stages][K | V]
 constexpr int OFF_STG = OFF_KV + kKvStages * 2 * KV_BYTES;   // [NT tiles]
-constexpr int OFF_LSUM = OFF_STG + NT * STG_BYTES;            // [NT][2][BQ] fp32 partial row sums (kWG = 2)
-constexpr int OFF_BAR = OFF_LSUM + (RNAMSM_COL_WG == 2 ? NT * 2 * BQ * 4 : 0);
+constexpr int OFF_BAR = OFF_STG + NT * STG_BYTES;
 constexpr int kSmem = OFF_BAR + 512 + 1024;
-constexpr int kWG = RNAMSM_COL_WG;                           // softmax warpgroups per tile (1: a thread owns 128 keys of a step, 2: 64)
-constexpr int CW = BKV / kWG;                                // key columns per softmax thread and step
 constexpr int kRoleWarps = 8;                                // two warpgroups of single-thread roles (3 warps idle)
-constexpr int kWarps = kRoleWarps + 4 * NT * kWG;
-constexpr int kThreads = 32 * kWarps;                        // 512 (kWG = 1) or 768 threads
-constexpr int kRoleRegs = kWG == 1 ? 40 : 32, kSoftmaxRegs = kWG == 1 ? 216 : 104;   // setmaxnreg; kWG = 1: 256 x 40 + 256 x 216 = 65536 (launch 512 x 128); kWG = 2: 256 x 32 + 512 x 104 = 61440 = launch 768 x 80
+constexpr int kThreads = 512;                                // the role warps + one softmax warpgroup per tile
+constexpr int kRoleRegs = 40, kSoftmaxRegs = 216;            // setmaxnreg: 256 x 40 + 256 x 216 = 65536 = launch 512 x 128
 constexpr int kTmemCols = 512;
 constexpr int TM_S = 0, TM_P = 128, TM_O = 192, TM_TILE = 256;
 constexpr float kLog2e = 1.4426950408889634f;
@@ -70,41 +61,7 @@ __device__ __forceinline__ float ex2(float x) {
 // Orders a volatile asm (a barrier probe) behind the computation of v without emitting an instruction.
 __device__ __forceinline__ void anchor_after(float v) { asm volatile("" ::"f"(v) : "memory"); }
 
-// 2^x for a packed pair on the FMA / ALU pipes instead of the XU: x = n + f by the 1.5 * 2^23 magic add, degree-3
-// minimax polynomial for 2^f on [-0.5, 0.5] (max relative error 7.5e-5, below the 16-bit rounding of P), n added
-// into the exponent field.
-__device__ __forceinline__ void exp2_poly2(uint64_t x, float& r0, float& r1) {
-  float x0, x1;
-  f32x2_unpack(x, x0, x1);
-  const uint64_t xc = f32x2_pack(fmaxf(x0, -126.f), fmaxf(x1, -126.f));
-  const uint64_t t = f32x2_add(xc, f32x2_pack(12582912.f, 12582912.f));
-  const uint64_t fl = f32x2_add(t, f32x2_pack(-12582912.f, -12582912.f));
-  const uint64_t fr = f32x2_fma(fl, f32x2_pack(-1.f, -1.f), xc);
-  uint64_t p = f32x2_fma(f32x2_pack(0.05517144873738289f, 0.05517144873738289f), fr,
-                         f32x2_pack(0.2426108419895172f, 0.2426108419895172f));
-  p = f32x2_fma(p, fr, f32x2_pack(0.6932609677314758f, 0.6932609677314758f));
-  p = f32x2_fma(p, fr, f32x2_pack(0.9999281167984009f, 0.9999281167984009f));
-  float p0, p1, t0, t1;
-  f32x2_unpack(p, p0, p1);
-  f32x2_unpack(t, t0, t1);
-  r0 = __uint_as_float(__float_as_uint(p0) + (__float_as_uint(t0) << 23));
-  r1 = __uint_as_float(__float_as_uint(p1) + (__float_as_uint(t1) << 23));
-}
-
 struct Item { int c, h, i0; };
-
-// Debug timeline (RNAMSM_COL_TRACE=<file>): CTA 0 logs clock64() at the hand-over points of its first steps, one row per
-// role thread; dumped by the launcher.  Compiled into a separate instantiation only.
-constexpr int kTraceRoles = 7, kTraceLen = 512;
-__device__ long long g_trace[kTraceRoles][kTraceLen];
-template <bool kTrace>
-struct Tracer {
-  int role, n;
-  __device__ __forceinline__ Tracer(int r) : role(r), n(0) {}
-  __device__ __forceinline__ void log(int code) {
-    if (kTrace && blockIdx.x == 0 && n < kTraceLen) g_trace[role][n++] = (clock64() << 4) | code;
-  }
-};
 
 __device__ __forceinline__ Item decode_item(int item, int nqb, int H) {
   Item it;
@@ -115,13 +72,11 @@ __device__ __forceinline__ Item decode_item(int item, int nqb, int H) {
   return it;
 }
 
-// kPoly: 0 = every exponential on the XU; n > 0 = the second pair of every n-th group of four keys on the FMA pipe
-// (exp2_poly2): 1 -> 50 % of the exponentials, 2 -> 25 %, 4 -> 12.5 %
-template <bool kFp16, int kPoly, bool kTrace>
+template <bool kFp16>
 __global__ void __launch_bounds__(kThreads, 1)
 col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_kv,
                    const __grid_constant__ CUtensorMap tm_o, int R, int C, int H, int col_major, int n_items,
-                   const uint8_t* __restrict__ pad, int stagger, int tight) {
+                   const uint8_t* __restrict__ pad) {
   constexpr int fp16 = kFp16 ? 1 : 0;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -150,8 +105,8 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       mbar_init(&q_full[b], 1);
       mbar_init(&q_empty[b], NT);               // one commit per MMA issuer
       mbar_init(&s_full[b], 1);
-      mbar_init(&s_free[b], 4 * kWG);
-      mbar_init(&p_full[b], 4 * kWG);
+      mbar_init(&s_free[b], 4);
+      mbar_init(&p_full[b], 4);
       mbar_init(&pv_done[b], 1);
     }
     for (int b = 0; b < 4; ++b) {
@@ -178,7 +133,6 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     int kv_stage = 0;
     uint32_t kv_phase = 0;
     int li = 0;
-    Tracer<kTrace> tr(0);
     for (int item = blockIdx.x; item < n_items; item += gridDim.x, ++li) {
       const Item it = decode_item(item, nqb, H);
       const int qb = li & 1, quse = li >> 1;
@@ -190,7 +144,6 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
                     col_major ? it.i0 + t * BQ : it.c, col_major ? it.c : it.i0 + t * BQ);
       for (int j = 0; j < nblk; ++j) {
         mbar_wait_relaxed(&kv_empty[kv_stage], kv_phase ^ 1);
-        tr.log(1);
         uint8_t* sk = smem + OFF_KV + kv_stage * 2 * KV_BYTES;
         mbar_expect_tx(&kv_full[kv_stage], 2 * KV_BYTES);
         tma_load_3d(sk, &tm_kv, &kv_full[kv_stage], D + it.h * HD, col_major ? j * BKV : it.c, col_major ? it.c : j * BKV);
@@ -211,19 +164,13 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     int s_stage = 0;
     uint32_t s_phase = 0;
     long long gs = 0;
-    Tracer<kTrace> tr(1 + t);
     for (int li = 0; li < my_items; ++li) {
       const int qb = li & 1, quse = li >> 1;
       mbar_wait_relaxed(&q_full[qb], quse & 1);
       const uint32_t qa = smem_u32(smem + OFF_Q + (qb * NT + t) * Q_BYTES);
       for (int j = 0; j < nblk; ++j, ++gs) {
         mbar_wait_relaxed(&kv_full[s_stage], s_phase);
-        tr.log(1);                                                           // K/V stage landed
-        if (gs > 0) {                                                        // softmax t holds S(gs-1) in registers
-          if (tight) mbar_wait_quiet(&s_free[t], (uint32_t)((gs - 1) & 1));
-          else mbar_wait_relaxed(&s_free[t], (uint32_t)((gs - 1) & 1));
-        }
-        tr.log(2);                                                           // S columns free
+        if (gs > 0) mbar_wait_quiet(&s_free[t], (uint32_t)((gs - 1) & 1));   // softmax t holds S(gs-1) in registers
         tc_fence_after();
         const uint32_t ka = smem_u32(smem + OFF_KV + s_stage * 2 * KV_BYTES);
 #pragma unroll
@@ -231,7 +178,6 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
           umma_16(tmem_S, make_smem_desc_sw128(qa + k * 32, 16, 1024), make_smem_desc_sw128(ka + k * 32, 16, 1024), idesc_s,
                   (uint32_t)(k != 0));
         umma_commit(&s_full[t]);
-        tr.log(3);                                                           // S issued
         if (j == nblk - 1) umma_commit(&q_empty[qb]);            // this tile's Q fully consumed
         if (++s_stage == kKvStages) { s_stage = 0; s_phase ^= 1; }
       }
@@ -245,21 +191,16 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     const uint32_t tmem_P = tmem_base + t * TM_TILE + TM_P, tmem_O = tmem_base + t * TM_TILE + TM_O;
     int o_j = 0, o_stage = 0;
     uint32_t o_phase = 0;
-    Tracer<kTrace> tr(3 + t);
     for (long long g = 0; g < total_steps; ++g) {
       const uint32_t va = smem_u32(smem + OFF_KV + o_stage * 2 * KV_BYTES + KV_BYTES);
       mbar_wait_relaxed(&kv_full[o_stage], o_phase);             // (complete long ago: this thread's own acquire of V)
-      tr.log(2);
-      if (tight) mbar_wait_quiet(&p_full[t], (uint32_t)(g & 1));   // P_t(g) in TMEM, O_t rescaled if needed
-      else mbar_wait_relaxed(&p_full[t], (uint32_t)(g & 1));
-      tr.log(1);                                                 // P seen
+      mbar_wait_quiet(&p_full[t], (uint32_t)(g & 1));             // P_t(g) in TMEM, O_t rescaled if needed
       tc_fence_after();
 #pragma unroll
       for (int k = 0; k < BKV / 16; ++k)                         // 16 keys = 8 packed TMEM columns per instruction
         umma_16_ts(tmem_O, tmem_P + k * 8, make_smem_desc_sw128(va + k * 2048, 8192, 1024), idesc_o,
                    (uint32_t)((o_j | k) != 0));
       umma_commit(&pv_done[t]);
-      tr.log(3);                                                 // PV issued
       umma_commit(&kv_empty[o_stage]);                           // this tile is done with K_j and V_j
       if (++o_j == nblk) o_j = 0;
       if (++o_stage == kKvStages) { o_stage = 0; o_phase ^= 1; }
@@ -268,20 +209,15 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
   } else {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kSoftmaxRegs));
     // ================================ softmax warpgroups ==========================
-    // kWG warpgroups per tile: warpgroup `half` owns key columns [half * CW, half * CW + CW) of every step; a thread is one
-    // query row (TMEM lane) restricted to those columns.
-    const int sw = warp - kRoleWarps;
-    const int t = sw / (4 * kWG);                  // tile
-    const int half = (sw >> 2) % kWG;              // which CW-key part of the 128 keys of a step
+    // One warpgroup per tile; a thread is one query row (TMEM lane) and owns its 128 keys of every step.
+    const int t = (warp - kRoleWarps) / 4;         // tile
     const int quad = warp & 3;                     // TMEM lane quadrant of this warp
     const int row = quad * 32 + lane;              // query row inside the tile == TMEM lane
     const uint32_t lane_off = (uint32_t)(quad * 32) << 16;
     const uint32_t tmem_S = tmem_base + t * TM_TILE + TM_S + lane_off;
-    const uint32_t tmem_P = tmem_base + t * TM_TILE + TM_P + lane_off + half * (CW / 2);
+    const uint32_t tmem_P = tmem_base + t * TM_TILE + TM_P + lane_off;
     const uint32_t tmem_O = tmem_base + t * TM_TILE + TM_O + lane_off;
     uint8_t* srow = smem + OFF_STG + t * STG_BYTES + row * 128;
-    float* lsum = reinterpret_cast<float*>(smem + OFF_LSUM) + (t * 2) * BQ + row;   // [tile][half][row] partial row sums
-    const int pair_bar = 1 + t * 4 + quad;         // named barrier of the kWG warps that share these 32 rows
     const uint32_t b_s_full = smem_u32(&s_full[t]), b_s_free = smem_u32(&s_free[t]), b_p_full = smem_u32(&p_full[t]),
                    b_pv_done = smem_u32(&pv_done[t]);
     const float neg_masked = -10000.f;             // masked_fill value, modules.py:911-915
@@ -290,24 +226,16 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     // exponentials: PV(last) of the finished item completes behind them instead of being waited for (ncu: 13 probes
     // per item on that wait = 6 % of the softmax warps' time at R = 1024, more for shallower MSAs).
     bool have_prev = false, s_ok = false;
-    Tracer<kTrace> tr(half == 0 && quad == 0 && lane == 0 ? 5 + t : -1);
     Item prev_it{0, 0, 0};
     float prev_l = 0.f;
-    auto read_out = [&](const Item& pit, float l_part) {
+    auto read_out = [&](const Item& pit, float l) {
       // 16-bit rows staged in shared memory (SWIZZLE_128B pattern of the store's tensor map), one asynchronous TMA
-      // store per 32 rows.  With two warpgroups per tile each normalises and stages its own 32 of the 64 output columns;
-      // the row sums meet through shared memory.
-      if (half == 0 && lane == 0) bulk_wait_read0();   // the staged rows of the item before have been read by their store
-      float l_tot = l_part;
-      if (kWG == 2) {
-        asm volatile("bar.sync %0, 64;" ::"r"(pair_bar) : "memory");   // partner's partial sum written, staging free
-        l_tot += lsum[(half ^ 1) * BQ];
-      } else {
-        __syncwarp();
-      }
-      const float inv = 1.f / l_tot;
+      // store per 32 rows.
+      if (lane == 0) bulk_wait_read0();            // the staged rows of the item before have been read by their store
+      __syncwarp();
+      const float inv = 1.f / l;
 #pragma unroll 1
-      for (int hlf = (kWG == 2 ? half : 0); hlf < (kWG == 2 ? half + 1 : 2); ++hlf) {
+      for (int hlf = 0; hlf < 2; ++hlf) {
         uint32_t ov[32];
         tmem_ld_32x32(tmem_O + hlf * 32, ov);
         tmem_ld_wait();
@@ -329,75 +257,32 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
         }
       }
       fence_proxy_async_smem();     // staged rows -> visible to the TMA (async proxy)
-      if (kWG == 2) asm volatile("bar.sync %0, 64;" ::"r"(pair_bar) : "memory");   // both column halves staged
-      else __syncwarp();
+      __syncwarp();
       const int i_warp = pit.i0 + t * BQ + quad * 32;          // first query row of this warp; rows >= R are clipped
-      if (half == 0 && lane == 0 && i_warp < R) {
+      if (lane == 0 && i_warp < R) {
         tma_store_3d(&tm_o, smem + OFF_STG + t * STG_BYTES + quad * 32 * 128, pit.h * HD, pit.c, i_warp);
         bulk_commit();
       }
     };
-    // (kWG == 1) The two tiles' warps share each sub-partition's XU; tile 1 may start late once (kStagger cycles).
-    if (stagger > 0 && t == 1) {
-      const long long t_start = clock64();
-      while (clock64() - t_start < stagger) {}
-    }
     for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
       const Item it = decode_item(item, nqb, H);
       float m_ref = -INFINITY, l_run = 0.f;
       for (int j = 0; j < nblk; ++j, ++g) {
-        const int j0 = j * BKV + half * CW;        // first key of this thread's columns
+        const int j0 = j * BKV;
         if (!s_ok) mbar_wait_quiet_u32(b_s_full, (uint32_t)(g & 1));   // (probed inside the previous step)
         tc_fence_after();
-        if (tr.role >= 0) tr.log(s_ok ? 1 : 2);                  // S ready (1: the early probe had seen it)
-        uint32_t sv[CW / 32][32];
-        float mx_other = -INFINITY;
+        uint32_t sv[BKV / 32][32];
 #pragma unroll
-        for (int q = 0; q < CW / 32; ++q) tmem_ld_32x32(tmem_S + half * CW + q * 32, sv[q]);
-        if (kWG == 2) {
-          // the row maximum needs all 128 logits: the other warpgroup's 64 columns are read as well (tensor-memory reads
-          // are cheap: 8 KiB per warp in ~35 cycles), only for the maximum -- identical arithmetic in both warpgroups, so
-          // both take the same rescaling decisions without talking to each other
-          const bool slow = pad != nullptr || j * BKV + BKV > R;
-          const int jo = j * BKV + (half ^ 1) * CW;
-#pragma unroll 1
-          for (int q = 0; q < CW / 32; ++q) {
-            uint32_t ot[32];
-            tmem_ld_32x32(tmem_S + (half ^ 1) * CW + q * 32, ot);
-            tmem_ld_wait();
-            uint32_t mbits = 0;
-            if (slow && pad != nullptr) {
-              const int jk = jo + q * 32 + lane;
-              mbits = __ballot_sync(0xffffffffu, jk < R && pad[(size_t)jk * C + it.c] != 0);
-            }
-            float m0 = -INFINITY, m1 = -INFINITY;
-#pragma unroll
-            for (int e = 0; e < 32; e += 2) {
-              float v0 = __uint_as_float(ot[e]), v1 = __uint_as_float(ot[e + 1]);
-              if (slow) {
-                if ((mbits >> e) & 1u) v0 = neg_masked;
-                if ((mbits >> (e + 1)) & 1u) v1 = neg_masked;
-                if (jo + q * 32 + e >= R) v0 = -INFINITY;
-                if (jo + q * 32 + e + 1 >= R) v1 = -INFINITY;
-              }
-              m0 = fmaxf(m0, v0);
-              m1 = fmaxf(m1, v1);
-            }
-            mx_other = fmaxf(mx_other, fmaxf(m0, m1));
-          }
-        } else {
-          tmem_ld_wait();
-        }
+        for (int q = 0; q < BKV / 32; ++q) tmem_ld_32x32(tmem_S + q * 32, sv[q]);
+        tmem_ld_wait();
         tc_fence_before();
-        if (kWG == 2) __syncwarp();
-        else __syncwarp();
-        if (tr.role >= 0) tr.log(3);                             // S in registers
+        __syncwarp();
         if (lane == 0) mbar_arrive_u32(b_s_free);   // S columns may be overwritten by the next step's S
 
         if (pad != nullptr || j * BKV + BKV > R) {               // warp-uniform slow path: key masks
           const int n_valid = R - j0;
 #pragma unroll
-          for (int q = 0; q < CW / 32; ++q) {
+          for (int q = 0; q < BKV / 32; ++q) {
             uint32_t mbits = 0;
             if (pad != nullptr) {
               const int jk = j0 + q * 32 + lane;
@@ -412,9 +297,9 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
             }
           }
         }
-        float mx0 = mx_other, mx1 = -INFINITY, mx2 = -INFINITY, mx3 = -INFINITY;
+        float mx0 = -INFINITY, mx1 = -INFINITY, mx2 = -INFINITY, mx3 = -INFINITY;
 #pragma unroll
-        for (int q = 0; q < CW / 32; ++q) {
+        for (int q = 0; q < BKV / 32; ++q) {
 #pragma unroll
           for (int e = 0; e < 32; e += 4) {
             mx0 = fmaxf(mx0, __uint_as_float(sv[q][e]));
@@ -439,7 +324,7 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
         const uint64_t c_l2e = f32x2_pack(kLog2e, kLog2e), c_negm = f32x2_pack(-m_ref, -m_ref);
         uint64_t acc0 = f32x2_pack(0.f, 0.f), acc1 = acc0;
 #pragma unroll
-        for (int q = 0; q < CW / 32; ++q) {
+        for (int q = 0; q < BKV / 32; ++q) {
 #pragma unroll
           for (int e = 0; e < 32; e += 4) {
             const uint64_t x0 = f32x2_fma(f32x2_pack(__uint_as_float(sv[q][e]), __uint_as_float(sv[q][e + 1])), c_l2e, c_negm);
@@ -447,20 +332,15 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
             float a0, a1, a2, a3;
             f32x2_unpack(x0, a0, a1);
             a0 = ex2(a0); a1 = ex2(a1);
-            if (q == CW / 32 - 1 && e == 16) {
+            if (q == BKV / 32 - 1 && e == 16) {
               // probe "PV(g-1) done" seven eighths through (a test_wait is non-blocking; its ~100 cycles of latency pass
               // behind the last exponentials; the in-kernel timeline puts PV(g-1)'s completion ~1300 cycles after P(g-1)
               // was handed over: a barrier hand-over between threads costs ~350 cycles each way)
               anchor_after(a1);
               if (g > 0) pv_ok = mbar_test_wait_u32(b_pv_done, (uint32_t)((g - 1) & 1));
             }
-            constexpr int kP = kPoly > 0 ? kPoly : 1;
-            if (kPoly > 0 && (((q * 32 + e) >> 2) % kP) == kP - 1) {
-              exp2_poly2(x1, a2, a3);
-            } else {
-              f32x2_unpack(x1, a2, a3);
-              a2 = ex2(a2); a3 = ex2(a3);
-            }
+            f32x2_unpack(x1, a2, a3);
+            a2 = ex2(a2); a3 = ex2(a3);
             acc0 = f32x2_add(acc0, f32x2_pack(a0, a1));
             acc1 = f32x2_add(acc1, f32x2_pack(a2, a3));
             const int w = (q * 32 + e) >> 1;                 // P word index inside this thread's columns
@@ -475,15 +355,13 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
           l_run += (s0 + s1) + (s2 + s3);
         }
         s_ok = mbar_test_wait_u32(b_s_full, (uint32_t)((g + 1) & 1));   // next step's S; the answer is used ~400 cycles on
-        if (tr.role >= 0) tr.log(pv_ok ? 4 : 5);                 // exponentials done (4: the probe had seen PV(g-1) done)
         if (!pv_ok) mbar_wait_quiet_u32(b_pv_done, (uint32_t)((g - 1) & 1));   // PV(g-1) done: P columns free, O_t stable
         tc_fence_after();
-        if (tr.role >= 0) tr.log(6);                             // PV(g-1) done
         if (j == 0 && have_prev) read_out(prev_it, prev_l);     // the finished item's O, before PV(g) overwrites it
         if (rescale) {                              // warp-uniform; rare once the max has settled
           uint32_t ov[32];
 #pragma unroll 1
-          for (int hlf = (kWG == 2 ? half : 0); hlf < (kWG == 2 ? half + 1 : 2); ++hlf) {
+          for (int hlf = 0; hlf < 2; ++hlf) {
             tmem_ld_32x32(tmem_O + hlf * 32, ov);
             tmem_ld_wait();
 #pragma unroll
@@ -492,16 +370,14 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
           }
         }
 #pragma unroll
-        for (int q = 0; q < CW / 64; ++q) tmem_st_32x32(tmem_P + q * 32, sv[q]);   // P(g): two keys per column, A operand of P V
+        for (int q = 0; q < BKV / 64; ++q) tmem_st_32x32(tmem_P + q * 32, sv[q]);   // P(g): two keys per column, A operand of P V
         tmem_st_wait();
         tc_fence_before();                          // our tcgen05.ld / st precede the MMA that follows the barrier
         __syncwarp();
-        if (tr.role >= 0) tr.log(7);                             // P handed over
         if (lane == 0) mbar_arrive_u32(b_p_full);
       }
       prev_it = it;
       prev_l = l_run;
-      if (kWG == 2) lsum[half * BQ] = l_run;        // read by the partner warpgroup behind the first barrier of read_out
       have_prev = true;
     }
     if (have_prev) {                                // the last item of this CTA
@@ -518,25 +394,12 @@ col_attn_fa_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
   if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
 }
 
-// Experiment knobs (defaults = the measured best): RNAMSM_COL_STAGGER=<cycles> delays tile 1's softmax warps once,
-// RNAMSM_COL_TIGHT=0 lets the S / PV issuing threads sleep on their barriers instead of probing them back to back.
-int knob_stagger() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("RNAMSM_COL_STAGGER"); v = e ? atoi(e) : 0; }
-  return v;
-}
-int knob_tight() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("RNAMSM_COL_TIGHT"); v = e ? atoi(e) : 1; }
-  return v;
-}
-
-template <bool kFp16, int kPoly, bool kTrace = false>
+template <bool kFp16>
 int launch_fa(const CUtensorMap& tq, const CUtensorMap& tkv, const CUtensorMap& to, int R, int C, int H, int col_major,
               const uint8_t* pad, cudaStream_t st) {
   static bool attr_set = false;
   if (!attr_set) {
-    RNAMSM_CHECK_CUDA(cudaFuncSetAttribute(col_attn_fa_kernel<kFp16, kPoly, kTrace>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));
+    RNAMSM_CHECK_CUDA(cudaFuncSetAttribute(col_attn_fa_kernel<kFp16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));
     attr_set = true;
   }
   const long long n_items = (long long)C * H * ((R + NT * BQ - 1) / (NT * BQ));
@@ -547,21 +410,10 @@ int launch_fa(const CUtensorMap& tq, const CUtensorMap& tkv, const CUtensorMap& 
   if (sms <= 0) sms = 148;
   const int grid = (int)std::min<long long>(n_items, sms);
   ProfScope prof(KC_COL_ATTN, st);
-  RNAMSM_CHECK_CUDA(launch_pdl(col_attn_fa_kernel<kFp16, kPoly, kTrace>, dim3(grid), dim3(kThreads), kSmem, st, tq, tkv, to, R, C, H,
-                               col_major, (int)n_items, pad, knob_stagger(), knob_tight()));
+  RNAMSM_CHECK_CUDA(launch_pdl(col_attn_fa_kernel<kFp16>, dim3(grid), dim3(kThreads), kSmem, st, tq, tkv, to, R, C, H,
+                               col_major, (int)n_items, pad));
   count_launch();
   RNAMSM_CHECK_CUDA(cudaGetLastError());
-  if (kTrace) {
-    static long long h[kTraceRoles][kTraceLen];
-    RNAMSM_CHECK_CUDA(cudaStreamSynchronize(st));
-    RNAMSM_CHECK_CUDA(cudaMemcpyFromSymbol(h, g_trace, sizeof(h)));
-    if (FILE* f = fopen(getenv("RNAMSM_COL_TRACE"), "w")) {
-      static const char* names[kTraceRoles] = {"tma", "s0", "s1", "pv0", "pv1", "softmax0", "softmax1"};
-      for (int r = 0; r < kTraceRoles; ++r)
-        for (int i = 0; i < kTraceLen && h[r][i] != 0; ++i) fprintf(f, "%s %lld %d\n", names[r], h[r][i] >> 4, (int)(h[r][i] & 15));
-      fclose(f);
-    }
-  }
   return 0;
 }
 
@@ -586,23 +438,8 @@ int launch_col_attn_fa_16(const void* qkv, int R, int C, int H, int fp16, int co
   uint64_t ostrides[2] = {(uint64_t)H * HD * 2, (uint64_t)C * H * HD * 2};
   uint32_t box_o[3] = {HD, 1, 32};
   if (encode_tmap(&to, in_dt, ctx, 3, odims, ostrides, box_o)) return 3;
-  static int poly = -1;
-  if (poly < 0) {
-    const char* e = getenv("RNAMSM_COL_POLY");
-    poly = e ? atoi(e) : 0;
-  }
-  if (fp16 && getenv("RNAMSM_COL_TRACE")) return launch_fa<true, 0, true>(tq, tkv, to, R, C, H, col_major, pad, st);
-  if (poly == 4)
-    return fp16 ? launch_fa<true, 4>(tq, tkv, to, R, C, H, col_major, pad, st)
-                : launch_fa<false, 4>(tq, tkv, to, R, C, H, col_major, pad, st);
-  if (poly == 1)
-    return fp16 ? launch_fa<true, 1>(tq, tkv, to, R, C, H, col_major, pad, st)
-                : launch_fa<false, 1>(tq, tkv, to, R, C, H, col_major, pad, st);
-  if (poly == 2)
-    return fp16 ? launch_fa<true, 2>(tq, tkv, to, R, C, H, col_major, pad, st)
-                : launch_fa<false, 2>(tq, tkv, to, R, C, H, col_major, pad, st);
-  return fp16 ? launch_fa<true, 0>(tq, tkv, to, R, C, H, col_major, pad, st)
-              : launch_fa<false, 0>(tq, tkv, to, R, C, H, col_major, pad, st);
+  return fp16 ? launch_fa<true>(tq, tkv, to, R, C, H, col_major, pad, st)
+              : launch_fa<false>(tq, tkv, to, R, C, H, col_major, pad, st);
 }
 
 }  // namespace rnamsm

@@ -3,7 +3,7 @@
 //                   replaced by -10000 where key j of column c is padded (masked_fill, modules.py:911-915)
 //   P[h, c, i, j] = softmax_j(s_ij)
 //   mean[h, i, j] = (1/C) sum_c P[h, c, i, j]        (without the full tensor existing anywhere)
-// The flash kernels (col_attn_umma.cu, col_attn_fa.cu, col_attn_ws.cu, simt_f32.cu) never form P, so these read the
+// The flash kernels (col_attn_umma.cu, col_attn_fa.cu, simt_f32.cu) never form P, so these read the
 // same q|k buffer and pad flags again, in two passes:
 //   1. lse: one CTA per (column, head, query tile) streams the key blocks of its column and keeps a running max / sum;
 //      the row's max m[h, c, i] and log-sum log(sum_j exp(s_ij - m)) go to two fp32 [H, C, R] scratch arrays.  They stay

@@ -1,5 +1,5 @@
 // K7, 16-bit path, shallow MSAs (R <= 128): flash-style column attention on tcgen05 (modules.py:896-923).
-// Deeper MSAs run the persistent warp-specialised kernel in col_attn_ws.cu.
+// Deeper MSAs run the persistent warp-specialised kernel in col_attn_fa.cu.
 //
 // For every alignment column c and head h the MSA depth R is the sequence axis:
 //   ctx[i,c,h,:] = sum_j softmax_j(q[i,c,h,:] . k[j,c,h,:]) v[j,c,h,:]          (q pre-scaled by 64^-0.5)
@@ -16,8 +16,6 @@
 // math.  64 KiB smem and 128 TMEM columns per CTA -> 3 CTAs per SM interleave MMA and softmax.
 #include "../../include/rnamsm_b200.h"
 #include "common.cuh"
-#include <stdlib.h>
-
 #include "launch.h"
 
 namespace rnamsm {
@@ -229,36 +227,6 @@ col_attn_umma_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
   if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
 }
 
-}  // namespace
-
-int launch_col_attn_ws_16(const void* qkv, int R, int C, int H, int fp16, int col_major, const uint8_t* pad, void* ctx,
-                          cudaStream_t st);   // col_attn_ws.cu
-int launch_col_attn_fa_16(const void* qkv, int R, int C, int H, int fp16, int col_major, const uint8_t* pad, void* ctx,
-                          cudaStream_t st);   // col_attn_fa.cu
-
-// Dispatch: MSAs deeper than one 128-row query tile run the persistent warp-specialised kernel
-// (col_attn_ws.cu: two query tiles ping-pong per CTA); shallow ones (R <= 128) keep this
-// one-tile-per-CTA kernel, whose single tile wastes nothing.  RNAMSM_COL_ATTN=small|ws forces one.
-int launch_col_attn_small_16(const void* qkv, int R, int C, int H, int fp16, int col_major, const uint8_t* pad, void* ctx,
-                             cudaStream_t st);
-int launch_col_attn_16(const void* qkv, int R, int C, int H, int fp16, int col_major, const uint8_t* pad, void* ctx,
-                       cudaStream_t st) {
-  static int forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("RNAMSM_COL_ATTN");
-    forced = !e ? 0 : (e[0] == 's' ? 1 : (e[0] == 'w' ? 2 : 0));
-  }
-  const bool use_ws = forced == 2 || (forced == 0 && R > 128);
-  if (!use_ws) return launch_col_attn_small_16(qkv, R, C, H, fp16, col_major, pad, ctx, st);
-  static int impl = -1;                  // default: the 128-key-step kernel with P in tensor memory (col_attn_fa.cu);
-  if (impl < 0) {                        // RNAMSM_COL_IMPL=ws keeps the round-1 four-tile / 64-key kernel (col_attn_ws.cu)
-    const char* e = getenv("RNAMSM_COL_IMPL");
-    impl = (e && e[0] == 'w') ? 0 : 1;
-  }
-  return impl == 1 ? launch_col_attn_fa_16(qkv, R, C, H, fp16, col_major, pad, ctx, st)
-                   : launch_col_attn_ws_16(qkv, R, C, H, fp16, col_major, pad, ctx, st);
-}
-
 int launch_col_attn_small_16(const void* qkv, int R, int C, int H, int fp16, int col_major, const uint8_t* pad, void* ctx,
                              cudaStream_t st) {
   RNAMSM_REQUIRE(R >= 1 && C >= 1 && H >= 1 && C <= 2147483647 / 1 && H <= 65535, "col_attn_bf16: bad shape");
@@ -280,6 +248,20 @@ int launch_col_attn_small_16(const void* qkv, int R, int C, int H, int fp16, int
   count_launch();
   RNAMSM_CHECK_CUDA(cudaGetLastError());
   return 0;
+}
+
+}  // namespace
+
+int launch_col_attn_fa_16(const void* qkv, int R, int C, int H, int fp16, int col_major, const uint8_t* pad, void* ctx,
+                          cudaStream_t st);   // col_attn_fa.cu
+
+// Dispatch: MSAs deeper than one 128-row query tile run the persistent warp-specialised kernel
+// (col_attn_fa.cu: two query tiles per work item); shallow ones (R <= 128) keep this
+// one-tile-per-CTA kernel, whose single tile wastes nothing.
+int launch_col_attn_16(const void* qkv, int R, int C, int H, int fp16, int col_major, const uint8_t* pad, void* ctx,
+                       cudaStream_t st) {
+  if (R <= 128) return launch_col_attn_small_16(qkv, R, C, H, fp16, col_major, pad, ctx, st);
+  return launch_col_attn_fa_16(qkv, R, C, H, fp16, col_major, pad, ctx, st);
 }
 
 }  // namespace rnamsm
