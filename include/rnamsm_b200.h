@@ -349,6 +349,22 @@ int rnamsm_msa_forward_batch(const rnamsm_model_weights* m, int n_msa, const int
                              const uint8_t* has_pad, int dtype, float* x, float* const* row_attn_out, void* workspace,
                              size_t workspace_bytes, void* stream);
 
+/* Masked marginals of the LM head for one MSA (pseudo-log-likelihood, zero-shot mutant scores; utils/likelihood.py).
+ * Entry k of the outputs is computed on `tokens` [R, C] with token (row, cols[k]) replaced by mask_idx: the LM-head
+ * logits at (row, cols[k]) into logits_out [n_cols, vocab] (NULL = not wanted) and their log_softmax into
+ * logprobs_out [n_cols, vocab].  mask_idx < 0: nothing is masked, one forward, every listed column read from it.
+ * cols: DEVICE int32 [n_cols]; an entry that is out of range or names a <pad> token of `row` gives a NaN row in both
+ * outputs.  dtype: as rnamsm_msa_forward (RNAMSM_F32_TENSOR included).  16-bit with R >= 2: the masked grids run in
+ * passes of `group` through the layer path of rnamsm_msa_forward_batch; otherwise one forward per grid.  Only the scored
+ * token of each grid goes through the final LayerNorm and the LM head.  The logits are bit-identical to
+ * rnamsm_msa_forward's logits of the masked grid at that token.  workspace: rnamsm_score_workspace_bytes(..., group)
+ * bytes, 256 B aligned; `group` sizes it (0 = invalid arguments). */
+size_t rnamsm_score_workspace_bytes(int R, int C, int D, int H, int F, int dtype, int group);
+int rnamsm_msa_masked_marginals(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad,
+                                int dtype, int row, const int* cols, int n_cols, int mask_idx, int group,
+                                float* logits_out, float* logprobs_out, void* workspace, size_t workspace_bytes,
+                                void* stream);
+
 /* ---- one deep MSA sharded over the GPUs of a box (SURVEY.md 8e; rna-msm_b200/sharded.py) -----------
  * The reference has no multi-GPU forward; these entry points implement the partition its math allows:
  * rows for the tied row attention (sum of partial logits over ranks), columns for the column attention

@@ -100,6 +100,9 @@ SIGNATURES = {
     "rnamsm_batch_workspace_bytes": (_sz, [_i, C.POINTER(_i), C.POINTER(_i), _i, _i, _i, _i]),
     "rnamsm_msa_forward_batch": (_i, [C.POINTER(ModelWeights), _i, _vp, C.POINTER(_i), C.POINTER(_i), C.c_char_p, _i, _vp,
                                       C.POINTER(_vp), _vp, _sz, _vp]),
+    "rnamsm_score_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i]),
+    "rnamsm_msa_masked_marginals": (_i, [C.POINTER(ModelWeights), _vp, _i, _i, _i, _i, _i, _vp, _i, _i, _i, _vp, _vp,
+                                         _vp, _sz, _vp]),
     "rnamsm_rsa_pack": (_i, [_vp, _i, _i, _i, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]),
 }
 

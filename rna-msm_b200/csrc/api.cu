@@ -499,6 +499,55 @@ static int layer_forward_batch(const rnamsm_layer_weights* w, int D, int H, int 
   return 0;
 }
 
+// Embedding and layer stack of rnamsm_msa_forward_batch: everything but its final in-place LayerNorm.  Also the layer
+// path of the scoring entry, which reads one token per grid and normalises only that row.
+static int msa_forward_batch_layers(const rnamsm_model_weights* m, int n_msa, const int64_t* tokens, const int* R,
+                                    const int* C, const uint8_t* has_pad, int dtype, float* x, float* const* row_attn_out,
+                                    uint8_t* ws, const BatchPlan& bp, cudaStream_t st) {
+  const int D = m->embed_dim, H = m->num_heads, F = m->ffn_dim, N = m->num_layers;
+  uint8_t* pad = ws + bp.off_pad;
+  bool any_pad = false;
+  long long off = 0;
+  int rc;
+  for (int i = 0; i < n_msa; ++i) {
+    any_pad = any_pad || (has_pad && has_pad[i]);
+    if ((rc = launch_embed_ln(tokens + off, R[i], C[i], m->tok_emb, m->vocab, m->pos_emb, m->n_pos, m->row_pos,
+                              m->ln_before_w, m->ln_before_b, D, m->pad_idx, m->ln_eps, x + (size_t)off * D, pad + off, st)))
+      return rc;
+    off += (long long)R[i] * C[i];
+  }
+  for (int l = 0; l < N; ++l) {
+    NextLn next{nullptr, nullptr, dtype};
+    if (l + 1 < N)
+      next = NextLn{m->layers[l + 1].row.ln_w, m->layers[l + 1].row.ln_b, block_dtype(m->layers[l + 1].row.dtype, dtype)};
+    if ((rc = layer_forward_batch(&m->layers[l], D, H, F, m->ln_eps, x, n_msa, R, C, has_pad, any_pad, dtype, l,
+                                  row_attn_out, ws, bp, st, l > 0, next.w ? &next : nullptr)))
+      return rc;
+  }
+  return 0;
+}
+
+// RobertaLMHead (modules.py:313-319) on M rows: dense -> erf-GELU -> LayerNorm -> tied projection + bias.
+// lm16: dense + GELU on tcgen05 from xn16 (the final LayerNorm's 16-bit output, 16-bit h), LayerNorm with fp32
+// statistics -> fp32, 12-wide tied projection in fp32.  Otherwise FFMA (or tf32 x 3 with split scratch) from x, the
+// final LayerNorm's fp32 output.  hbuf: M * D * 4 bytes, h32: M * D fp32.
+static int lm_head_rows(const rnamsm_model_weights* m, const float* x, const void* xn16, long long M, int dtype, bool lm16,
+                        uint8_t* hbuf, float* h32, uint8_t* tf32_split, float* logits_out, cudaStream_t st) {
+  const int D = m->embed_dim;
+  int rc;
+  LinearEpilogue e{RNAMSM_EPI_BIAS_GELU, m->lm_dense_b, 1.f, 0, nullptr};
+  if (lm16) {
+    if ((rc = launch_linear_16(xn16, m->lm_dense_w16, M, D, D, dtype == RNAMSM_F16, e, hbuf, st))) return rc;
+    if ((rc = launch_layernorm((const float*)hbuf, m->lm_ln_w, m->lm_ln_b, h32, RNAMSM_F32, M, D, m->ln_eps, st, 0, 0,
+                               dtype)))
+      return rc;
+  } else {
+    if ((rc = linear_any(x, m->lm_dense_w, M, D, D, RNAMSM_F32, e, hbuf, st, nullptr, tf32_split))) return rc;
+    if ((rc = launch_layernorm((const float*)hbuf, m->lm_ln_w, m->lm_ln_b, h32, RNAMSM_F32, M, D, m->ln_eps, st))) return rc;
+  }
+  return launch_vocab_proj(h32, m->tok_emb, m->lm_bias, M, m->vocab, D, logits_out, st);
+}
+
 }  // namespace rnamsm
 
 using namespace rnamsm;
@@ -681,7 +730,7 @@ static int layer_forward_entry(const rnamsm_layer_weights* w, int D, int H, int 
 static int msa_forward_entry(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad, int dtype,
                              float* x, float* row_attn_out, float* col_probs_out, float* col_mean_out,
                              float* const* rep_out, float* logits_out, void* workspace, size_t workspace_bytes,
-                             void* stream) {
+                             void* stream, bool final_ln = true) {
   cudaStream_t st = (cudaStream_t)stream;
   const int D = m->embed_dim, H = m->num_heads, F = m->ffn_dim, N = m->num_layers;
   RNAMSM_REQUIRE(D == H * 64, "msa_forward: head_dim must be 64 (D=%d H=%d)", D, H);
@@ -717,6 +766,7 @@ static int msa_forward_entry(const rnamsm_model_weights* m, const int64_t* token
                             next.w ? &next : nullptr, f32_tensor, want_col ? &colp : nullptr)))
       return rc;
   }
+  if (!final_ln) return 0;   // the scoring entry normalises only the rows it reads (x stays pre-LayerNorm)
   // 16-bit path with logits wanted: the LM head's dense GEMM runs on the tensor cores, so it needs the final
   // LayerNorm's output in 16 bits as well -- written by a second (16-bit output) LayerNorm launch on the same rows
   // before the in-place fp32 one
@@ -726,25 +776,12 @@ static int msa_forward_entry(const rnamsm_model_weights* m, const int64_t* token
   // emb_layer_norm_after in place (model.py:396): fp32 -> fp32, each warp reads its row before writing it
   if ((rc = launch_layernorm(x, m->ln_after_w, m->ln_after_b, x, RNAMSM_F32, (long long)T, D, m->ln_eps, st))) return rc;
   if (logits_out) {
-    // RobertaLMHead (modules.py:313-319): dense -> erf-GELU -> LayerNorm -> tied projection + bias.
-    // 16-bit path: dense + GELU on tcgen05 (16-bit h), LayerNorm with fp32 statistics -> fp32, 12-wide tied projection in
-    // fp32.  fp32 path: FFMA throughout.  Scratch: the q|k|v|ctx region.
+    // LM head; scratch: the q|k|v|ctx region
     uint8_t* hbuf = ws + p.off_qkvh;
     float* h32 = reinterpret_cast<float*>(hbuf + align256(T * D * 4));
-    LinearEpilogue e{RNAMSM_EPI_BIAS_GELU, m->lm_dense_b, 1.f, 0, nullptr};
-    if (lm16) {
-      if ((rc = launch_linear_16(ws + p.off_xn, m->lm_dense_w16, (long long)T, D, D, dtype == RNAMSM_F16, e, hbuf, st))) return rc;
-      if ((rc = launch_layernorm((const float*)hbuf, m->lm_ln_w, m->lm_ln_b, h32, RNAMSM_F32, (long long)T, D, m->ln_eps, st, 0,
-                                 0, dtype)))
-        return rc;
-    } else {
-      if ((rc = linear_any(x, m->lm_dense_w, (long long)T, D, D, RNAMSM_F32, e, hbuf, st, nullptr,
-                           (dtype == RNAMSM_F32 && f32_tensor) ? ws + p.off_split : nullptr)))
-        return rc;
-      if ((rc = launch_layernorm((const float*)hbuf, m->lm_ln_w, m->lm_ln_b, h32, RNAMSM_F32, (long long)T, D, m->ln_eps, st)))
-        return rc;
-    }
-    if ((rc = launch_vocab_proj(h32, m->tok_emb, m->lm_bias, (long long)T, m->vocab, D, logits_out, st))) return rc;
+    if ((rc = lm_head_rows(m, x, ws + p.off_xn, (long long)T, dtype, lm16, hbuf, h32,
+                           (dtype == RNAMSM_F32 && f32_tensor) ? ws + p.off_split : nullptr, logits_out, st)))
+      return rc;
   }
   return 0;
 }
@@ -791,7 +828,7 @@ int rnamsm_msa_forward_batch(const rnamsm_model_weights* m, int n_msa, const int
                              const uint8_t* has_pad, int dtype, float* x, float* const* row_attn_out, void* workspace,
                              size_t workspace_bytes, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
-  const int D = m->embed_dim, H = m->num_heads, F = m->ffn_dim, N = m->num_layers;
+  const int D = m->embed_dim, H = m->num_heads, F = m->ffn_dim;
   RNAMSM_REQUIRE(D == H * 64, "msa_forward_batch: head_dim must be 64 (D=%d H=%d)", D, H);
   RNAMSM_REQUIRE(is16(dtype), "msa_forward_batch: 16-bit operand types only (dtype %d); the fp32 parity path runs one MSA per call",
                  dtype);
@@ -801,26 +838,151 @@ int rnamsm_msa_forward_batch(const rnamsm_model_weights* m, int n_msa, const int
   if ((rc = make_batch_plan(n_msa, R, C, D, H, F, dtype, &bp))) return rc;
   RNAMSM_REQUIRE(workspace_bytes >= bp.total, "msa_forward_batch: workspace %zu < required %zu", workspace_bytes, bp.total);
   RNAMSM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "msa_forward_batch: workspace must be 256 B aligned");
-  uint8_t* ws = (uint8_t*)workspace;
-  uint8_t* pad = ws + bp.off_pad;
-  bool any_pad = false;
-  long long off = 0;
-  for (int i = 0; i < n_msa; ++i) {
-    any_pad = any_pad || (has_pad && has_pad[i]);
-    if ((rc = launch_embed_ln(tokens + off, R[i], C[i], m->tok_emb, m->vocab, m->pos_emb, m->n_pos, m->row_pos,
-                              m->ln_before_w, m->ln_before_b, D, m->pad_idx, m->ln_eps, x + (size_t)off * D, pad + off, st)))
-      return rc;
-    off += (long long)R[i] * C[i];
-  }
-  for (int l = 0; l < N; ++l) {
-    NextLn next{nullptr, nullptr, dtype};
-    if (l + 1 < N)
-      next = NextLn{m->layers[l + 1].row.ln_w, m->layers[l + 1].row.ln_b, block_dtype(m->layers[l + 1].row.dtype, dtype)};
-    if ((rc = layer_forward_batch(&m->layers[l], D, H, F, m->ln_eps, x, n_msa, R, C, has_pad, any_pad, dtype, l,
-                                  row_attn_out, ws, bp, st, l > 0, next.w ? &next : nullptr)))
-      return rc;
-  }
+  if ((rc = msa_forward_batch_layers(m, n_msa, tokens, R, C, has_pad, dtype, x, row_attn_out, (uint8_t*)workspace, bp, st)))
+    return rc;
   return launch_layernorm(x, m->ln_after_w, m->ln_after_b, x, RNAMSM_F32, bp.T, D, m->ln_eps, st);
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// LM-head scoring of one alignment (rnamsm_msa_masked_marginals).  Entry k is the LM-head output at (row, cols[k]) of
+// the grid with that token masked (or of the grid itself, mask_idx < 0).  The entry runs ceil(n_cols / group) passes;
+// a pass builds its variant grids on the device, runs them through the layer stack, gathers the one pre-final-LayerNorm
+// row each grid is scored at, and runs the final LayerNorm and the LM head on those rows only.
+//   16-bit, R >= 2: the pass's grids go through the batch layer path together (token-local kernels once per pass,
+//                   attention per grid), exactly as rnamsm_msa_forward_batch runs them.
+//   fp32 / tf32 x 3, or R == 1: one forward per grid (msa_forward_entry without its final LayerNorm and head).
+// Every kernel a row meets is row-local or has fixed tiles independent of the row count, so the logits are bit-identical
+// to rnamsm_msa_forward's logits of the masked grid at that token.
+// Workspace for `group` grids of R x C tokens (every region 256 B aligned):
+//   tok   [g, T] int64           the pass's variant grids
+//   x     [g or 1, T, D] fp32    hidden states: the pass's g grids (batch route) or the current grid
+//   fwd                          the forward's own workspace: the batch plan of g grids, or the one-MSA plan + pad flags
+//   rows  [g, D] fp32            the gathered rows (normalised in place when the head runs in fp32)
+//   xn16  [g, D] 16-bit          the final LayerNorm's 16-bit output (16-bit dtypes)
+//   h     [g, D] <= 4 B          LM-head dense + GELU
+//   h32   [g, D] fp32            LM-head LayerNorm
+//   split                        tf32 x 3 operand halves of the dense GEMM (RNAMSM_F32_TENSOR)
+// The logits land in the caller's logprobs_out and become log-probabilities in place.
+// ---------------------------------------------------------------------------------------------
+namespace rnamsm {
+
+struct ScorePlan {
+  bool batch;
+  size_t fwd_bytes, off_tok, off_x, off_fwd, off_rows, off_xn16, off_h, off_h32, off_split, total;
+};
+
+static int make_score_plan(int R, int C, int D, int H, int F, int dtype, int group, ScorePlan* out) {
+  const bool f32_tensor = (dtype & RNAMSM_F32_TENSOR) != 0;
+  const int dt = dtype & 0xff;
+  RNAMSM_REQUIRE((dtype & ~(0xff | RNAMSM_F32_TENSOR)) == 0 && (dt == RNAMSM_F32 || (is16(dt) && !f32_tensor)),
+                 "score: unknown dtype %d", dtype);
+  RNAMSM_REQUIRE(R >= 1 && C >= 1 && D > 0 && H > 0 && F > 0 && group >= 1, "score: bad shape R=%d C=%d D=%d H=%d F=%d group=%d",
+                 R, C, D, H, F, group);
+  const size_t T = (size_t)R * C, g = (size_t)group;
+  ScorePlan s{};
+  s.batch = is16(dt) && R >= 2;
+  if (s.batch) {
+    std::vector<int> Rs(group, R), Cs(group, C);
+    BatchPlan bp;
+    int rc;
+    if ((rc = make_batch_plan(group, Rs.data(), Cs.data(), D, H, F, dt, &bp))) return rc;
+    s.fwd_bytes = bp.total;
+  } else {
+    s.fwd_bytes = make_plan(R, C, D, H, F, dt, f32_tensor).total + align256(T);
+  }
+  size_t o = 0;
+  s.off_tok = o;   o += align256(g * T * 8);
+  s.off_x = o;     o += align256((s.batch ? g : 1) * T * D * 4);
+  s.off_fwd = o;   o += align256(s.fwd_bytes);
+  s.off_rows = o;  o += align256(g * D * 4);
+  s.off_xn16 = o;  o += is16(dt) ? align256(g * D * 2) : 0;
+  s.off_h = o;     o += align256(g * D * 4);
+  s.off_h32 = o;   o += align256(g * D * 4);
+  s.off_split = o; o += (dt == RNAMSM_F32 && f32_tensor) ? tf32_scratch_bytes((long long)g, D, D) : 0;
+  s.total = o;
+  *out = s;
+  return 0;
+}
+
+}  // namespace rnamsm
+
+extern "C" {
+
+size_t rnamsm_score_workspace_bytes(int R, int C, int D, int H, int F, int dtype, int group) {
+  ScorePlan sp;
+  if (make_score_plan(R, C, D, H, F, dtype, group, &sp)) return 0;
+  return sp.total;
+}
+
+int rnamsm_msa_masked_marginals(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad,
+                                int dtype, int row, const int* cols, int n_cols, int mask_idx, int group,
+                                float* logits_out, float* logprobs_out, void* workspace, size_t workspace_bytes,
+                                void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  const int D = m->embed_dim, H = m->num_heads, F = m->ffn_dim, V = m->vocab;
+  RNAMSM_REQUIRE(D == H * 64, "masked_marginals: head_dim must be 64 (D=%d H=%d)", D, H);
+  ScorePlan sp;
+  int rc;
+  if ((rc = make_score_plan(R, C, D, H, F, dtype, group, &sp))) return rc;
+  RNAMSM_REQUIRE(row >= 0 && row < R, "masked_marginals: row %d outside the %d MSA rows", row, R);
+  RNAMSM_REQUIRE(n_cols >= 0 && (n_cols == 0 || (cols && logprobs_out)), "masked_marginals: cols and logprobs_out required");
+  RNAMSM_REQUIRE(workspace_bytes >= sp.total, "masked_marginals: workspace %zu < required %zu", workspace_bytes, sp.total);
+  RNAMSM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "masked_marginals: workspace must be 256 B aligned");
+  if (n_cols == 0) return 0;
+  const int dt = dtype & 0xff;
+  const bool f32_tensor = (dtype & RNAMSM_F32_TENSOR) != 0;
+  const long long T = (long long)R * C;
+  uint8_t* ws = (uint8_t*)workspace;
+  int64_t* grids = reinterpret_cast<int64_t*>(ws + sp.off_tok);
+  float* x = reinterpret_cast<float*>(ws + sp.off_x);
+  float* rows = reinterpret_cast<float*>(ws + sp.off_rows);
+  void* xn16 = ws + sp.off_xn16;
+  const bool lm16 = is16(dt) && m->lm_dense_w16 != nullptr;   // the head msa_forward_entry runs for this dtype
+  std::vector<int> Rs(group, R), Cs(group, C);
+  std::vector<uint8_t> pads(group, has_pad ? 1 : 0);
+  // n grids of the pass (back to back) through embedding + layer stack; x: their pre-final-LayerNorm hidden states
+  auto layers = [&](const int64_t* tok, int n) -> int {
+    if (!sp.batch)
+      return msa_forward_entry(m, tok, R, C, has_pad, dtype, x, nullptr, nullptr, nullptr, nullptr, nullptr,
+                               ws + sp.off_fwd, sp.fwd_bytes, st, false);
+    BatchPlan bp;
+    int r;
+    if ((r = make_batch_plan(n, Rs.data(), Cs.data(), D, H, F, dt, &bp))) return r;
+    return msa_forward_batch_layers(m, n, tok, Rs.data(), Cs.data(), pads.data(), dt, x, nullptr, ws + sp.off_fwd, bp, st);
+  };
+  if (mask_idx < 0 && (rc = layers(tokens, 1))) return rc;   // wt-marginals: one forward, every column read from it
+  for (int k0 = 0; k0 < n_cols; k0 += group) {
+    const int n = std::min(group, n_cols - k0);
+    const int* ck = cols + k0;
+    if (mask_idx < 0) {
+      if ((rc = launch_score_gather(x, 0, row, C, ck, n, D, rows, st))) return rc;
+    } else {
+      if ((rc = launch_score_variants(tokens, T, row, C, ck, n, mask_idx, m->pad_idx, grids, st))) return rc;
+      if (sp.batch) {
+        if ((rc = layers(grids, n))) return rc;
+        if ((rc = launch_score_gather(x, T, row, C, ck, n, D, rows, st))) return rc;
+      } else {
+        for (int i = 0; i < n; ++i) {
+          if ((rc = layers(grids + (size_t)i * T, 1))) return rc;
+          if ((rc = launch_score_gather(x, 0, row, C, ck + i, 1, D, rows + (size_t)i * D, st))) return rc;
+        }
+      }
+    }
+    // final LayerNorm on the n rows (the 16-bit operand of the tensor-core head, or fp32 in place), LM head, log_softmax
+    if ((rc = launch_layernorm(rows, m->ln_after_w, m->ln_after_b, lm16 ? xn16 : (void*)rows, lm16 ? dt : RNAMSM_F32, n, D,
+                               m->ln_eps, st)))
+      return rc;
+    float* lp = logprobs_out + (size_t)k0 * V;
+    if ((rc = lm_head_rows(m, rows, xn16, n, dt, lm16, ws + sp.off_h, reinterpret_cast<float*>(ws + sp.off_h32),
+                           (dt == RNAMSM_F32 && f32_tensor) ? ws + sp.off_split : nullptr, lp, st)))
+      return rc;
+    if ((rc = launch_score_log_softmax(lp, logits_out ? logits_out + (size_t)k0 * V : nullptr, n, V, tokens, row, C, ck,
+                                       m->pad_idx, st)))
+      return rc;
+  }
+  return 0;
 }
 
 }  // extern "C"

@@ -110,4 +110,14 @@ size_t col_probs_scratch_bytes(int R, int C, int H);
 int launch_col_probs(const void* qkv, int R, int C, int H, int dtype, int col_major, const uint8_t* pad, float* probs,
                      float* mean, void* scratch, cudaStream_t st);
 
+// score.cu -- LM-head scoring: n variant grids of T tokens with (row, cols[k]) masked; the pre-final-LayerNorm row
+// (row, cols[k]) of grid k (grids grid_stride tokens apart) into out [n, D]; log_softmax of lp [n, V] in place, with
+// the logits copied to logits_out (optional).  Invalid columns (out of range, pad) give NaN rows.
+int launch_score_variants(const int64_t* tokens, long long T, int row, int C, const int* cols, int n, int mask_idx,
+                          int pad_idx, int64_t* out, cudaStream_t st);
+int launch_score_gather(const float* x, long long grid_stride, int row, int C, const int* cols, int n, int D, float* out,
+                        cudaStream_t st);
+int launch_score_log_softmax(float* lp, float* logits_out, int n, int V, const int64_t* tokens, int row, int C,
+                             const int* cols, int pad_idx, cudaStream_t st);
+
 }  // namespace rnamsm

@@ -328,3 +328,117 @@ class MSATransformer(nn.Module, _PrecisionMixin):
                 o["row_attentions"] = maps[i]
             outs.append(o)
         return outs
+
+    # -- LM-head scoring ---------------------------------------------------------------------------
+    def _score_grid(self, tokens, row: int):
+        """[1, R, C] or [R, C] CUDA tokens -> (int64 [R, C] grid, has_pad, host pad flags of ``row``) after the input
+        limits of ``forward``.  One host sync."""
+        _infer_only(self)
+        t = tokens[0] if tokens.ndim == 3 and tokens.shape[0] == 1 else tokens
+        if t.ndim != 2:
+            raise ValueError(f"scoring takes one MSA, [1, R, C] or [R, C]; got shape {tuple(tokens.shape)}")
+        L.require_cuda(t, "tokens")
+        if t.device != self.device:
+            raise RuntimeError(f"tokens on {t.device} but model on {self.device}")
+        L.device_check(t.device)
+        t = t.long().contiguous()
+        R, Cc = t.shape
+        if not 0 <= row < R:
+            raise ValueError(f"row {row} outside the {R} MSA rows")
+        pad = t.eq(self.vocab.pad_idx)
+        host = torch.cat([(~pad).sum(-1), pad[row].long()]).cpu()     # non-pad count per row | pad flags of `row`
+        n_nonpad_max = int(host[:R].max())
+        self.check_msa_shape(R, Cc, n_nonpad_max)
+        return t, bool(int(host[:R].min()) < Cc), host[R:].bool().tolist()
+
+    def _marginals(self, t, has_pad, row_pad, positions, row, masked, token_budget, return_logits):
+        R, Cc = t.shape
+        start = int(self.vocab.prepend_bos)
+        if positions is None:
+            positions = [c for c in range(start, Cc) if not row_pad[c]]
+        positions = [int(c) for c in positions]
+        for c in positions:
+            if not 0 <= c < Cc:
+                raise ValueError(f"position {c} outside the {Cc} grid columns")
+            if row_pad[c]:
+                raise ValueError(f"position {c} is a padding token of row {row}")
+        P, V = len(positions), len(self.vocab)
+        dev = t.device
+        lp = torch.empty((P, V), dtype=torch.float32, device=dev)
+        logits = torch.empty((P, V), dtype=torch.float32, device=dev) if return_logits else None
+        if P:
+            group, _ = plan_score_group(R, Cc, P, token_budget)
+            D, H = self.embed_dim, self.num_attention_heads
+            cols = torch.tensor(positions, dtype=torch.int32).to(dev)
+            with torch.cuda.device(dev):
+                m = self.c_weights(self._code)
+                fcode = self._fwd_code
+                nbytes = L.lib.rnamsm_score_workspace_bytes(R, Cc, D, H, 4 * D, fcode, group)
+                if nbytes == 0:
+                    raise RuntimeError("rnamsm_score_workspace_bytes: " + L.lib.rnamsm_last_error().decode(errors="replace"))
+                ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+                L.check(L.lib.rnamsm_msa_masked_marginals(
+                    C.byref(m), L.ptr(t), R, Cc, int(has_pad), fcode, row, L.ptr(cols), P,
+                    self.vocab.mask_idx if masked else -1, group, L.ptr(logits), L.ptr(lp), L.ptr(ws), nbytes,
+                    L.stream_ptr()), "msa_masked_marginals")
+        return positions, lp, logits
+
+    @torch.no_grad()
+    def masked_marginals(self, tokens, positions: Optional[Iterable[int]] = None, row: int = 0, masked: bool = True,
+                         token_budget: int = 262144, return_logits: bool = False):
+        """LM-head log-probabilities of ``row`` under masking (``rnamsm_msa_masked_marginals``).
+
+        Row ``k`` of the result is ``log_softmax`` of the logits at ``(row, positions[k])`` of the grid with that token
+        replaced by ``<mask>``; ``masked=False`` reads every position from one forward of ``tokens`` itself
+        ("wt-marginals").  ``tokens``: ``[1, R, C]`` or ``[R, C]`` on the model's device.  ``positions``: grid columns;
+        by default every non-pad column of ``row`` except the BOS column 0.  The masked grids run ``group =
+        max(1, token_budget // (R * C))`` at a time (``plan_score_group``).  Returns fp32 ``[P, V]`` on the device, and
+        the logits ``[P, V]`` too with ``return_logits=True``; the logits are bit-identical to
+        ``forward(masked grid)["logits"][0, row, col]``.  One host sync per call."""
+        t, has_pad, row_pad = self._score_grid(tokens, row)
+        _, lp, logits = self._marginals(t, has_pad, row_pad, positions, row, masked, token_budget, return_logits)
+        return (lp, logits) if return_logits else lp
+
+    @torch.no_grad()
+    def pseudo_log_likelihood(self, tokens, row: int = 0, token_budget: int = 262144):
+        """-> ``(pll, per_position)``: ``per_position[i] = log p(wt_i | wt_i masked)`` (fp32, device) over the default
+        positions of ``masked_marginals`` (the non-pad residues of ``row``), ``pll`` their float64 sum.  The
+        pseudo-perplexity is ``exp(-pll / L)`` with ``L = len(per_position)``."""
+        t, has_pad, row_pad = self._score_grid(tokens, row)
+        positions, lp, _ = self._marginals(t, has_pad, row_pad, None, row, True, token_budget, False)
+        wt = t[row, positions].view(-1, 1)
+        per_position = lp.gather(1, wt).view(-1)
+        return float(per_position.double().sum()), per_position
+
+    @torch.no_grad()
+    def score_mutations(self, tokens, mutations, row: int = 0, method: str = "masked-marginals",
+                        token_budget: int = 262144) -> torch.Tensor:
+        """Zero-shot mutant scores: float64 ``[len(mutations)]`` on the CPU, mutant ``i`` scoring
+        ``sum over its substitutions of logp[pos, mt] - logp[pos, wt]``.  Mutants are strings such as ``"G12A"`` or
+        ``"G12A:C30U"`` (``rnamsm_b200.mutations``): 1-based residues of query ``row``, so residue ``k`` is grid column
+        ``k``.  ``method``: ``"masked-marginals"`` (logp at a position from the grid with that position masked) or
+        ``"wt-marginals"`` (all from one unmasked forward).  Marginals are computed once for the union of mutated
+        positions: one forward per distinct position, not per mutant.  ``ValueError`` on a malformed mutant, a wild
+        type that does not match the query, an index out of range or on a pad / BOS column, or a repeated position."""
+        from .mutations import parse_mutant
+        if method not in ("masked-marginals", "wt-marginals"):
+            raise ValueError(f"method {method!r}: expected 'masked-marginals' or 'wt-marginals'")
+        t, has_pad, row_pad = self._score_grid(tokens, row)
+        query = t[row].cpu().tolist()
+        parsed = [parse_mutant(s, query, self.vocab) for s in mutations]
+        positions = sorted({c for subs in parsed for c, _, _ in subs})
+        _, lp, _ = self._marginals(t, has_pad, row_pad, positions, row, method == "masked-marginals", token_budget, False)
+        lp = lp.cpu().double()
+        at = {c: i for i, c in enumerate(positions)}
+        scores = torch.zeros(len(parsed), dtype=torch.float64)
+        for i, subs in enumerate(parsed):
+            scores[i] = sum(float(lp[at[c], mt] - lp[at[c], wt]) for c, wt, mt in subs)
+        return scores
+
+
+def plan_score_group(R: int, C: int, n_positions: int, token_budget: int = 262144):
+    """-> ``(group, passes)`` of ``masked_marginals``: ``group = max(1, token_budget // (R * C))`` grids per pass (the
+    token budget of ``plan_batches``), at most ``n_positions``, and ``passes = ceil(n_positions / group)``; the last
+    pass may be partial."""
+    group = max(1, min(int(token_budget) // (R * C), n_positions))
+    return group, -(-n_positions // group)
