@@ -154,6 +154,7 @@ row_softmax_p2p_kernel(PeerPtrs partial, int n_ranks, int rank, int n_splits, in
       const int j = lane + 32 * t;
       if (j < ld_lp || j < C) emit(j, j < C ? vals[t] * inv : 0.f);
     }
+    for (int j = 32 * kMaxPerLane + lane; j < ld_lp; j += 32) emit(j, 0.f);   // (ld_lp may exceed 32 kMaxPerLane)
   } else {
     for (int j = lane; j < ld_lp || j < C; j += 32) emit(j, j < C ? __expf(logit(j) - mx) * inv : 0.f);
   }
