@@ -365,6 +365,26 @@ int rnamsm_msa_masked_marginals(const rnamsm_model_weights* m, const int64_t* to
                                 float* logits_out, float* logprobs_out, void* workspace, size_t workspace_bytes,
                                 void* stream);
 
+/* Sequences generated from one MSA by iterative masked sampling with the LM head.  n_chains chains start from
+ * `tokens` [R, C] (NULL: from the states already in tokens_out, to resume a run) and take steps start_step ..
+ * start_step + steps - 1.  Step s of chain k masks token (r, c) when r is in `rows`, c >= 1, the token is not <pad> and
+ * u_mask(seed, k, s, r, c) < mask_prob; runs the masked grid through the forward; runs the final LayerNorm and the LM
+ * head on the `rows` only; and replaces each masked token by a draw from softmax(logits / temperature) over the tokens
+ * of allowed_bitmask (bit v = vocabulary entry v; not <pad>, not <mask>, which is the last vocabulary entry) by inverse
+ * CDF with u_draw(seed, k, s, r, c); temperature 0 takes the argmax, ties to the lowest index.  The uniforms are
+ * Philox4x32-10 with key (seed low, seed high) and counter (k, s, r * C + c, 0 = mask | 1 = draw), u = (word0 >> 8) *
+ * 2^-24 (csrc/sample.cu), so a result depends on none of group, the call split of the steps or the GPU.  rows: DEVICE
+ * int32 [n_rows], ascending and distinct, in [0, R).  tokens_out: int64 [n_chains, R, C], the chains' final states.
+ * dtype: as rnamsm_msa_forward (RNAMSM_F32_TENSOR included).  16-bit with R >= 2: `group` chains per pass through the
+ * layer path of rnamsm_msa_forward_batch; otherwise one forward per grid.  Enqueues only: no synchronisation, no
+ * allocation.  workspace: rnamsm_sample_workspace_bytes(..., group, n_rows) bytes, 256 B aligned (0 = invalid
+ * arguments). */
+size_t rnamsm_sample_workspace_bytes(int R, int C, int D, int H, int F, int dtype, int group, int n_rows);
+int rnamsm_msa_gibbs_sample(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad, int dtype,
+                            const int* rows, int n_rows, int n_chains, int steps, int start_step, float mask_prob,
+                            float temperature, unsigned allowed_bitmask, unsigned long long seed, int group,
+                            int64_t* tokens_out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- one deep MSA sharded over the GPUs of a box (SURVEY.md 8e; rna-msm_b200/sharded.py) -----------
  * The reference has no multi-GPU forward; these entry points implement the partition its math allows:
  * rows for the tied row attention (sum of partial logits over ranks), columns for the column attention

@@ -103,6 +103,9 @@ SIGNATURES = {
     "rnamsm_score_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i]),
     "rnamsm_msa_masked_marginals": (_i, [C.POINTER(ModelWeights), _vp, _i, _i, _i, _i, _i, _vp, _i, _i, _i, _vp, _vp,
                                          _vp, _sz, _vp]),
+    "rnamsm_sample_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i, _i]),
+    "rnamsm_msa_gibbs_sample": (_i, [C.POINTER(ModelWeights), _vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, C.c_float,
+                                     C.c_float, C.c_uint, C.c_ulonglong, _i, _vp, _vp, _sz, _vp]),
     "rnamsm_rsa_pack": (_i, [_vp, _i, _i, _i, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]),
 }
 

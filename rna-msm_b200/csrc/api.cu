@@ -986,3 +986,148 @@ int rnamsm_msa_masked_marginals(const rnamsm_model_weights* m, const int64_t* to
 }
 
 }  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// Iterative masked sampling of one alignment with the LM head (rnamsm_msa_gibbs_sample; the algorithm and its random
+// numbers are in sample.cu).  Chains run `group` at a time; a pass loops over all steps of its chains, enqueuing only.
+// One step of a pass of g chains:
+//   copy the g states into the grid buffer, mask kernel -> the g masked grids
+//   layer stack: 16-bit with R >= 2, the g grids through the batch layer path together; fp32 / tf32 x 3 or R == 1, one
+//   msa_forward_entry per grid without its final LayerNorm (the routes of the scoring entry)
+//   row gather (only when n_rows < R) -> the sampled rows' pre-final-LayerNorm states
+//   final LayerNorm and LM head on those g * n_rows * C rows only, draw kernel -> the g states
+// Workspace for `group` grids of R x C tokens, M = group * n_rows * C head rows (every region 256 B aligned):
+//   tok   [g, T] int64           the pass's masked grids
+//   x     [g, T, D] fp32         hidden states of the pass's grids
+//   fwd                          the forward's own workspace: the batch plan of g grids, or the one-MSA plan + pad flags
+//   hx    [M, D] fp32            the gathered rows (n_rows < R only; otherwise the head reads x)
+//   xn16  [M, D] 16-bit          the final LayerNorm's 16-bit output (16-bit dtypes)
+//   h     [M, D] <= 4 B          LM-head dense + GELU, then the logits [M, V]
+//   h32   [M, D] fp32            LM-head LayerNorm
+//   split                        tf32 x 3 operand halves of the dense GEMM (RNAMSM_F32_TENSOR)
+// ---------------------------------------------------------------------------------------------
+namespace rnamsm {
+
+struct SamplePlan {
+  bool batch;
+  size_t fwd_bytes, off_tok, off_x, off_fwd, off_hx, off_xn16, off_h, off_h32, off_split, total;
+};
+
+static int make_sample_plan(int R, int C, int D, int H, int F, int dtype, int group, int n_rows, SamplePlan* out) {
+  const bool f32_tensor = (dtype & RNAMSM_F32_TENSOR) != 0;
+  const int dt = dtype & 0xff;
+  RNAMSM_REQUIRE((dtype & ~(0xff | RNAMSM_F32_TENSOR)) == 0 && (dt == RNAMSM_F32 || (is16(dt) && !f32_tensor)),
+                 "sample: unknown dtype %d", dtype);
+  RNAMSM_REQUIRE(R >= 1 && C >= 1 && D > 0 && H > 0 && F > 0 && group >= 1 && n_rows >= 1 && n_rows <= R,
+                 "sample: bad shape R=%d C=%d D=%d H=%d F=%d group=%d n_rows=%d", R, C, D, H, F, group, n_rows);
+  const size_t T = (size_t)R * C, g = (size_t)group, M = g * n_rows * C;
+  SamplePlan s{};
+  s.batch = is16(dt) && R >= 2;
+  if (s.batch) {
+    std::vector<int> Rs(group, R), Cs(group, C);
+    BatchPlan bp;
+    int rc;
+    if ((rc = make_batch_plan(group, Rs.data(), Cs.data(), D, H, F, dt, &bp))) return rc;
+    s.fwd_bytes = bp.total;
+  } else {
+    s.fwd_bytes = make_plan(R, C, D, H, F, dt, f32_tensor).total + align256(T);
+  }
+  size_t o = 0;
+  s.off_tok = o;   o += align256(g * T * 8);
+  s.off_x = o;     o += align256(g * T * D * 4);
+  s.off_fwd = o;   o += align256(s.fwd_bytes);
+  s.off_hx = o;    o += n_rows < R ? align256(M * D * 4) : 0;
+  s.off_xn16 = o;  o += is16(dt) ? align256(M * D * 2) : 0;
+  s.off_h = o;     o += align256(M * D * 4);
+  s.off_h32 = o;   o += align256(M * D * 4);
+  s.off_split = o; o += (dt == RNAMSM_F32 && f32_tensor) ? tf32_scratch_bytes((long long)M, D, D) : 0;
+  s.total = o;
+  *out = s;
+  return 0;
+}
+
+}  // namespace rnamsm
+
+extern "C" {
+
+size_t rnamsm_sample_workspace_bytes(int R, int C, int D, int H, int F, int dtype, int group, int n_rows) {
+  SamplePlan sp;
+  if (make_sample_plan(R, C, D, H, F, dtype, group, n_rows, &sp)) return 0;
+  return sp.total;
+}
+
+int rnamsm_msa_gibbs_sample(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad, int dtype,
+                            const int* rows, int n_rows, int n_chains, int steps, int start_step, float mask_prob,
+                            float temperature, unsigned allowed_bitmask, unsigned long long seed, int group,
+                            int64_t* tokens_out, void* workspace, size_t workspace_bytes, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  const int D = m->embed_dim, H = m->num_heads, F = m->ffn_dim, V = m->vocab;
+  const int mask_idx = V - 1;   // the RNA alphabet appends <mask> after its residues (msm/data.py)
+  RNAMSM_REQUIRE(D == H * 64, "gibbs_sample: head_dim must be 64 (D=%d H=%d)", D, H);
+  SamplePlan sp;
+  int rc;
+  if ((rc = make_sample_plan(R, C, D, H, F, dtype, group, n_rows, &sp))) return rc;
+  RNAMSM_REQUIRE(rows && tokens_out, "gibbs_sample: rows and tokens_out required");
+  RNAMSM_REQUIRE(n_chains >= 1 && steps >= 0 && start_step >= 0 && steps <= INT_MAX - start_step,
+                 "gibbs_sample: n_chains=%d steps=%d start_step=%d", n_chains, steps, start_step);
+  RNAMSM_REQUIRE(mask_prob >= 0.f && mask_prob <= 1.f, "gibbs_sample: mask_prob %g outside [0, 1]", (double)mask_prob);
+  RNAMSM_REQUIRE(temperature >= 0.f, "gibbs_sample: temperature %g < 0", (double)temperature);
+  RNAMSM_REQUIRE(V >= 2 && V <= 32 && V <= D, "gibbs_sample: vocabulary of %d tokens (2 .. 32, <= D)", V);
+  RNAMSM_REQUIRE(allowed_bitmask != 0 && (V == 32 || (allowed_bitmask >> V) == 0) &&
+                     !((allowed_bitmask >> m->pad_idx) & 1u) && !((allowed_bitmask >> mask_idx) & 1u),
+                 "gibbs_sample: allowed_bitmask 0x%x must be a non-empty set of vocabulary tokens other than <pad> and <mask>",
+                 allowed_bitmask);
+  RNAMSM_REQUIRE(workspace_bytes >= sp.total, "gibbs_sample: workspace %zu < required %zu", workspace_bytes, sp.total);
+  RNAMSM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "gibbs_sample: workspace must be 256 B aligned");
+  const int dt = dtype & 0xff;
+  const bool f32_tensor = (dtype & RNAMSM_F32_TENSOR) != 0;
+  const long long T = (long long)R * C;
+  if (tokens)
+    for (int k = 0; k < n_chains; ++k)
+      RNAMSM_CHECK_CUDA(cudaMemcpyAsync(tokens_out + (size_t)k * T, tokens, (size_t)T * 8, cudaMemcpyDeviceToDevice, st));
+  uint8_t* ws = (uint8_t*)workspace;
+  int64_t* grids = reinterpret_cast<int64_t*>(ws + sp.off_tok);
+  float* x = reinterpret_cast<float*>(ws + sp.off_x);
+  float* hx = n_rows < R ? reinterpret_cast<float*>(ws + sp.off_hx) : x;
+  void* xn16 = ws + sp.off_xn16;
+  uint8_t* h = ws + sp.off_h;
+  const bool lm16 = is16(dt) && m->lm_dense_w16 != nullptr;   // the head msa_forward_entry runs for this dtype
+  std::vector<int> Rs(group, R), Cs(group, C);
+  std::vector<uint8_t> pads(group, has_pad ? 1 : 0);
+  for (int k0 = 0; k0 < n_chains; k0 += group) {
+    const int n = std::min(group, n_chains - k0);
+    const long long M = (long long)n * n_rows * C;
+    BatchPlan bp;
+    if (sp.batch && (rc = make_batch_plan(n, Rs.data(), Cs.data(), D, H, F, dt, &bp))) return rc;
+    for (int s = start_step; s < start_step + steps; ++s) {
+      RNAMSM_CHECK_CUDA(cudaMemcpyAsync(grids, tokens_out + (size_t)k0 * T, (size_t)n * T * 8, cudaMemcpyDeviceToDevice, st));
+      if ((rc = launch_sample_mask(tokens_out, grids, n, R, C, rows, n_rows, m->pad_idx, mask_idx, mask_prob, seed, k0, s, st)))
+        return rc;
+      if (sp.batch) {
+        if ((rc = msa_forward_batch_layers(m, n, grids, Rs.data(), Cs.data(), pads.data(), dt, x, nullptr, ws + sp.off_fwd,
+                                           bp, st)))
+          return rc;
+      } else {
+        for (int i = 0; i < n; ++i)
+          if ((rc = msa_forward_entry(m, grids + (size_t)i * T, R, C, has_pad, dtype, x + (size_t)i * T * D, nullptr, nullptr,
+                                      nullptr, nullptr, nullptr, ws + sp.off_fwd, sp.fwd_bytes, st, false)))
+            return rc;
+      }
+      if (n_rows < R && (rc = launch_sample_gather_rows(x, n, R, C, rows, n_rows, D, hx, st))) return rc;
+      // final LayerNorm on the M head rows (the 16-bit operand of the tensor-core head, or fp32 in place), LM head, draw
+      if ((rc = launch_layernorm(hx, m->ln_after_w, m->ln_after_b, lm16 ? xn16 : (void*)hx, lm16 ? dt : RNAMSM_F32, M, D,
+                                 m->ln_eps, st)))
+        return rc;
+      float* logits = reinterpret_cast<float*>(h);   // h is free again once the head's LayerNorm has read it
+      if ((rc = lm_head_rows(m, hx, xn16, M, dt, lm16, h, reinterpret_cast<float*>(ws + sp.off_h32),
+                             (dt == RNAMSM_F32 && f32_tensor) ? ws + sp.off_split : nullptr, logits, st)))
+        return rc;
+      if ((rc = launch_sample_draw(logits, V, temperature, allowed_bitmask, tokens_out, n, R, C, rows, n_rows, m->pad_idx,
+                                   mask_prob, seed, k0, s, st)))
+        return rc;
+    }
+  }
+  return 0;
+}
+
+}  // extern "C"

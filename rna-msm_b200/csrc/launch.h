@@ -120,4 +120,16 @@ int launch_score_gather(const float* x, long long grid_stride, int row, int C, c
 int launch_score_log_softmax(float* lp, float* logits_out, int n, int V, const int64_t* tokens, int row, int C,
                              const int* cols, int pad_idx, cudaStream_t st);
 
+// sample.cu -- iterative masked sampling: a pass of n chains (k0 .. k0 + n - 1, states [n_chains, R, C]) over the
+// sampled rows rows[0 .. n_rows).  mask: grids [n, R, C] (a copy of the pass's states) get mask_idx at this step's
+// masked tokens; gather_rows: the sampled rows of x [n, R, C, D] into out [n, n_rows, C, D]; draw: each masked token
+// drawn from logits [n, n_rows, C, V] into its chain's state.
+int launch_sample_mask(const int64_t* states, int64_t* grids, int n, int R, int C, const int* rows, int n_rows, int pad_idx,
+                       int mask_idx, float p, unsigned long long seed, int k0, int step, cudaStream_t st);
+int launch_sample_gather_rows(const float* x, int n, int R, int C, const int* rows, int n_rows, int D, float* out,
+                              cudaStream_t st);
+int launch_sample_draw(const float* logits, int V, float temperature, unsigned allowed, int64_t* states, int n, int R, int C,
+                       const int* rows, int n_rows, int pad_idx, float p, unsigned long long seed, int k0, int step,
+                       cudaStream_t st);
+
 }  // namespace rnamsm

@@ -435,10 +435,101 @@ class MSATransformer(nn.Module, _PrecisionMixin):
             scores[i] = sum(float(lp[at[c], mt] - lp[at[c], wt]) for c, wt, mt in subs)
         return scores
 
+    # -- generation with the LM head ---------------------------------------------------------------
+    @torch.no_grad()
+    def sample_msa(self, tokens, steps: int, mask_prob: float = 0.1, temperature: float = 1.0,
+                   rows: Optional[Iterable[int]] = None, n_chains: int = 1, seed: int = 0, start_step: int = 0,
+                   allowed: str = "AGCU-", token_budget: int = 262144) -> torch.Tensor:
+        """New sequences from one alignment by iterative masked sampling (``rnamsm_msa_gibbs_sample``).
+
+        Each of ``n_chains`` chains starts from ``tokens`` and takes steps ``start_step .. start_step + steps - 1``.  A
+        step masks every non-pad token of ``rows`` (default: all rows) outside the BOS column with probability
+        ``mask_prob``, runs the model on the masked grid and replaces each masked token by a draw from
+        ``softmax(logits / temperature)`` over the ``allowed`` tokens (``temperature=0``: the argmax).  The random
+        numbers are a stateless function of ``(seed, chain, step, row, column)`` (DESIGN.md §4.11), so the result does
+        not depend on ``token_budget`` and ``steps=a+b`` equals ``steps=a`` followed by ``steps=b, start_step=a`` on its
+        output.  ``tokens``: ``[R, C]`` or ``[1, R, C]`` (every chain starts there) or ``[n_chains, R, C]`` (chain ``k``
+        starts from ``tokens[k]``; the grids share one pad layout) on the model's device.  Chains run
+        ``plan_score_group(R, C, n_chains, token_budget)[0]`` at a time.  Returns int64 ``[n_chains, R, C]`` on the
+        device; the steps are enqueued without a host sync."""
+        if not 0.0 <= mask_prob <= 1.0:
+            raise ValueError(f"mask_prob {mask_prob} outside [0, 1]")
+        if not temperature >= 0.0:
+            raise ValueError(f"temperature {temperature} must be >= 0")
+        if steps < 0 or start_step < 0:
+            raise ValueError(f"steps {steps} and start_step {start_step} must be >= 0")
+        if n_chains < 1:
+            raise ValueError(f"n_chains {n_chains} must be >= 1")
+        if not 0 <= seed < 1 << 64:
+            raise ValueError(f"seed {seed} outside [0, 2**64)")
+        bitmask = self._allowed_bitmask(allowed)
+        R = tokens.shape[-2]
+        rows = list(range(R)) if rows is None else sorted({int(r) for r in rows})
+        if not rows:
+            raise ValueError("rows is empty")
+        if rows[0] < 0 or rows[-1] >= R:
+            raise ValueError(f"rows {rows[0]} .. {rows[-1]} outside the {R} MSA rows")
+        t, has_pad = self._sample_grid(tokens, n_chains)
+        Cc = t.shape[2]
+        dev = t.device
+        out = torch.empty((n_chains, R, Cc), dtype=torch.int64, device=dev)
+        if t.shape[0] > 1:
+            out.copy_(t)
+        group, _ = plan_score_group(R, Cc, n_chains, token_budget)
+        D, H = self.embed_dim, self.num_attention_heads
+        rows_d = torch.tensor(rows, dtype=torch.int32).to(dev)
+        with torch.cuda.device(dev):
+            m = self.c_weights(self._code)
+            fcode = self._fwd_code
+            nbytes = L.lib.rnamsm_sample_workspace_bytes(R, Cc, D, H, 4 * D, fcode, group, len(rows))
+            if nbytes == 0:
+                raise RuntimeError("rnamsm_sample_workspace_bytes: " + L.lib.rnamsm_last_error().decode(errors="replace"))
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            L.check(L.lib.rnamsm_msa_gibbs_sample(
+                C.byref(m), L.ptr(t[0]) if t.shape[0] == 1 else None, R, Cc, int(has_pad), fcode, L.ptr(rows_d),
+                len(rows), n_chains, steps, start_step, mask_prob, temperature, bitmask, seed, group, L.ptr(out),
+                L.ptr(ws), nbytes, L.stream_ptr()), "msa_gibbs_sample")
+        return out
+
+    def _allowed_bitmask(self, allowed) -> int:
+        """``allowed`` (a string of residue / gap letters such as ``"AGCU-"``, or an iterable of them) -> the bit set
+        of their vocabulary indices.  ``ValueError`` when empty or when an entry is not one of ``A G C U X N -``."""
+        from .alphabet import RNA_TOKS
+        letters = list(allowed)
+        if not letters:
+            raise ValueError("allowed is empty")
+        bits = 0
+        for a in letters:
+            if a not in RNA_TOKS:
+                raise ValueError(f"allowed token {a!r} is not a residue or gap ({' '.join(RNA_TOKS)})")
+            bits |= 1 << self.vocab.tokens_to_idx[a]
+        return bits
+
+    def _sample_grid(self, tokens, n_chains: int):
+        """[R, C], [1, R, C] or [n_chains, R, C] CUDA tokens -> (int64 [1 or n_chains, R, C], has_pad) after the input
+        limits of ``forward``.  One host sync."""
+        _infer_only(self)
+        t = tokens.unsqueeze(0) if tokens.ndim == 2 else tokens
+        if t.ndim != 3 or t.shape[0] not in (1, n_chains):
+            raise ValueError(f"sampling takes one MSA, [R, C], [1, R, C] or [n_chains={n_chains}, R, C]; "
+                             f"got shape {tuple(tokens.shape)}")
+        L.require_cuda(t, "tokens")
+        if t.device != self.device:
+            raise RuntimeError(f"tokens on {t.device} but model on {self.device}")
+        L.device_check(t.device)
+        t = t.long().contiguous()
+        R, Cc = t.shape[1:]
+        pad = t.eq(self.vocab.pad_idx)
+        host = torch.cat([(~pad[0]).sum(-1), (pad != pad[:1]).any().view(1).long()]).cpu()   # non-pad counts | layouts differ
+        if int(host[R]):
+            raise ValueError("the chains' starting grids must share one pad layout")
+        self.check_msa_shape(R, Cc, int(host[:R].max()))
+        return t, bool(int(host[:R].min()) < Cc)
+
 
 def plan_score_group(R: int, C: int, n_positions: int, token_budget: int = 262144):
-    """-> ``(group, passes)`` of ``masked_marginals``: ``group = max(1, token_budget // (R * C))`` grids per pass (the
-    token budget of ``plan_batches``), at most ``n_positions``, and ``passes = ceil(n_positions / group)``; the last
-    pass may be partial."""
+    """-> ``(group, passes)`` of ``masked_marginals`` (and of ``sample_msa``, with its chains as the positions):
+    ``group = max(1, token_budget // (R * C))`` grids per pass (the token budget of ``plan_batches``), at most
+    ``n_positions``, and ``passes = ceil(n_positions / group)``; the last pass may be partial."""
     group = max(1, min(int(token_budget) // (R * C), n_positions))
     return group, -(-n_positions // group)
