@@ -402,7 +402,7 @@ int rnamsm_ipc_close(void* p);
 /* LayerNorm of this rank's row shard x [Rn*C, D] (rows r0..r0+Rn of an R-row MSA) whose 16-bit output
  * rows go straight into the column owners' buffers: token (r, c) -> peer_dst[c / (C/n)], row
  * (c % (C/n)) * R + r, i.e. each peer ends with its column shard in [C/n, R, D] (column-major) order.
- * Replaces LayerNorm + the row->column all-to-all. */
+ * Replaces LayerNorm + the row->column all-to-all.  0 <= r0 and r0 + Rn <= R. */
 int rnamsm_layernorm_push(const float* x, const float* w, const float* b, void* const* peer_dst, int n_ranks, int Rn,
                           int C, int R, int r0, int D, float eps, int y_dtype, void* stream);
 
@@ -410,7 +410,8 @@ int rnamsm_layernorm_push(const float* x, const float* w, const float* b, void* 
  * those rows of every rank's partial logits (peer_partial[g]: fp32 [n_splits, H, C, C]), sums them,
  * applies logit_scale / key mask / softmax, writes the fp32 map rows it owns into map_out (THIS rank's
  * [H, C, C] map slab of the layer, or NULL; rows of other owners are left untouched) and the 16-bit
- * probabilities into every rank's peer_probs[g] [H, C, ld_lp].  Replaces all-reduce + rnamsm_row_softmax. */
+ * probabilities into every rank's peer_probs[g] [H, C, ld_lp] (columns >= C zero-filled).  Replaces all-reduce +
+ * rnamsm_row_softmax. */
 int rnamsm_row_softmax_p2p(void* const* peer_partial, int n_ranks, int rank, int n_splits, int H, int C,
                            const uint8_t* key_pad, float logit_scale, float* map_out, void* const* peer_probs,
                            int ld_lp, int dtype, void* stream);
@@ -439,7 +440,7 @@ int rnamsm_host_unregister(void* p);
  *                   (GEMM + exchange + residual add in one kernel; 4 bytes per element over NVLink);
  *   as_delta16 = 1: peer_x are 16-bit receive buffers, the epilogue TMA-stores the result (2 bytes per
  *                   element); the owner adds it with rnamsm_add_layernorm on its next LayerNorm pass.
- * Cn % 16 == 0. */
+ * Cn % 16 == 0.  The shard is one of the n_ranks shards of C: c0 >= 0, c0 % Cn == 0, c0 + Cn <= C, c0 / Cn < n_ranks. */
 int rnamsm_linear_residual_scatter(const void* ctx, const void* W, const float* bias, int R, int Cn, int N, int K,
                                    int dtype, void* const* peer_x, int n_ranks, int Rn, int C, int c0, int as_delta16,
                                    void* stream);

@@ -241,6 +241,9 @@ row_softmax_p2p_vec_kernel(PeerPtrs partial, int n_ranks, int rank, int n_splits
         *reinterpret_cast<uint2*>(reinterpret_cast<uint16_t*>(probs.p[(rank + t) % n_ranks]) + lp_off + j) = make_uint2(0u, 0u);
     }
   }
+  for (int j = 512 * kP2pT + 4 * tid; j < ld_lp; j += 512)            // padding past column 512 kP2pT (C = 4096 < ld_lp)
+    for (int t = 0; t < n_ranks; ++t)
+      *reinterpret_cast<uint2*>(reinterpret_cast<uint16_t*>(probs.p[(rank + t) % n_ranks]) + lp_off + j) = make_uint2(0u, 0u);
 }
 
 
@@ -314,6 +317,7 @@ int rnamsm_layernorm_push(const float* x, const float* w, const float* b, void* 
   RNAMSM_REQUIRE(n_ranks >= 1 && n_ranks <= RNAMSM_MAX_PEERS, "layernorm_push: %d ranks (max %d)", n_ranks, RNAMSM_MAX_PEERS);
   RNAMSM_REQUIRE(C % n_ranks == 0 && D % 128 == 0 && D <= 1024, "layernorm_push: C=%d must divide by %d ranks; D=%d", C, n_ranks, D);
   RNAMSM_REQUIRE(y_dtype == RNAMSM_BF16 || y_dtype == RNAMSM_F16, "layernorm_push: 16-bit output only");
+  RNAMSM_REQUIRE(Rn >= 0 && r0 >= 0 && r0 + Rn <= R, "layernorm_push: rows [%d, %d + %d) outside the R=%d rows of the MSA", r0, r0, Rn, R);
   PeerPtrs dst{};
   for (int g = 0; g < n_ranks; ++g) dst.p[g] = peer_dst[g];
   const long long n_rows = (long long)Rn * C;

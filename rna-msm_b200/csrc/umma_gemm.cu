@@ -822,6 +822,9 @@ int launch_linear_16_scatter(const void* x, const void* W, const float* bias, in
   RNAMSM_REQUIRE(N % 64 == 0 && K % BLOCK_K == 0 && K >= BLOCK_K, "linear_scatter: N=%d and K=%d must be multiples of 64", N, K);
   RNAMSM_REQUIRE(n_ranks >= 1 && n_ranks <= RNAMSM_MAX_PEERS && Rn * n_ranks == R, "linear_scatter: R=%d != %d ranks x Rn=%d", R, n_ranks, Rn);
   RNAMSM_REQUIRE(Cn % 16 == 0, "linear_scatter: columns per rank Cn=%d must be a multiple of 16 (TMA box rows)", Cn);
+  // the shard is the (c0 / Cn)-th of n_ranks inside the owners' C columns (m_tile_shift relies on c0 / Cn < n_ranks)
+  RNAMSM_REQUIRE(Cn > 0 && c0 >= 0 && c0 % Cn == 0 && c0 + Cn <= C && c0 / Cn < n_ranks,
+                 "linear_scatter: column shard [%d, %d + %d) is not one of %d shards of C=%d", c0, c0, Cn, n_ranks, C);
   const int in_dt = fp16 ? TMAP_F16 : TMAP_BF16;
   const int box_rows = Cn % 32 == 0 ? 32 : 16;
   CUtensorMap ta, tb;
