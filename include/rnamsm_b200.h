@@ -385,6 +385,35 @@ int rnamsm_msa_gibbs_sample(const rnamsm_model_weights* m, const int64_t* tokens
                             float temperature, unsigned allowed_bitmask, unsigned long long seed, int group,
                             int64_t* tokens_out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Categorical Jacobian of the LM head for one query row (Zhang et al., PNAS 2024): how the logits of every listed
+ * residue move when one residue is substituted.  With G(i, a) = `tokens` [R, C] with token (row, positions[i]) replaced
+ * by alphabet[a], and f(G)[j, b] the LM-head logit of G at (row, positions[j]) for token alphabet[b]:
+ *   jacobian_out[i, a, j, b] = f(G(i, a))[j, b] - f(tokens)[j, b]        fp32 [P, A, P, A]
+ * Only the slabs listed in `entries` run (one forward each, plus one of `tokens`); every other slab is exactly 0 --
+ * callers list every (i, a) whose alphabet[a] differs from the wild type at positions[i].  positions: HOST int32 [P],
+ * grid columns; alphabet: HOST int32 [A], vocabulary indices; entries: HOST int32 [n_entries], the slabs i * A + a,
+ * strictly ascending.  They are staged into the workspace with one cudaMemcpyAsync.  dtype: as rnamsm_msa_forward
+ * (RNAMSM_F32_TENSOR included).  16-bit with R >= 2: `group` grids per pass through the layer path of
+ * rnamsm_msa_forward_batch; otherwise one forward per grid.  Only the query row of each grid goes through the final
+ * LayerNorm and the LM head, so each slab is bit-identical to the difference of rnamsm_msa_forward's logits.  Enqueues
+ * only: no synchronisation, no allocation.  workspace: rnamsm_jacobian_workspace_bytes(..., group, P, A, n_entries)
+ * bytes, 256 B aligned (0 = invalid arguments). */
+size_t rnamsm_jacobian_workspace_bytes(int R, int C, int D, int H, int F, int dtype, int group, int P, int A,
+                                       int n_entries);
+int rnamsm_msa_categorical_jacobian(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad,
+                                    int dtype, int row, const int* positions, int P, const int* alphabet, int A,
+                                    const int* entries, int n_entries, int group, float* jacobian_out, void* workspace,
+                                    size_t workspace_bytes, void* stream);
+
+/* Contact map [P, P] fp32 from a categorical Jacobian J [P, A, P, A] (csrc/jacobian.cu): centre J over each of its four
+ * axes in turn (i, a, j, b), F[i, j] = Frobenius norm of the centred A x A block (i, j) with F[i, i] = 0, average
+ * product correction F - rowsum colsum^T / total (0 when total == 0) with the diagonal zeroed again, and
+ * (F + F^T) / 2.  Fixed-order float64 reductions, no atomics: bitwise reproducible.  scratch:
+ * rnamsm_jacobian_contacts_scratch_bytes(P, A) bytes, 256 B aligned (8 (P A)^2 + 8 P^2 + small). */
+size_t rnamsm_jacobian_contacts_scratch_bytes(int P, int A);
+int rnamsm_jacobian_contacts(const float* J, int P, int A, float* contacts_out, void* scratch, size_t scratch_bytes,
+                             void* stream);
+
 /* ---- one deep MSA sharded over the GPUs of a box (SURVEY.md 8e; rna-msm_b200/sharded.py) -----------
  * The reference has no multi-GPU forward; these entry points implement the partition its math allows:
  * rows for the tied row attention (sum of partial logits over ranks), columns for the column attention

@@ -6,7 +6,7 @@ the CUDA library and raises if it is missing -- there is no CPU or PyTorch fallb
 """
 from . import _lib  # noqa: F401  (loads librnamsm_b200.so, fails loudly when absent)
 from .alphabet import Alphabet, Vocab, read_msa, tokenize_msa  # noqa: F401
-from .model import MSATransformer, plan_score_group  # noqa: F401
+from .model import MSATransformer, jacobian_entries, plan_score_group  # noqa: F401
 from .mutations import parse_mutant  # noqa: F401
 from .modules import (AxialTransformerLayer, ColumnSelfAttention, ContactPredictionHead,  # noqa: F401
                       FeedForwardNetwork, LearnedPositionalEmbedding, NormalizedResidualBlock, RobertaLMHead,
@@ -19,4 +19,5 @@ __all__ = ["MSATransformer", "AxialTransformerLayer", "RowSelfAttention", "Colum
            "FeedForwardNetwork", "NormalizedResidualBlock", "LearnedPositionalEmbedding", "RobertaLMHead",
            "ContactPredictionHead", "Alphabet", "Vocab", "read_msa", "tokenize_msa", "extract_features",
            "run_inference", "ingest_msa", "pack_ss_input", "extract_features_streamed", "extract_features_batch",
-           "extract_features_batch_streamed", "pack_rsa_input", "plan_batches", "plan_score_group", "parse_mutant"]
+           "extract_features_batch_streamed", "pack_rsa_input", "plan_batches", "plan_score_group", "parse_mutant",
+           "jacobian_entries"]

@@ -106,6 +106,11 @@ SIGNATURES = {
     "rnamsm_sample_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i, _i]),
     "rnamsm_msa_gibbs_sample": (_i, [C.POINTER(ModelWeights), _vp, _i, _i, _i, _i, _vp, _i, _i, _i, _i, C.c_float,
                                      C.c_float, C.c_uint, C.c_ulonglong, _i, _vp, _vp, _sz, _vp]),
+    "rnamsm_jacobian_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i, _i, _i, _i]),
+    "rnamsm_msa_categorical_jacobian": (_i, [C.POINTER(ModelWeights), _vp, _i, _i, _i, _i, _i, C.POINTER(_i), _i,
+                                             C.POINTER(_i), _i, C.POINTER(_i), _i, _i, _vp, _vp, _sz, _vp]),
+    "rnamsm_jacobian_contacts_scratch_bytes": (_sz, [_i, _i]),
+    "rnamsm_jacobian_contacts": (_i, [_vp, _i, _i, _vp, _vp, _sz, _vp]),
     "rnamsm_rsa_pack": (_i, [_vp, _i, _i, _i, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]),
 }
 

@@ -868,6 +868,31 @@ int rnamsm_msa_forward_batch(const rnamsm_model_weights* m, int n_msa, const int
 // ---------------------------------------------------------------------------------------------
 namespace rnamsm {
 
+// The layer route of the LM-head entries (scoring, sampling, the categorical Jacobian): n grids of R x C tokens, back to
+// back in tok, through the embedding and the layer stack without the final LayerNorm; x [n, T, D] receives their
+// pre-final-LayerNorm hidden states.
+//   batch (16-bit, R >= 2): the n grids together through the batch layer path; fwd holds its plan for n grids.
+//   otherwise: one msa_forward_entry per grid; fwd holds the one-MSA plan + pad flags (fwd_bytes).
+static int grids_forward_layers(const rnamsm_model_weights* m, const int64_t* tok, int n, int R, int C, int has_pad,
+                                int dtype, bool batch, float* x, uint8_t* fwd, size_t fwd_bytes, cudaStream_t st) {
+  const int D = m->embed_dim;
+  const size_t T = (size_t)R * C;
+  int rc;
+  if (!batch) {
+    for (int i = 0; i < n; ++i)
+      if ((rc = msa_forward_entry(m, tok + i * T, R, C, has_pad, dtype, x + i * T * D, nullptr, nullptr, nullptr, nullptr,
+                                  nullptr, fwd, fwd_bytes, st, false)))
+        return rc;
+    return 0;
+  }
+  const int dt = dtype & 0xff;
+  std::vector<int> Rs(n, R), Cs(n, C);
+  std::vector<uint8_t> pads(n, has_pad ? 1 : 0);
+  BatchPlan bp;
+  if ((rc = make_batch_plan(n, Rs.data(), Cs.data(), D, m->num_heads, m->ffn_dim, dt, &bp))) return rc;
+  return msa_forward_batch_layers(m, n, tok, Rs.data(), Cs.data(), pads.data(), dt, x, nullptr, fwd, bp, st);
+}
+
 struct ScorePlan {
   bool batch;
   size_t fwd_bytes, off_tok, off_x, off_fwd, off_rows, off_xn16, off_h, off_h32, off_split, total;
@@ -940,17 +965,9 @@ int rnamsm_msa_masked_marginals(const rnamsm_model_weights* m, const int64_t* to
   float* rows = reinterpret_cast<float*>(ws + sp.off_rows);
   void* xn16 = ws + sp.off_xn16;
   const bool lm16 = is16(dt) && m->lm_dense_w16 != nullptr;   // the head msa_forward_entry runs for this dtype
-  std::vector<int> Rs(group, R), Cs(group, C);
-  std::vector<uint8_t> pads(group, has_pad ? 1 : 0);
-  // n grids of the pass (back to back) through embedding + layer stack; x: their pre-final-LayerNorm hidden states
+  // x holds one grid on the per-grid route, so that route runs the grids of a pass one call at a time
   auto layers = [&](const int64_t* tok, int n) -> int {
-    if (!sp.batch)
-      return msa_forward_entry(m, tok, R, C, has_pad, dtype, x, nullptr, nullptr, nullptr, nullptr, nullptr,
-                               ws + sp.off_fwd, sp.fwd_bytes, st, false);
-    BatchPlan bp;
-    int r;
-    if ((r = make_batch_plan(n, Rs.data(), Cs.data(), D, H, F, dt, &bp))) return r;
-    return msa_forward_batch_layers(m, n, tok, Rs.data(), Cs.data(), pads.data(), dt, x, nullptr, ws + sp.off_fwd, bp, st);
+    return grids_forward_layers(m, tok, n, R, C, has_pad, dtype, sp.batch, x, ws + sp.off_fwd, sp.fwd_bytes, st);
   };
   if (mask_idx < 0 && (rc = layers(tokens, 1))) return rc;   // wt-marginals: one forward, every column read from it
   for (int k0 = 0; k0 < n_cols; k0 += group) {
@@ -959,7 +976,7 @@ int rnamsm_msa_masked_marginals(const rnamsm_model_weights* m, const int64_t* to
     if (mask_idx < 0) {
       if ((rc = launch_score_gather(x, 0, row, C, ck, n, D, rows, st))) return rc;
     } else {
-      if ((rc = launch_score_variants(tokens, T, row, C, ck, n, mask_idx, m->pad_idx, grids, st))) return rc;
+      if ((rc = launch_score_variants(tokens, T, row, C, ck, nullptr, n, mask_idx, m->pad_idx, grids, st))) return rc;
       if (sp.batch) {
         if ((rc = layers(grids, n))) return rc;
         if ((rc = launch_score_gather(x, T, row, C, ck, n, D, rows, st))) return rc;
@@ -1092,27 +1109,15 @@ int rnamsm_msa_gibbs_sample(const rnamsm_model_weights* m, const int64_t* tokens
   void* xn16 = ws + sp.off_xn16;
   uint8_t* h = ws + sp.off_h;
   const bool lm16 = is16(dt) && m->lm_dense_w16 != nullptr;   // the head msa_forward_entry runs for this dtype
-  std::vector<int> Rs(group, R), Cs(group, C);
-  std::vector<uint8_t> pads(group, has_pad ? 1 : 0);
   for (int k0 = 0; k0 < n_chains; k0 += group) {
     const int n = std::min(group, n_chains - k0);
     const long long M = (long long)n * n_rows * C;
-    BatchPlan bp;
-    if (sp.batch && (rc = make_batch_plan(n, Rs.data(), Cs.data(), D, H, F, dt, &bp))) return rc;
     for (int s = start_step; s < start_step + steps; ++s) {
       RNAMSM_CHECK_CUDA(cudaMemcpyAsync(grids, tokens_out + (size_t)k0 * T, (size_t)n * T * 8, cudaMemcpyDeviceToDevice, st));
       if ((rc = launch_sample_mask(tokens_out, grids, n, R, C, rows, n_rows, m->pad_idx, mask_idx, mask_prob, seed, k0, s, st)))
         return rc;
-      if (sp.batch) {
-        if ((rc = msa_forward_batch_layers(m, n, grids, Rs.data(), Cs.data(), pads.data(), dt, x, nullptr, ws + sp.off_fwd,
-                                           bp, st)))
-          return rc;
-      } else {
-        for (int i = 0; i < n; ++i)
-          if ((rc = msa_forward_entry(m, grids + (size_t)i * T, R, C, has_pad, dtype, x + (size_t)i * T * D, nullptr, nullptr,
-                                      nullptr, nullptr, nullptr, ws + sp.off_fwd, sp.fwd_bytes, st, false)))
-            return rc;
-      }
+      if ((rc = grids_forward_layers(m, grids, n, R, C, has_pad, dtype, sp.batch, x, ws + sp.off_fwd, sp.fwd_bytes, st)))
+        return rc;
       if (n_rows < R && (rc = launch_sample_gather_rows(x, n, R, C, rows, n_rows, D, hx, st))) return rc;
       // final LayerNorm on the M head rows (the 16-bit operand of the tensor-core head, or fp32 in place), LM head, draw
       if ((rc = launch_layernorm(hx, m->ln_after_w, m->ln_after_b, lm16 ? xn16 : (void*)hx, lm16 ? dt : RNAMSM_F32, M, D,
@@ -1126,6 +1131,144 @@ int rnamsm_msa_gibbs_sample(const rnamsm_model_weights* m, const int64_t* tokens
                                    mask_prob, seed, k0, s, st)))
         return rc;
     }
+  }
+  return 0;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// Categorical Jacobian of the LM head for one query row (rnamsm_msa_categorical_jacobian; the definition and the
+// contact map are in jacobian.cu).  Entry e names slab s = i * A + a of J: the grid with token (row, positions[i])
+// replaced by alphabet[a].  J is zeroed first, so every slab no entry names (the wild type's) is exactly 0.  One forward
+// of `tokens` gives the wild-type logits of the query row; the entries then run `group` grids per pass:
+//   variant kernel (score.cu, with per-entry tokens) -> the pass's substituted grids
+//   layer stack on the route of the scoring and sampling entries (grids_forward_layers)
+//   row gather (R >= 2 only) -> the query row of each grid, M = g * C head rows
+//   final LayerNorm and LM head on those rows, collect kernel -> f - f_wt into the entries' slabs
+// Workspace: the sampling plan of `group` grids with one sampled row (tok / x / fwd / hx / xn16 / h / h32 / split for
+// M = g * C head rows; the pass's logits [M, V] land in h), then
+//   wt    [C, V <= D] fp32               the wild-type logits of the query row (sized [C, D])
+//   list  int32 [1 + P + A + 3 n]        row | positions | alphabet | per entry: column, token, slab
+// ---------------------------------------------------------------------------------------------
+namespace rnamsm {
+
+struct JacobianPlan {
+  SamplePlan sp;
+  size_t off_wt, off_list, total;
+};
+
+static int make_jacobian_plan(int R, int C, int D, int H, int F, int dtype, int group, int P, int A, int n_entries,
+                              JacobianPlan* out) {
+  RNAMSM_REQUIRE(P >= 1 && A >= 1 && n_entries >= 0, "jacobian: P=%d A=%d n_entries=%d", P, A, n_entries);
+  JacobianPlan j{};
+  int rc;
+  if ((rc = make_sample_plan(R, C, D, H, F, dtype, group, 1, &j.sp))) return rc;
+  size_t o = j.sp.total;
+  j.off_wt = o;   o += align256((size_t)C * D * 4);
+  j.off_list = o; o += align256((1 + (size_t)P + A + 3 * (size_t)n_entries) * 4);
+  j.total = o;
+  *out = j;
+  return 0;
+}
+
+}  // namespace rnamsm
+
+extern "C" {
+
+size_t rnamsm_jacobian_workspace_bytes(int R, int C, int D, int H, int F, int dtype, int group, int P, int A,
+                                       int n_entries) {
+  JacobianPlan jp;
+  if (make_jacobian_plan(R, C, D, H, F, dtype, group, P, A, n_entries, &jp)) return 0;
+  return jp.total;
+}
+
+int rnamsm_msa_categorical_jacobian(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad,
+                                    int dtype, int row, const int* positions, int P, const int* alphabet, int A,
+                                    const int* entries, int n_entries, int group, float* jacobian_out, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  const int D = m->embed_dim, H = m->num_heads, F = m->ffn_dim, V = m->vocab;
+  RNAMSM_REQUIRE(D == H * 64, "categorical_jacobian: head_dim must be 64 (D=%d H=%d)", D, H);
+  JacobianPlan jp;
+  int rc;
+  if ((rc = make_jacobian_plan(R, C, D, H, F, dtype, group, P, A, n_entries, &jp))) return rc;
+  RNAMSM_REQUIRE(V >= 1 && V <= D, "categorical_jacobian: vocabulary of %d tokens (<= D=%d)", V, D);
+  RNAMSM_REQUIRE(row >= 0 && row < R, "categorical_jacobian: row %d outside the %d MSA rows", row, R);
+  RNAMSM_REQUIRE(tokens && positions && alphabet && jacobian_out && (n_entries == 0 || entries),
+                 "categorical_jacobian: tokens, positions, alphabet, entries and jacobian_out required");
+  RNAMSM_REQUIRE(workspace_bytes >= jp.total, "categorical_jacobian: workspace %zu < required %zu", workspace_bytes, jp.total);
+  RNAMSM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "categorical_jacobian: workspace must be 256 B aligned");
+  // the host list, checked here and staged into the workspace with one copy
+  std::vector<int> list(1 + (size_t)P + A + 3 * (size_t)n_entries);
+  int* l_pos = list.data() + 1;
+  int* l_alph = l_pos + P;
+  int* l_col = l_alph + A;
+  int* l_tok = l_col + n_entries;
+  int* l_slab = l_tok + n_entries;
+  list[0] = row;
+  for (int i = 0; i < P; ++i) {
+    RNAMSM_REQUIRE(positions[i] >= 0 && positions[i] < C, "categorical_jacobian: position %d outside the %d columns",
+                   positions[i], C);
+    l_pos[i] = positions[i];
+  }
+  for (int a = 0; a < A; ++a) {
+    RNAMSM_REQUIRE(alphabet[a] >= 0 && alphabet[a] < V, "categorical_jacobian: token %d outside the vocabulary of %d",
+                   alphabet[a], V);
+    l_alph[a] = alphabet[a];
+  }
+  for (int e = 0; e < n_entries; ++e) {
+    const int s = entries[e];
+    RNAMSM_REQUIRE(s >= 0 && s < P * A && (e == 0 || s > entries[e - 1]),
+                   "categorical_jacobian: entry %d (slab %d) must be ascending in [0, P*A = %d)", e, s, P * A);
+    l_col[e] = positions[s / A];
+    l_tok[e] = alphabet[s % A];
+    l_slab[e] = s;
+  }
+  const int dt = dtype & 0xff;
+  const bool f32_tensor = (dtype & RNAMSM_F32_TENSOR) != 0;
+  const long long T = (long long)R * C;
+  const SamplePlan& sp = jp.sp;
+  uint8_t* ws = (uint8_t*)workspace;
+  int64_t* grids = reinterpret_cast<int64_t*>(ws + sp.off_tok);
+  float* x = reinterpret_cast<float*>(ws + sp.off_x);
+  float* hx = R > 1 ? reinterpret_cast<float*>(ws + sp.off_hx) : x;
+  void* xn16 = ws + sp.off_xn16;
+  uint8_t* h = ws + sp.off_h;
+  float* wt = reinterpret_cast<float*>(ws + jp.off_wt);
+  int* d_list = reinterpret_cast<int*>(ws + jp.off_list);
+  const int* d_pos = d_list + 1;
+  const int* d_alph = d_pos + P;
+  const int* d_col = d_alph + A;
+  const int* d_tok = d_col + n_entries;
+  const int* d_slab = d_tok + n_entries;
+  const bool lm16 = is16(dt) && m->lm_dense_w16 != nullptr;   // the head msa_forward_entry runs for this dtype
+  RNAMSM_CHECK_CUDA(cudaMemcpyAsync(d_list, list.data(), list.size() * 4, cudaMemcpyHostToDevice, st));
+  RNAMSM_CHECK_CUDA(cudaMemsetAsync(jacobian_out, 0, (size_t)P * A * P * A * 4, st));
+  if (n_entries == 0) return 0;
+  // the query row of the n grids in x -> final LayerNorm (the 16-bit operand of the tensor-core head, or fp32 in place)
+  // -> LM head -> logits [n * C, V]
+  auto head = [&](int n, float* logits) -> int {
+    const long long M = (long long)n * C;
+    int r;
+    if (R > 1 && (r = launch_sample_gather_rows(x, n, R, C, d_list, 1, D, hx, st))) return r;
+    if ((r = launch_layernorm(hx, m->ln_after_w, m->ln_after_b, lm16 ? xn16 : (void*)hx, lm16 ? dt : RNAMSM_F32, M, D,
+                              m->ln_eps, st)))
+      return r;
+    return lm_head_rows(m, hx, xn16, M, dt, lm16, h, reinterpret_cast<float*>(ws + sp.off_h32),
+                        (dt == RNAMSM_F32 && f32_tensor) ? ws + sp.off_split : nullptr, logits, st);
+  };
+  if ((rc = grids_forward_layers(m, tokens, 1, R, C, has_pad, dtype, sp.batch, x, ws + sp.off_fwd, sp.fwd_bytes, st)))
+    return rc;
+  if ((rc = head(1, wt))) return rc;
+  float* logits = reinterpret_cast<float*>(h);   // h is free again once the head's LayerNorm has read it
+  for (int k0 = 0; k0 < n_entries; k0 += group) {
+    const int n = std::min(group, n_entries - k0);
+    if ((rc = launch_score_variants(tokens, T, row, C, d_col + k0, d_tok + k0, n, 0, m->pad_idx, grids, st))) return rc;
+    if ((rc = grids_forward_layers(m, grids, n, R, C, has_pad, dtype, sp.batch, x, ws + sp.off_fwd, sp.fwd_bytes, st)))
+      return rc;
+    if ((rc = head(n, logits))) return rc;
+    if ((rc = launch_jacobian_collect(logits, wt, n, C, V, d_pos, P, d_alph, A, d_slab + k0, jacobian_out, st))) return rc;
   }
   return 0;
 }

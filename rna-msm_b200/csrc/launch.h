@@ -110,11 +110,12 @@ size_t col_probs_scratch_bytes(int R, int C, int H);
 int launch_col_probs(const void* qkv, int R, int C, int H, int dtype, int col_major, const uint8_t* pad, float* probs,
                      float* mean, void* scratch, cudaStream_t st);
 
-// score.cu -- LM-head scoring: n variant grids of T tokens with (row, cols[k]) masked; the pre-final-LayerNorm row
+// score.cu -- LM-head scoring: n variant grids of T tokens with (row, cols[k]) masked (set to toks[k] when toks is not
+// NULL: the substituted grids of the categorical Jacobian); the pre-final-LayerNorm row
 // (row, cols[k]) of grid k (grids grid_stride tokens apart) into out [n, D]; log_softmax of lp [n, V] in place, with
 // the logits copied to logits_out (optional).  Invalid columns (out of range, pad) give NaN rows.
-int launch_score_variants(const int64_t* tokens, long long T, int row, int C, const int* cols, int n, int mask_idx,
-                          int pad_idx, int64_t* out, cudaStream_t st);
+int launch_score_variants(const int64_t* tokens, long long T, int row, int C, const int* cols, const int* toks, int n,
+                          int mask_idx, int pad_idx, int64_t* out, cudaStream_t st);
 int launch_score_gather(const float* x, long long grid_stride, int row, int C, const int* cols, int n, int D, float* out,
                         cudaStream_t st);
 int launch_score_log_softmax(float* lp, float* logits_out, int n, int V, const int64_t* tokens, int row, int C,
@@ -131,5 +132,10 @@ int launch_sample_gather_rows(const float* x, int n, int R, int C, const int* ro
 int launch_sample_draw(const float* logits, int V, float temperature, unsigned allowed, int64_t* states, int n, int R, int C,
                        const int* rows, int n_rows, int pad_idx, float p, unsigned long long seed, int k0, int step,
                        cudaStream_t st);
+
+// jacobian.cu -- categorical Jacobian: J[slabs[k], j, b] = logits[k * C + positions[j], alphabet[b]] -
+// wt[positions[j], alphabet[b]] for the n grids of a pass (logits [n * C, V], wt [C, V]; J [P, A, P, A]).
+int launch_jacobian_collect(const float* logits, const float* wt, int n, int C, int V, const int* positions, int P,
+                            const int* alphabet, int A, const int* slabs, float* J, cudaStream_t st);
 
 }  // namespace rnamsm

@@ -4,7 +4,8 @@
 //
 // Entry k of a pass is grid k with token (row, cols[k]) masked.  An entry whose column is out of range or names a pad
 // token of the row is left unmasked, gathers zeros and comes back as a row of NaN; nothing is read or written out of
-// bounds for it.
+// bounds for it.  The variant kernel also builds the substituted grids of the categorical Jacobian (jacobian.cu): there
+// token (row, cols[k]) becomes toks[k] instead of the mask token.
 #include "common.cuh"
 #include "launch.h"
 
@@ -14,17 +15,17 @@ __device__ __forceinline__ bool score_col_ok(const int64_t* __restrict__ tokens,
   return col >= 0 && col < C && tokens[(long long)row * C + col] != pad_idx;
 }
 
-// out[k * T + t] = tokens[t], except (row, cols[k]) -> mask_idx
+// out[k * T + t] = tokens[t], except (row, cols[k]) -> toks[k], or mask_idx when toks is NULL
 __global__ void __launch_bounds__(256)
-score_variants_kernel(const int64_t* __restrict__ tokens, long long T, int row, int C, const int* __restrict__ cols, int n,
-                      int mask_idx, int pad_idx, int64_t* __restrict__ out) {
+score_variants_kernel(const int64_t* __restrict__ tokens, long long T, int row, int C, const int* __restrict__ cols,
+                      const int* __restrict__ toks, int n, int mask_idx, int pad_idx, int64_t* __restrict__ out) {
   const long long total = (long long)n * T;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int k = (int)(i / T);
     const long long t = i - (long long)k * T;
     const int c = cols[k];
     const bool hit = t == (long long)row * C + c && score_col_ok(tokens, row, C, c, pad_idx);
-    out[i] = hit ? (int64_t)mask_idx : tokens[t];
+    out[i] = hit ? (int64_t)(toks ? toks[k] : mask_idx) : tokens[t];
   }
 }
 
@@ -59,12 +60,12 @@ score_log_softmax_kernel(float* __restrict__ lp, float* __restrict__ logits_out,
   }
 }
 
-int launch_score_variants(const int64_t* tokens, long long T, int row, int C, const int* cols, int n, int mask_idx,
-                          int pad_idx, int64_t* out, cudaStream_t st) {
+int launch_score_variants(const int64_t* tokens, long long T, int row, int C, const int* cols, const int* toks, int n,
+                          int mask_idx, int pad_idx, int64_t* out, cudaStream_t st) {
   RNAMSM_REQUIRE(n > 0 && T > 0, "score_variants: empty pass (n=%d T=%lld)", n, T);
   const long long total = (long long)n * T;
   const int blocks = (int)std::min<long long>((total + 255) / 256, 148LL * 16);
-  score_variants_kernel<<<blocks, 256, 0, st>>>(tokens, T, row, C, cols, n, mask_idx, pad_idx, out);
+  score_variants_kernel<<<blocks, 256, 0, st>>>(tokens, T, row, C, cols, toks, n, mask_idx, pad_idx, out);
   count_launch();
   RNAMSM_CHECK_CUDA(cudaGetLastError());
   return 0;

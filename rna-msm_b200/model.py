@@ -12,7 +12,7 @@ of scope (SURVEY.md section 2.1).
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Iterable, Optional
+from typing import Dict, Iterable, List, Optional, Sequence
 
 import torch
 import torch.nn as nn
@@ -331,8 +331,8 @@ class MSATransformer(nn.Module, _PrecisionMixin):
 
     # -- LM-head scoring ---------------------------------------------------------------------------
     def _score_grid(self, tokens, row: int):
-        """[1, R, C] or [R, C] CUDA tokens -> (int64 [R, C] grid, has_pad, host pad flags of ``row``) after the input
-        limits of ``forward``.  One host sync."""
+        """[1, R, C] or [R, C] CUDA tokens -> (int64 [R, C] grid, has_pad, host pad flags of ``row``, host tokens of
+        ``row``) after the input limits of ``forward``.  One host sync."""
         _infer_only(self)
         t = tokens[0] if tokens.ndim == 3 and tokens.shape[0] == 1 else tokens
         if t.ndim != 2:
@@ -346,10 +346,10 @@ class MSATransformer(nn.Module, _PrecisionMixin):
         if not 0 <= row < R:
             raise ValueError(f"row {row} outside the {R} MSA rows")
         pad = t.eq(self.vocab.pad_idx)
-        host = torch.cat([(~pad).sum(-1), pad[row].long()]).cpu()     # non-pad count per row | pad flags of `row`
+        host = torch.cat([(~pad).sum(-1), pad[row].long(), t[row]]).cpu()   # non-pad count per row | pad flags | tokens of `row`
         n_nonpad_max = int(host[:R].max())
         self.check_msa_shape(R, Cc, n_nonpad_max)
-        return t, bool(int(host[:R].min()) < Cc), host[R:].bool().tolist()
+        return t, bool(int(host[:R].min()) < Cc), host[R:R + Cc].bool().tolist(), host[R + Cc:].tolist()
 
     def _marginals(self, t, has_pad, row_pad, positions, row, masked, token_budget, return_logits):
         R, Cc = t.shape
@@ -395,7 +395,7 @@ class MSATransformer(nn.Module, _PrecisionMixin):
         max(1, token_budget // (R * C))`` at a time (``plan_score_group``).  Returns fp32 ``[P, V]`` on the device, and
         the logits ``[P, V]`` too with ``return_logits=True``; the logits are bit-identical to
         ``forward(masked grid)["logits"][0, row, col]``.  One host sync per call."""
-        t, has_pad, row_pad = self._score_grid(tokens, row)
+        t, has_pad, row_pad, _ = self._score_grid(tokens, row)
         _, lp, logits = self._marginals(t, has_pad, row_pad, positions, row, masked, token_budget, return_logits)
         return (lp, logits) if return_logits else lp
 
@@ -404,7 +404,7 @@ class MSATransformer(nn.Module, _PrecisionMixin):
         """-> ``(pll, per_position)``: ``per_position[i] = log p(wt_i | wt_i masked)`` (fp32, device) over the default
         positions of ``masked_marginals`` (the non-pad residues of ``row``), ``pll`` their float64 sum.  The
         pseudo-perplexity is ``exp(-pll / L)`` with ``L = len(per_position)``."""
-        t, has_pad, row_pad = self._score_grid(tokens, row)
+        t, has_pad, row_pad, _ = self._score_grid(tokens, row)
         positions, lp, _ = self._marginals(t, has_pad, row_pad, None, row, True, token_budget, False)
         wt = t[row, positions].view(-1, 1)
         per_position = lp.gather(1, wt).view(-1)
@@ -423,8 +423,7 @@ class MSATransformer(nn.Module, _PrecisionMixin):
         from .mutations import parse_mutant
         if method not in ("masked-marginals", "wt-marginals"):
             raise ValueError(f"method {method!r}: expected 'masked-marginals' or 'wt-marginals'")
-        t, has_pad, row_pad = self._score_grid(tokens, row)
-        query = t[row].cpu().tolist()
+        t, has_pad, row_pad, query = self._score_grid(tokens, row)
         parsed = [parse_mutant(s, query, self.vocab) for s in mutations]
         positions = sorted({c for subs in parsed for c, _, _ in subs})
         _, lp, _ = self._marginals(t, has_pad, row_pad, positions, row, method == "masked-marginals", token_budget, False)
@@ -434,6 +433,86 @@ class MSATransformer(nn.Module, _PrecisionMixin):
         for i, subs in enumerate(parsed):
             scores[i] = sum(float(lp[at[c], mt] - lp[at[c], wt]) for c, wt, mt in subs)
         return scores
+
+    # -- categorical Jacobian of the LM head ------------------------------------------------------------
+    @torch.no_grad()
+    def categorical_jacobian(self, tokens, row: int = 0, positions: Optional[Iterable[int]] = None,
+                             alphabet: str = "AGCU", token_budget: int = 262144, return_jacobian: bool = False):
+        """Contacts of query ``row`` read from the LM head alone (Zhang et al., PNAS 2024), with no contact regression
+        (``rnamsm_msa_categorical_jacobian``, ``rnamsm_jacobian_contacts``).
+
+        ``J[i, a, j, b] = f(G(i, a))[j, b] - f(tokens)[j, b]``, fp32 ``[P, A, P, A]``: ``G(i, a)`` is ``tokens`` with
+        ``(row, positions[i])`` replaced by ``alphabet[a]``, ``f(G)[j, b]`` the LM-head logit of ``G`` at
+        ``(row, positions[j])`` for ``alphabet[b]``.  A substitution by the wild type is not run and its slab is exactly
+        0, so a call runs ``sum_i (A - [wt_i in alphabet]) + 1`` forwards: ``3P + 1`` for ``"AGCU"`` over a gap-free
+        query, in passes of ``plan_score_group(R, C, n_substitutions, token_budget)[0]`` grids.  The cost grows as
+        ``P`` forwards of the whole ``R x C`` alignment: about ``3C`` forwards, so ~106 at 512 x 36 and ~766 at
+        512 x 256.  Each slab is bit-identical to the difference of ``forward(G(i, a))["logits"]`` and
+        ``forward(tokens)["logits"]`` at those entries.
+
+        Contacts ``[P, P]`` fp32: ``J`` centred over each of its axes in turn (i, a, j, b), the Frobenius norm of each
+        ``A x A`` block with a zero diagonal, average product correction, then ``(F + F^T) / 2``.
+
+        ``tokens``: ``[1, R, C]`` or ``[R, C]`` on the model's device.  ``positions``: grid columns of ``row``; by
+        default every non-pad column except the BOS column 0.  ``alphabet``: distinct letters of ``A G C U X N -``.
+        Returns the contacts on the device, and ``(contacts, J)`` with ``return_jacobian=True``.  One host sync.
+        ``ValueError`` on a bad alphabet, a row or position out of range, a position on a pad token or on the BOS
+        column, or fewer than two positions."""
+        alph = self._alphabet_indices(alphabet)
+        t, has_pad, row_pad, query = self._score_grid(tokens, row)
+        R, Cc = t.shape
+        start = int(self.vocab.prepend_bos)
+        if positions is None:
+            positions = [c for c in range(start, Cc) if not row_pad[c]]
+        positions = [int(c) for c in positions]
+        for c in positions:
+            if not 0 <= c < Cc:
+                raise ValueError(f"position {c} outside the {Cc} grid columns")
+            if c < start:
+                raise ValueError(f"position {c} is the BOS column")
+            if row_pad[c]:
+                raise ValueError(f"position {c} is a padding token of row {row}")
+        P, A = len(positions), len(alph)
+        if P < 2:
+            raise ValueError(f"a Jacobian needs at least two positions, got {P}")
+        entries = jacobian_entries([query[c] for c in positions], alph)
+        n = len(entries)
+        dev = t.device
+        J = torch.empty((P, A, P, A), dtype=torch.float32, device=dev)
+        contacts = torch.empty((P, P), dtype=torch.float32, device=dev)
+        group, _ = plan_score_group(R, Cc, max(n, 1), token_budget)
+        D, H = self.embed_dim, self.num_attention_heads
+        IntP = lambda v: (C.c_int * len(v))(*v)
+        with torch.cuda.device(dev):
+            m = self.c_weights(self._code)
+            fcode = self._fwd_code
+            nbytes = L.lib.rnamsm_jacobian_workspace_bytes(R, Cc, D, H, 4 * D, fcode, group, P, A, n)
+            if nbytes == 0:
+                raise RuntimeError("rnamsm_jacobian_workspace_bytes: " + L.lib.rnamsm_last_error().decode(errors="replace"))
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            st = L.stream_ptr()
+            L.check(L.lib.rnamsm_msa_categorical_jacobian(
+                C.byref(m), L.ptr(t), R, Cc, int(has_pad), fcode, row, IntP(positions), P, IntP(alph), A,
+                IntP(entries), n, group, L.ptr(J), L.ptr(ws), nbytes, st), "msa_categorical_jacobian")
+            del ws
+            sbytes = L.lib.rnamsm_jacobian_contacts_scratch_bytes(P, A)
+            scratch = torch.empty(sbytes, dtype=torch.uint8, device=dev)
+            L.check(L.lib.rnamsm_jacobian_contacts(L.ptr(J), P, A, L.ptr(contacts), L.ptr(scratch), sbytes, st),
+                    "jacobian_contacts")
+        return (contacts, J) if return_jacobian else contacts
+
+    def _alphabet_indices(self, alphabet) -> List[int]:
+        """``alphabet`` (a string of distinct letters of ``A G C U X N -``) -> their vocabulary indices, in order."""
+        from .alphabet import RNA_TOKS
+        letters = list(alphabet)
+        if not letters:
+            raise ValueError("alphabet is empty")
+        for a in letters:
+            if a not in RNA_TOKS:
+                raise ValueError(f"alphabet letter {a!r} is not a residue or gap ({' '.join(RNA_TOKS)})")
+        if len(set(letters)) != len(letters):
+            raise ValueError(f"alphabet {alphabet!r} repeats a letter")
+        return [self.vocab.tokens_to_idx[a] for a in letters]
 
     # -- generation with the LM head ---------------------------------------------------------------
     @torch.no_grad()
@@ -533,3 +612,11 @@ def plan_score_group(R: int, C: int, n_positions: int, token_budget: int = 26214
     ``n_positions``, and ``passes = ceil(n_positions / group)``; the last pass may be partial."""
     group = max(1, min(int(token_budget) // (R * C), n_positions))
     return group, -(-n_positions // group)
+
+
+def jacobian_entries(wild_type: Sequence[int], alphabet: Sequence[int]) -> List[int]:
+    """The substitutions ``categorical_jacobian`` runs, as slabs ``i * A + a`` of ``J`` in ascending order: every
+    ``(i, a)`` with ``alphabet[a] != wild_type[i]`` (token indices).  A wild type outside the alphabet (``N``, ``X``,
+    ``-``) gets all ``A`` substitutions."""
+    A = len(alphabet)
+    return [i * A + a for i, w in enumerate(wild_type) for a, v in enumerate(alphabet) if v != w]
