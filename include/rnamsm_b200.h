@@ -414,6 +414,35 @@ size_t rnamsm_jacobian_contacts_scratch_bytes(int P, int A);
 int rnamsm_jacobian_contacts(const float* J, int P, int A, float* contacts_out, void* scratch, size_t scratch_bytes,
                              void* stream);
 
+/* Full-length features of an alignment longer than the learned column positions, from overlapping windows
+ * (csrc/windows.cu).  tokens [R, C] with BOS at column 0, L = C - 1 residues, no EOS.  W = min(window, L); window k
+ * starts at residue s_k = min(k * stride, L - W), k < K = 1 + ceil((L - W) / stride), and is the grid [R, W + 1] of
+ * column 0 and columns 1 + s_k .. W + s_k, run as an MSA of its own.
+ * rnamsm_window_starts: the one implementation of that plan.  Returns K and writes s_0 .. s_{K-1} to HOST starts_out
+ * (when not NULL); 0 for invalid arguments (L < 1, or not 1 <= stride <= window), with the reason in rnamsm_last_error.
+ * rnamsm_msa_forward_windows: each window's row 0 of the final representation and its N*H row-attention maps (and, with
+ * contacts_out, its contact-head map with regression weights contact_w [N*H] and contact_b [1] or NULL), BOS stripped,
+ * stitched with tent weights w_k(p) = min(p - s_k + 1, s_k + W - p):
+ *   emb_out [L, D]          emb[p] = sum_k c_k(p) emb_k[p - s_k],  c_k(p) = w_k(p) / sum_k' w_k'(p)
+ *   atp_out [N*H, L, L]     atp[h, i, j] = sum_k c_k(i, j) map_k[h, i - s_k, j - s_k] over the windows holding i and j,
+ *                           c_k(i, j) = w_k(i) w_k(j) / sum_k' w_k'(i) w_k'(j); exactly 0 where no window holds both
+ *   contacts_out [L, L]     as atp, or NULL
+ * Coefficients: float64 quotients of the integer sums rounded once to fp32; fp32 sums acc = fmaf(c_k, v_k, acc) from 0 in
+ * ascending k, so the outputs do not depend on `group`, and an entry one window covers is that window's value bit for
+ * bit.  Every output element is written (no clearing needed).  window <= n_pos - pad_idx - 2 (the learned positions).
+ * dtype: as rnamsm_msa_forward (RNAMSM_F32_TENSOR included); the windows run `group` per pass on the route of
+ * rnamsm_msa_masked_marginals (16-bit with R >= 2: the batch layer path; otherwise one forward per grid).  has_pad: the
+ * input holds pad tokens (a window without any gives the same bits either way).  Enqueues only: no synchronisation, no
+ * allocation.  workspace: rnamsm_windows_workspace_bytes(R, C, D, H, F, N layers, dtype, group, window, stride,
+ * contacts wanted) bytes, 256 B aligned (0 = invalid arguments). */
+int rnamsm_window_starts(int L, int window, int stride, int* starts_out);
+size_t rnamsm_windows_workspace_bytes(int R, int C, int D, int H, int F, int N, int dtype, int group, int window, int stride,
+                                      int want_contacts);
+int rnamsm_msa_forward_windows(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad, int dtype,
+                               int window, int stride, int group, float* emb_out, float* atp_out, float* contacts_out,
+                               const float* contact_w, const float* contact_b, void* workspace, size_t workspace_bytes,
+                               void* stream);
+
 /* ---- one deep MSA sharded over the GPUs of a box (SURVEY.md 8e; rna-msm_b200/sharded.py) -----------
  * The reference has no multi-GPU forward; these entry points implement the partition its math allows:
  * rows for the tied row attention (sum of partial logits over ranks), columns for the column attention

@@ -12,7 +12,8 @@ from .modules import (AxialTransformerLayer, ColumnSelfAttention, ContactPredict
                       FeedForwardNetwork, LearnedPositionalEmbedding, NormalizedResidualBlock, RobertaLMHead,
                       RowSelfAttention)
 from .inference import (extract_features, extract_features_batch, extract_features_batch_streamed,  # noqa: F401
-                        extract_features_streamed, pack_rsa_input, pack_ss_input, plan_batches, run_inference)
+                        extract_features_streamed, extract_features_windowed, pack_rsa_input, pack_ss_input,
+                        plan_batches, run_inference)
 from .ingest import ingest_msa  # noqa: F401
 
 __all__ = ["MSATransformer", "AxialTransformerLayer", "RowSelfAttention", "ColumnSelfAttention",
@@ -20,4 +21,4 @@ __all__ = ["MSATransformer", "AxialTransformerLayer", "RowSelfAttention", "Colum
            "ContactPredictionHead", "Alphabet", "Vocab", "read_msa", "tokenize_msa", "extract_features",
            "run_inference", "ingest_msa", "pack_ss_input", "extract_features_streamed", "extract_features_batch",
            "extract_features_batch_streamed", "pack_rsa_input", "plan_batches", "plan_score_group", "parse_mutant",
-           "jacobian_entries"]
+           "jacobian_entries", "extract_features_windowed"]

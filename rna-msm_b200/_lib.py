@@ -111,6 +111,10 @@ SIGNATURES = {
                                              C.POINTER(_i), _i, C.POINTER(_i), _i, _i, _vp, _vp, _sz, _vp]),
     "rnamsm_jacobian_contacts_scratch_bytes": (_sz, [_i, _i]),
     "rnamsm_jacobian_contacts": (_i, [_vp, _i, _i, _vp, _vp, _sz, _vp]),
+    "rnamsm_window_starts": (_i, [_i, _i, _i, C.POINTER(_i)]),
+    "rnamsm_windows_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i]),
+    "rnamsm_msa_forward_windows": (_i, [C.POINTER(ModelWeights), _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp,
+                                        _vp, _sz, _vp]),
     "rnamsm_rsa_pack": (_i, [_vp, _i, _i, _i, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]),
 }
 

@@ -37,7 +37,8 @@ static std::vector<ProfEvent> g_prof_events;
 static std::vector<cudaEvent_t> g_prof_pool;
 static const char* kClassNames[KC_COUNT] = {"embed_ln", "layernorm", "row_softmax", "vocab_proj", "linear_qkv",
                                             "linear_fc1_gelu", "linear_out_resid", "linear_fc2_resid",
-                                            "row_logits", "row_av", "col_attn", "contact_head", "row_attn_short"};
+                                            "row_logits", "row_av", "col_attn", "contact_head", "row_attn_short",
+                                            "window_build", "window_stitch"};
 static cudaEvent_t prof_get_event() {
   if (!g_prof_pool.empty()) { cudaEvent_t e = g_prof_pool.back(); g_prof_pool.pop_back(); return e; }
   cudaEvent_t e = nullptr;
@@ -870,27 +871,33 @@ namespace rnamsm {
 
 // The layer route of the LM-head entries (scoring, sampling, the categorical Jacobian): n grids of R x C tokens, back to
 // back in tok, through the embedding and the layer stack without the final LayerNorm; x [n, T, D] receives their
-// pre-final-LayerNorm hidden states.
+// pre-final-LayerNorm hidden states.  maps (optional): grid i's row-attention maps [N, H, C, C] at maps + i * N H C C.
 //   batch (16-bit, R >= 2): the n grids together through the batch layer path; fwd holds its plan for n grids.
 //   otherwise: one msa_forward_entry per grid; fwd holds the one-MSA plan + pad flags (fwd_bytes).
 static int grids_forward_layers(const rnamsm_model_weights* m, const int64_t* tok, int n, int R, int C, int has_pad,
-                                int dtype, bool batch, float* x, uint8_t* fwd, size_t fwd_bytes, cudaStream_t st) {
+                                int dtype, bool batch, float* x, uint8_t* fwd, size_t fwd_bytes, cudaStream_t st,
+                                float* maps = nullptr) {
   const int D = m->embed_dim;
   const size_t T = (size_t)R * C;
+  const size_t map_sz = (size_t)m->num_layers * m->num_heads * C * C;
   int rc;
   if (!batch) {
     for (int i = 0; i < n; ++i)
-      if ((rc = msa_forward_entry(m, tok + i * T, R, C, has_pad, dtype, x + i * T * D, nullptr, nullptr, nullptr, nullptr,
-                                  nullptr, fwd, fwd_bytes, st, false)))
+      if ((rc = msa_forward_entry(m, tok + i * T, R, C, has_pad, dtype, x + i * T * D, maps ? maps + i * map_sz : nullptr,
+                                  nullptr, nullptr, nullptr, nullptr, fwd, fwd_bytes, st, false)))
         return rc;
     return 0;
   }
   const int dt = dtype & 0xff;
   std::vector<int> Rs(n, R), Cs(n, C);
   std::vector<uint8_t> pads(n, has_pad ? 1 : 0);
+  std::vector<float*> map_ptrs;
+  if (maps)
+    for (int i = 0; i < n; ++i) map_ptrs.push_back(maps + i * map_sz);
   BatchPlan bp;
   if ((rc = make_batch_plan(n, Rs.data(), Cs.data(), D, m->num_heads, m->ffn_dim, dt, &bp))) return rc;
-  return msa_forward_batch_layers(m, n, tok, Rs.data(), Cs.data(), pads.data(), dt, x, nullptr, fwd, bp, st);
+  return msa_forward_batch_layers(m, n, tok, Rs.data(), Cs.data(), pads.data(), dt, x, maps ? map_ptrs.data() : nullptr,
+                                  fwd, bp, st);
 }
 
 struct ScorePlan {
@@ -1269,6 +1276,134 @@ int rnamsm_msa_categorical_jacobian(const rnamsm_model_weights* m, const int64_t
       return rc;
     if ((rc = head(n, logits))) return rc;
     if ((rc = launch_jacobian_collect(logits, wt, n, C, V, d_pos, P, d_alph, A, d_slab + k0, jacobian_out, st))) return rc;
+  }
+  return 0;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// Full-length features of an alignment longer than the learned column positions, from overlapping windows
+// (rnamsm_msa_forward_windows; the window plan and the definition and arithmetic of the stitched outputs are in
+// windows.cu).  The K windows run `group` at a time; a pass of g windows:
+//   build kernel -> the pass's window grids [g, R, W + 1]
+//   layer stack on the route of the LM-head entries (grids_forward_layers), with each grid's maps
+//   row gather (R >= 2 only) -> row 0 of each grid; final LayerNorm on those g (W + 1) rows only
+//   contact head per window (contacts wanted)
+//   stitch kernel -> emb_out, atp_out (and contacts_out)
+// Every step is the one rnamsm_msa_forward runs on that grid, so each window's outputs are bit-identical to a forward of
+// its grid.  Workspace for `group` (at most K) windows, every region 256 B aligned:
+//   tok   [g, R, W + 1] int64        the pass's window grids
+//   x     [g, R, W + 1, D] fp32      their pre-final-LayerNorm hidden states
+//   fwd                              the forward's own workspace: the batch plan of g grids, or the one-MSA plan + pads
+//   maps  [g, N H, W + 1, W + 1]     their row-attention maps, BOS row and column included
+//   hx    [g, W + 1, D] fp32         row 0 of each grid, normalised in place (R >= 2; otherwise x itself)
+//   cw    [g, W, W] fp32             each window's contacts (contacts wanted)
+//   ca    [N H (W + 1)] fp32         the contact head's scratch (contacts wanted)
+//   list  int32 [K + 1]              the window starts, then 0 (the row the gather reads)
+// ---------------------------------------------------------------------------------------------
+namespace rnamsm {
+
+struct WindowPlan {
+  bool batch;
+  int W, K, group;
+  size_t fwd_bytes, off_tok, off_x, off_fwd, off_maps, off_hx, off_cw, off_ca, off_list, total;
+};
+
+static int make_window_plan(int R, int C, int D, int H, int F, int N, int dtype, int group, int window, int stride,
+                            bool want_contacts, WindowPlan* out) {
+  const bool f32_tensor = (dtype & RNAMSM_F32_TENSOR) != 0;
+  const int dt = dtype & 0xff;
+  RNAMSM_REQUIRE((dtype & ~(0xff | RNAMSM_F32_TENSOR)) == 0 && (dt == RNAMSM_F32 || (is16(dt) && !f32_tensor)),
+                 "windows: unknown dtype %d", dtype);
+  RNAMSM_REQUIRE(R >= 1 && C >= 2 && D > 0 && H > 0 && F > 0 && N > 0 && group >= 1,
+                 "windows: bad shape R=%d C=%d D=%d H=%d F=%d N=%d group=%d", R, C, D, H, F, N, group);
+  WindowPlan w{};
+  w.K = window_starts(C - 1, window, stride, nullptr);
+  if (w.K == 0) return 2;
+  w.W = std::min(window, C - 1);
+  w.group = std::min(group, w.K);
+  const int Cw = w.W + 1;
+  const size_t T = (size_t)R * Cw, g = (size_t)w.group, NH = (size_t)N * H;
+  w.batch = is16(dt) && R >= 2;
+  if (w.batch) {
+    std::vector<int> Rs(w.group, R), Cs(w.group, Cw);
+    BatchPlan bp;
+    int rc;
+    if ((rc = make_batch_plan(w.group, Rs.data(), Cs.data(), D, H, F, dt, &bp))) return rc;
+    w.fwd_bytes = bp.total;
+  } else {
+    w.fwd_bytes = make_plan(R, Cw, D, H, F, dt, f32_tensor).total + align256(T);
+  }
+  size_t o = 0;
+  w.off_tok = o;  o += align256(g * T * 8);
+  w.off_x = o;    o += align256(g * T * D * 4);
+  w.off_fwd = o;  o += align256(w.fwd_bytes);
+  w.off_maps = o; o += align256(g * NH * Cw * Cw * 4);
+  w.off_hx = o;   o += R > 1 ? align256(g * Cw * D * 4) : 0;
+  w.off_cw = o;   o += want_contacts ? align256(g * w.W * w.W * 4) : 0;
+  w.off_ca = o;   o += want_contacts ? align256(NH * Cw * 4) : 0;
+  w.off_list = o; o += align256(((size_t)w.K + 1) * 4);
+  w.total = o;
+  *out = w;
+  return 0;
+}
+
+}  // namespace rnamsm
+
+extern "C" {
+
+size_t rnamsm_windows_workspace_bytes(int R, int C, int D, int H, int F, int N, int dtype, int group, int window, int stride,
+                                      int want_contacts) {
+  WindowPlan wp;
+  if (make_window_plan(R, C, D, H, F, N, dtype, group, window, stride, want_contacts != 0, &wp)) return 0;
+  return wp.total;
+}
+
+int rnamsm_msa_forward_windows(const rnamsm_model_weights* m, const int64_t* tokens, int R, int C, int has_pad, int dtype,
+                               int window, int stride, int group, float* emb_out, float* atp_out, float* contacts_out,
+                               const float* contact_w, const float* contact_b, void* workspace, size_t workspace_bytes,
+                               void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  const int D = m->embed_dim, H = m->num_heads, F = m->ffn_dim, N = m->num_layers, NH = N * H;
+  RNAMSM_REQUIRE(D == H * 64, "forward_windows: head_dim must be 64 (D=%d H=%d)", D, H);
+  const int max_window = m->n_pos - m->pad_idx - 2;   // positions of a [R, W + 1] grid run up to W + 1 + pad_idx
+  RNAMSM_REQUIRE(window >= 1 && window <= max_window, "forward_windows: window %d outside [1, %d] (the learned positions)",
+                 window, max_window);
+  WindowPlan wp;
+  int rc;
+  if ((rc = make_window_plan(R, C, D, H, F, N, dtype, group, window, stride, contacts_out != nullptr, &wp))) return rc;
+  RNAMSM_REQUIRE(tokens && emb_out && atp_out, "forward_windows: tokens, emb_out and atp_out required");
+  RNAMSM_REQUIRE(!contacts_out || contact_w, "forward_windows: contacts need the regression weights contact_w");
+  RNAMSM_REQUIRE(workspace_bytes >= wp.total, "forward_windows: workspace %zu < required %zu", workspace_bytes, wp.total);
+  RNAMSM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "forward_windows: workspace must be 256 B aligned");
+  const int L = C - 1, W = wp.W, K = wp.K, Cw = W + 1;
+  std::vector<int> list((size_t)K + 1);
+  window_starts(L, window, stride, list.data());
+  list[K] = 0;
+  uint8_t* ws = (uint8_t*)workspace;
+  int64_t* grids = reinterpret_cast<int64_t*>(ws + wp.off_tok);
+  float* x = reinterpret_cast<float*>(ws + wp.off_x);
+  float* maps = reinterpret_cast<float*>(ws + wp.off_maps);
+  float* hx = R > 1 ? reinterpret_cast<float*>(ws + wp.off_hx) : x;
+  float* cw = contacts_out ? reinterpret_cast<float*>(ws + wp.off_cw) : nullptr;
+  float* ca = reinterpret_cast<float*>(ws + wp.off_ca);
+  int* d_starts = reinterpret_cast<int*>(ws + wp.off_list);
+  RNAMSM_CHECK_CUDA(cudaMemcpyAsync(d_starts, list.data(), list.size() * 4, cudaMemcpyHostToDevice, st));
+  for (int k0 = 0; k0 < K; k0 += wp.group) {
+    const int n = std::min(wp.group, K - k0);
+    if ((rc = launch_window_build(tokens, R, C, d_starts, k0, n, W, grids, st))) return rc;
+    if ((rc = grids_forward_layers(m, grids, n, R, Cw, has_pad, dtype, wp.batch, x, ws + wp.off_fwd, wp.fwd_bytes, st, maps)))
+      return rc;
+    if (R > 1 && (rc = launch_sample_gather_rows(x, n, R, Cw, d_starts + K, 1, D, hx, st))) return rc;
+    if ((rc = launch_layernorm(hx, m->ln_after_w, m->ln_after_b, hx, RNAMSM_F32, (long long)n * Cw, D, m->ln_eps, st)))
+      return rc;
+    for (int i = 0; contacts_out && i < n; ++i)
+      if ((rc = rnamsm_contact_head(maps + (size_t)i * NH * Cw * Cw, NH, Cw, 1, W, contact_w, contact_b,
+                                    cw + (size_t)i * W * W, ca, st)))
+        return rc;
+    if ((rc = launch_window_stitch(maps, NH, cw, hx, D, d_starts, K, k0, n, W, L, emb_out, atp_out, contacts_out, st)))
+      return rc;
   }
   return 0;
 }

@@ -14,7 +14,8 @@ long long launch_count();
 // for the live roofline figure and the per-kernel time shares.  Off by default: zero overhead.
 enum KernelClass {
   KC_EMBED_LN = 0, KC_LAYERNORM, KC_ROW_SOFTMAX, KC_VOCAB_PROJ, KC_LINEAR_QKV, KC_LINEAR_FC1, KC_LINEAR_OUT,
-  KC_LINEAR_FC2, KC_ROW_LOGITS, KC_ROW_AV, KC_COL_ATTN, KC_CONTACT, KC_ROW_SHORT, KC_COUNT
+  KC_LINEAR_FC2, KC_ROW_LOGITS, KC_ROW_AV, KC_COL_ATTN, KC_CONTACT, KC_ROW_SHORT, KC_WINDOW_BUILD,
+  KC_WINDOW_STITCH, KC_COUNT
 };
 struct ProfScope {
   int cls;
@@ -137,5 +138,14 @@ int launch_sample_draw(const float* logits, int V, float temperature, unsigned a
 // wt[positions[j], alphabet[b]] for the n grids of a pass (logits [n * C, V], wt [C, V]; J [P, A, P, A]).
 int launch_jacobian_collect(const float* logits, const float* wt, int n, int C, int V, const int* positions, int P,
                             const int* alphabet, int A, const int* slabs, float* J, cudaStream_t st);
+
+// windows.cu -- overlapping windows of a long alignment: the plan (K starts, or 0 with the reason set), the grids
+// [n, R, W + 1] of windows k0 .. k0 + n - 1, and the stitch of their outputs into emb [L, D], atp [NH, L, L] and
+// contacts [L, L] (maps [n, NH, W + 1, W + 1], cw [n, W, W] or NULL, hx [n, W + 1, D]).
+int window_starts(int L, int window, int stride, int* starts_out);
+int launch_window_build(const int64_t* tokens, int R, int C, const int* starts, int k0, int n, int W, int64_t* grids,
+                        cudaStream_t st);
+int launch_window_stitch(const float* maps, int NH, const float* cw, const float* hx, int D, const int* starts, int K,
+                         int k0, int n, int W, int L, float* emb_out, float* atp_out, float* contacts_out, cudaStream_t st);
 
 }  // namespace rnamsm

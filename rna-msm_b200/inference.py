@@ -11,6 +11,7 @@ from __future__ import annotations
 
 import argparse
 import os
+import sys
 from typing import Dict, Optional, Tuple
 
 import numpy as np
@@ -33,6 +34,17 @@ def extract_features(results: Dict[str, object], vocab: Vocab, num_layers: int) 
     end_idx = embedding.size(-2) - int(vocab.append_eos)
     emb = embedding[:, 0, start_idx:end_idx, :].squeeze(0).cpu().numpy()
     return emb, atp
+
+
+@torch.no_grad()
+def extract_features_windowed(model: MSATransformer, tokens: torch.Tensor, window: Optional[int] = None,
+                              stride: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
+    """``extract_features`` for an alignment of any length: ``MSATransformer.forward_windows`` (overlapping windows of
+    at most the learned positions, stitched with tent weights) -> ``(emb (L, D), atp (N*H, L, L))`` as numpy, the
+    ``*_emb.npy`` / ``*_atp.npy`` layout.  Pairs further apart than the windows reach are 0 in ``atp``.  For
+    ``L <= window`` this is exactly ``extract_features(model(tokens, ...))``."""
+    out = model.forward_windows(tokens.to(model.device), window=window, stride=stride)
+    return out["emb"].cpu().numpy(), out["atp"].cpu().numpy()
 
 
 @torch.no_grad()
@@ -247,16 +259,28 @@ def build_model(model_path: Optional[str], device: str = "cuda", precision: str 
 
 @torch.no_grad()
 def run_inference(model: MSATransformer, vocab: Vocab, root_path: str, MSA_path: str, rna_ids, max_seqs_per_msa=512,
-                  max_seqlen=1024, verbose=True, sample_method: str = "first") -> str:
+                  max_seqlen=1024, verbose=True, sample_method: str = "first", long_mode: str = "crop",
+                  window: Optional[int] = None, stride: Optional[int] = None) -> str:
+    """``long_mode``: what happens to an alignment longer than ``max_seqlen - 1`` columns.  ``"crop"`` (the reference's
+    behaviour) keeps its first ``max_seqlen - 1`` columns; ``"window"`` keeps every column and writes full-length
+    features from overlapping windows (``extract_features_windowed`` with ``window`` / ``stride``)."""
+    if long_mode not in ("crop", "window"):
+        raise ValueError(f"long_mode {long_mode!r}: expected 'crop' or 'window'")
+    if long_mode == "crop" and (window is not None or stride is not None):
+        raise ValueError("window and stride apply to long_mode='window' only")
     save_feat_path = os.path.join(root_path, MSA_path)
     os.makedirs(save_feat_path, exist_ok=True)
     for rna_id in sorted(rna_ids):
         msa_file = os.path.join(root_path, MSA_path, rna_id + ".a2m_msa2")
         # MSA ingest on the device (csrc/ingest.cu): cleaning, optional diversity sub-sampling, tokenisation
         from .ingest import ingest_msa
-        tokens, _ = ingest_msa(msa_file, vocab, max_seqs_per_msa, max_seqlen, sample_method, device=str(model.device))
-        results = model(tokens.unsqueeze(0), repr_layers=[model.num_layers], need_head_weights=True, want_logits=False)
-        emb, atp = extract_features(results, vocab, model.num_layers)
+        if long_mode == "window":
+            tokens, _ = ingest_msa(msa_file, vocab, max_seqs_per_msa, sys.maxsize, sample_method, device=str(model.device))
+            emb, atp = extract_features_windowed(model, tokens, window, stride)
+        else:
+            tokens, _ = ingest_msa(msa_file, vocab, max_seqs_per_msa, max_seqlen, sample_method, device=str(model.device))
+            results = model(tokens.unsqueeze(0), repr_layers=[model.num_layers], need_head_weights=True, want_logits=False)
+            emb, atp = extract_features(results, vocab, model.num_layers)
         np.save(os.path.join(save_feat_path, rna_id + "_atp.npy"), atp)
         np.save(os.path.join(save_feat_path, rna_id + "_emb.npy"), emb)
         if verbose:
@@ -266,7 +290,7 @@ def run_inference(model: MSATransformer, vocab: Vocab, root_path: str, MSA_path:
     return save_feat_path
 
 
-def main(argv=None):
+def parse_args(argv=None) -> argparse.Namespace:
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--device", default="cuda")
     ap.add_argument("--root_path", default=".")
@@ -284,7 +308,24 @@ def main(argv=None):
     ap.add_argument("--num_layers", type=int, default=10)
     ap.add_argument("--no_embed_positions_msa", action="store_true")
     ap.add_argument("--precision", default="fp16", choices=["fp16", "bf16", "bf16_pure", "tf32x3", "fp32"])
+    ap.add_argument("--long", default="crop", choices=["crop", "window"],
+                    help="alignments longer than max_seqlen - 1 columns: 'crop' keeps the first max_seqlen - 1 columns "
+                         "(the reference's behaviour); 'window' writes full-length features from overlapping windows")
+    ap.add_argument("--window", type=int, default=None,
+                    help="--long window: window width in residues (default: the learned positions, max_seqlen - 1)")
+    ap.add_argument("--stride", type=int, default=None, help="--long window: window stride (default: window // 2)")
     a = ap.parse_args(argv)
+    if a.long == "crop" and (a.window is not None or a.stride is not None):
+        ap.error("--window and --stride need --long window")
+    for name in ("window", "stride"):
+        v = getattr(a, name)
+        if v is not None and v < 1:
+            ap.error(f"--{name} must be >= 1 (got {v})")
+    return a
+
+
+def main(argv=None):
+    a = parse_args(argv)
     model, vocab = build_model(a.model_path, a.device, a.precision, a.embed_dim, a.num_attention_heads, a.num_layers,
                                not a.no_embed_positions_msa, a.max_tokens, a.max_seqlen)
     print(f"Maximum Number of MSA Seqs:{a.max_seqs_per_msa}")
@@ -292,7 +333,7 @@ def main(argv=None):
     with open(os.path.join(a.root_path, a.MSA_list)) as f:
         ids = f.read().splitlines()
     run_inference(model, vocab, a.root_path, a.MSA_path, ids, a.max_seqs_per_msa, a.max_seqlen,
-                  sample_method=a.sample_method)
+                  sample_method=a.sample_method, long_mode=a.long, window=a.window, stride=a.stride)
 
 
 if __name__ == "__main__":

@@ -329,6 +329,84 @@ class MSATransformer(nn.Module, _PrecisionMixin):
             outs.append(o)
         return outs
 
+    # -- full-length features from overlapping windows ---------------------------------------------
+    @torch.no_grad()
+    def forward_windows(self, tokens, window: Optional[int] = None, stride: Optional[int] = None,
+                        return_contacts: bool = False, token_budget: int = 262144) -> Dict[str, object]:
+        """Features of an alignment of any length, past the learned column positions (``rnamsm_msa_forward_windows``).
+
+        ``tokens``: ``[1, R, C]`` or ``[R, C]`` on the model's device, BOS at column 0, ``L = C - 1`` residues.  The
+        residues are covered by ``K`` windows of width ``W = min(window, L)`` starting at ``s_k = min(k * stride, L - W)``;
+        window ``k`` is the grid of column 0 and columns ``1 + s_k .. W + s_k`` and runs as an MSA of its own.  Its row 0
+        of the final representation and its ``N*H`` maps (BOS stripped) are blended with tent weights ``w_k(p) =
+        min(p - s_k + 1, s_k + W - p)``: a residue counts most in the windows where it sits centrally.  A pair of
+        residues that no window holds together (further apart than the windows reach) is exactly 0 in the maps and
+        contacts: this method does not see such pairs.  ``window`` defaults to ``embed_positions.max_positions - 1``
+        (1023) and ``stride`` to ``window // 2``; ``1 <= stride <= window <= max_positions - 1``.  When ``L <= window``
+        the outputs are bit-identical to ``extract_features(forward(tokens, ...))``.  The windows run
+        ``plan_score_group(R, W + 1, K, token_budget)[0]`` at a time; the result does not depend on that grouping.
+
+        Returns fp32 device tensors ``{"emb": [L, D], "atp": [N*H, L, L], "window_starts": [s_0, ...]}`` plus
+        ``"contacts": [L, L]`` with ``return_contacts``.  One host sync.  ``ValueError`` on bad arguments."""
+        _infer_only(self)
+        if self.vocab.append_eos or not self.vocab.prepend_bos:
+            raise ValueError("forward_windows needs a vocabulary that prepends BOS and appends no EOS")
+        t = tokens[0] if tokens.ndim == 3 and tokens.shape[0] == 1 else tokens
+        if t.ndim != 2:
+            raise ValueError(f"forward_windows takes one MSA, [1, R, C] or [R, C]; got shape {tuple(tokens.shape)}")
+        L.require_cuda(t, "tokens")
+        if t.device != self.device:
+            raise RuntimeError(f"tokens on {t.device} but model on {self.device}")
+        R, Cc = t.shape
+        Ls = Cc - 1
+        if Ls < 1:
+            raise ValueError(f"the alignment has no residues after the BOS column (C = {Cc})")
+        max_window = self.embed_positions.max_positions - 1
+        window = max_window if window is None else int(window)
+        stride = max(1, window // 2) if stride is None else int(stride)
+        if not 1 <= stride <= window <= max_window:
+            raise ValueError(f"need 1 <= stride <= window <= {max_window} (the learned positions); "
+                             f"got stride {stride}, window {window}")
+        if int(token_budget) < 1:
+            raise ValueError(f"token_budget {token_budget} must be >= 1")
+        K = L.lib.rnamsm_window_starts(Ls, window, stride, None)
+        if K == 0:
+            raise ValueError("rnamsm_window_starts: " + L.lib.rnamsm_last_error().decode(errors="replace"))
+        starts = (C.c_int * K)()
+        L.lib.rnamsm_window_starts(Ls, window, stride, starts)
+        W = min(window, Ls)
+        L.device_check(t.device)
+        t = t.long().contiguous()
+        has_pad = bool(t.eq(self.vocab.pad_idx).any())                     # the one host sync
+        self.check_msa_shape(R, W + 1, W + 1)                              # depth; a window grid fits the positions
+        group, _ = plan_score_group(R, W + 1, K, token_budget)
+        D, H, N = self.embed_dim, self.num_attention_heads, self.num_layers
+        dev = t.device
+        # allocated before the first launch, so a size that does not fit fails before any kernel runs
+        emb = torch.empty((Ls, D), dtype=torch.float32, device=dev)
+        atp = torch.empty((N * H, Ls, Ls), dtype=torch.float32, device=dev)
+        contacts = torch.empty((Ls, Ls), dtype=torch.float32, device=dev) if return_contacts else None
+        cw = cb = None
+        if return_contacts:
+            reg = self.contact_head.regression
+            cw = reg.weight.detach().float().reshape(-1).contiguous()
+            cb = reg.bias.detach().float().contiguous() if reg.bias is not None else None
+        with torch.cuda.device(dev):
+            m = self.c_weights(self._code)
+            fcode = self._fwd_code
+            nbytes = L.lib.rnamsm_windows_workspace_bytes(R, Cc, D, H, 4 * D, N, fcode, group, window, stride,
+                                                          int(return_contacts))
+            if nbytes == 0:
+                raise RuntimeError("rnamsm_windows_workspace_bytes: " + L.lib.rnamsm_last_error().decode(errors="replace"))
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            L.check(L.lib.rnamsm_msa_forward_windows(
+                C.byref(m), L.ptr(t), R, Cc, int(has_pad), fcode, window, stride, group, L.ptr(emb), L.ptr(atp),
+                L.ptr(contacts), L.ptr(cw), L.ptr(cb), L.ptr(ws), nbytes, L.stream_ptr()), "msa_forward_windows")
+        out: Dict[str, object] = {"emb": emb, "atp": atp, "window_starts": list(starts)}
+        if return_contacts:
+            out["contacts"] = contacts
+        return out
+
     # -- LM-head scoring ---------------------------------------------------------------------------
     def _score_grid(self, tokens, row: int):
         """[1, R, C] or [R, C] CUDA tokens -> (int64 [R, C] grid, has_pad, host pad flags of ``row``, host tokens of
