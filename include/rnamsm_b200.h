@@ -443,6 +443,30 @@ int rnamsm_msa_forward_windows(const rnamsm_model_weights* m, const int64_t* tok
                                const float* contact_w, const float* contact_b, void* workspace, size_t workspace_bytes,
                                void* stream);
 
+/* Statistics of an alignment itself, with no model (csrc/coevolution.cu; Morcos et al., PNAS 2011).  tokens: int64
+ * [N, C] as rnamsm_msa_tokenize writes them, column 0 BOS, residues 1 .. L = C - 1, N >= 1, L >= 1.  States: A G C U
+ * (vocabulary 4 .. 7) are 0 .. 3, every other token is the gap state 4 (q = 5).
+ * rnamsm_msa_seq_weights: row k is a neighbour of row n iff (double) m(n, k) >= theta * (double) L, with m the number of
+ * columns whose states are equal (gap == gap counts), 0 < theta <= 1; weights_out[n] = 1.0 / (neighbour count, itself
+ * included), float64 [N]; neff_out[0] = sum_n weights_out[n], float64.  The counts are exact integers.
+ * rnamsm_msa_dca: those weights, then mean-field DCA with pseudocount 0 < pseudocount < 1:
+ *   f_i(a) = (1 - lam) / Neff sum_n w_n [s_ni = a] + lam / q,  f_ij(a, b) = (1 - lam) / Neff sum_n w_n [s_ni = a][s_nj = b]
+ *   + lam / q^2 (i != j),  Cov[(i, a), (j, b)] = f_ij(a, b) - f_i(a) f_j(b) for a, b < 4 (f_ii(a, b) = f_i(a) d_ab),
+ *   e = -Cov^-1 (blocked float64 Cholesky factorisation and inverse), F[i, j] = Frobenius norm of the 4 x 4 block e_ij
+ *   padded with a zero gap row and column and put in the zero-sum gauge, F[i, i] = 0; contacts_out [L, L] fp32: the
+ *   APC and symmetrisation of rnamsm_jacobian_contacts applied to F.
+ * Fixed-order reductions, no atomics: bitwise reproducible.  A non-positive pivot of the factorisation leaves
+ * 1 + its index in the int32 at the start of the workspace (0 otherwise; read it after the stream has run); the
+ * contacts are then not valid.  Both entries enqueue only: no synchronisation, no allocation.  workspace:
+ * rnamsm_seq_weights_workspace_bytes(N, L) / rnamsm_dca_workspace_bytes(N, L) bytes, 256 B aligned (0 = invalid
+ * arguments); the DCA one holds two float64 matrices of side 4L rounded up to 64. */
+size_t rnamsm_seq_weights_workspace_bytes(int N, int L);
+int rnamsm_msa_seq_weights(const int64_t* tokens, int N, int C, double theta, double* weights_out, double* neff_out,
+                           void* workspace, size_t workspace_bytes, void* stream);
+size_t rnamsm_dca_workspace_bytes(int N, int L);
+int rnamsm_msa_dca(const int64_t* tokens, int N, int C, double theta, double pseudocount, double* weights_out,
+                   double* neff_out, float* contacts_out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- one deep MSA sharded over the GPUs of a box (SURVEY.md 8e; rna-msm_b200/sharded.py) -----------
  * The reference has no multi-GPU forward; these entry points implement the partition its math allows:
  * rows for the tied row attention (sum of partial logits over ranks), columns for the column attention

@@ -115,7 +115,11 @@ SIGNATURES = {
     "rnamsm_windows_workspace_bytes": (_sz, [_i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i]),
     "rnamsm_msa_forward_windows": (_i, [C.POINTER(ModelWeights), _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp,
                                         _vp, _sz, _vp]),
-    "rnamsm_rsa_pack": (_i, [_vp, _i, _i, _i, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]),
+    "rnamsm_seq_weights_workspace_bytes": (_sz, [_i, _i]),
+    "rnamsm_msa_seq_weights": (_i, [_vp, _i, _i, C.c_double, _vp, _vp, _vp, _sz, _vp]),
+    "rnamsm_dca_workspace_bytes": (_sz, [_i, _i]),
+    "rnamsm_msa_dca": (_i, [_vp, _i, _i, C.c_double, C.c_double, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "rnamsm_rsa_pack":(_i, [_vp, _i, _i, _i, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]),
 }
 
 if not os.path.exists(LIB_PATH):

@@ -114,6 +114,15 @@ int launch_jacobian_collect(const float* logits, const float* wt, int n, int C, 
   return 0;
 }
 
+int launch_apc_contacts(const double* F, int P, double* sums, float* out, cudaStream_t st) {
+  jacobian_margins_kernel<<<ceil_div(2 * P, 256), 256, 0, st>>>(F, P, sums);
+  jacobian_total_kernel<<<1, 1, 0, st>>>(sums, P);
+  jacobian_contacts_kernel<<<grid_blocks((long long)P * P), 256, 0, st>>>(F, sums, P, out);
+  count_launch(3);
+  RNAMSM_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
 // scratch: Jc [P, A, P, A] float64 | F [P, P] float64 | sums [2P + 1] float64 (every region 256 B aligned)
 static size_t align256_(size_t x) { return (x + 255) & ~(size_t)255; }
 
@@ -155,12 +164,9 @@ int rnamsm_jacobian_contacts(const float* J, int P, int A, float* contacts_out, 
   jacobian_center_kernel<double><<<grid_blocks(PA * A), 256, 0, st>>>(Jc, Jc, PA, P, A);
   jacobian_center_kernel<double><<<grid_blocks(PA * P), 256, 0, st>>>(Jc, Jc, PA * P, A, 1);
   jacobian_frobenius_kernel<<<grid_blocks((long long)P * P), 256, 0, st>>>(Jc, P, A, F);
-  jacobian_margins_kernel<<<ceil_div(2 * P, 256), 256, 0, st>>>(F, P, sums);
-  jacobian_total_kernel<<<1, 1, 0, st>>>(sums, P);
-  jacobian_contacts_kernel<<<grid_blocks((long long)P * P), 256, 0, st>>>(F, sums, P, contacts_out);
-  count_launch(8);
+  count_launch(5);
   RNAMSM_CHECK_CUDA(cudaGetLastError());
-  return 0;
+  return launch_apc_contacts(F, P, sums, contacts_out, st);
 }
 
 }  // extern "C"

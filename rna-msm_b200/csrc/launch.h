@@ -138,6 +138,9 @@ int launch_sample_draw(const float* logits, int V, float temperature, unsigned a
 // wt[positions[j], alphabet[b]] for the n grids of a pass (logits [n * C, V], wt [C, V]; J [P, A, P, A]).
 int launch_jacobian_collect(const float* logits, const float* wt, int n, int C, int V, const int* positions, int P,
                             const int* alphabet, int A, const int* slabs, float* J, cudaStream_t st);
+// contacts_out [P, P] fp32 from F [P, P] float64 with a zero diagonal: F - rowsum (x) colsum / total (0 when total == 0),
+// diagonal zeroed again, then (F + F^T) / 2; sums: 2P + 1 float64 of scratch.  Shared by the Jacobian and DCA contacts.
+int launch_apc_contacts(const double* F, int P, double* sums, float* out, cudaStream_t st);
 
 // windows.cu -- overlapping windows of a long alignment: the plan (K starts, or 0 with the reason set), the grids
 // [n, R, W + 1] of windows k0 .. k0 + n - 1, and the stitch of their outputs into emb [L, D], atp [NH, L, L] and
