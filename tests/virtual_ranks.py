@@ -14,7 +14,6 @@ the kernels:
 from __future__ import annotations
 
 import numpy as np
-import torch
 
 import softmax_cases as SC
 
@@ -65,34 +64,9 @@ def scatter_index(g: int, R: int, C: int, n: int):
 
 
 # ------------------------------------------------------------------------------------------ exact GEMM operands
-# ctx = i / 8 and W = j / 64 with integers |i|, |j| <= 8: every product is a multiple of 2^-9 of magnitude <= 1 / 8.
-# Bias and the residual x are multiples of 2^-9 with magnitude <= 4.  Every partial sum of x + ctx W^T + b, in any
-# order, is then a multiple of 2^-9 below (K / 8 + 8): for K <= 768 that is under 2^16 grid steps, far inside fp32's
-# 24-bit significand, so the tensor core's truncating fp32 adds are exact and the GEMM equals its float64 value.
-CTX_DEN, W_DEN, GRID = 8, 64, 2.0 ** -9
-AFFINE_MAX = 4.0
-
-
-def exact_sum_bound_ulps(K: int) -> int:
-    """Largest |x + sum_k ctx_k W_k + b| of the exact operands, in units of the 2^-9 grid."""
-    prod = 8 * 8                                  # |i j| / 512 <= 64 / 512 = 64 grid steps
-    return K * prod + 2 * int(AFFINE_MAX / GRID)
-
-
-def exact_gemm_operands(M: int, N: int, K: int, seed: int, device="cpu"):
-    """ctx [M, K], W [N, K], bias [N] as float32 tensors on `device` holding values exact in fp16 and bf16."""
-    rng = np.random.default_rng([seed, M, N, K])
-    ctx = torch.from_numpy(rng.integers(-8, 9, size=(M, K), dtype=np.int8)).to(device).float() / CTX_DEN
-    W = torch.from_numpy(rng.integers(-8, 9, size=(N, K), dtype=np.int8)).to(device).float() / W_DEN
-    bias = exact_affine((N,), rng, device)
-    return ctx, W, bias
-
-
-def exact_affine(shape, rng_or_seed, device="cpu") -> torch.Tensor:
-    """float32 multiples of 2^-9 with magnitude <= 4 (bias, the initial residual stream)."""
-    rng = np.random.default_rng(rng_or_seed) if not isinstance(rng_or_seed, np.random.Generator) else rng_or_seed
-    lim = int(AFFINE_MAX / GRID)
-    return torch.from_numpy(rng.integers(-lim, lim + 1, size=shape, dtype=np.int32)).to(device).float() * GRID
+# ctx = i / 8 and W = j / 64, bias and the residual stream on the 2^-9 grid: tests/gemm_exact.py.
+from gemm_exact import (AFFINE_MAX, CTX_DEN, GRID, W_DEN, exact_affine, exact_gemm_operands,  # noqa: E402,F401
+                        exact_sum_bound_ulps)
 
 
 # ------------------------------------------------------------------------------------------ softmax partials
