@@ -467,6 +467,29 @@ size_t rnamsm_dca_workspace_bytes(int N, int L);
 int rnamsm_msa_dca(const int64_t* tokens, int N, int C, double theta, double pseudocount, double* weights_out,
                    double* neff_out, float* contacts_out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Nested secondary structure from a pair map (csrc/fold.cu; DESIGN.md 4.15; tests/fold_ref.py restates it).  maps:
+ * host array of n device pointers to fp32 [L[m], L[m]] maps, of which only the upper triangle S[i, j], i < j, is read.
+ * A pair (i, j) is allowed iff j - i > min_loop (>= 0), S[i, j] > threshold (finite) and, with canonical != 0,
+ * {s_i, s_j} is AU, GC or GU in either order; seqs: host array of n device pointers to uint8 codes [L[m]], A G C U =
+ * 0 1 2 3, any other code never pairs (may be NULL without canonical).
+ *   RNAMSM_FOLD_MEA (maximum expected accuracy, S pair probabilities): w[i, j] = fp32(2 gamma) * S[i, j],
+ *     u[i] = fp32(1 - sum_{j != i} S[min(i, j), max(i, j)]) summed in float64 over ascending j;  gamma > 0.
+ *   RNAMSM_FOLD_SCORE (maximum-weight nested matching of any score): w[i, j] = S[i, j], u[i] = 0;  gamma ignored.
+ *   P[i][k] = w[i, k] + M[i+1][k-1] for an allowed pair, else -inf;  M[i][j] = max(M[i+1][j] + u[i],
+ *   max_{i < k <= j} P[i][k] + M[k+1][j]), fp32, M of an empty interval 0.  Traceback from (0, L - 1): i unpaired if
+ *   M[i][j] == M[i+1][j] + u[i], else paired with the smallest k matching.  pairs_out[m]: int32 [L[m]] device, partner
+ *   or -1;  scores_out: fp32 [n] device, M[0][L - 1].
+ * The result is bit-identical whatever the batch.  The int32 at the start of the workspace gets bit 1 for a non-finite
+ * S[i, j] (i < j) and bit 2 for a w or u that overflows fp32 (0 otherwise; read it after the stream has run); the
+ * outputs are then not valid.  Launches: 1 + ceil(L_max / T) + 1, T = 32 for L_max <= 1024, else 64.  Enqueues only: no
+ * synchronisation, no allocation.  workspace: rnamsm_fold_workspace_bytes(n, L) bytes (0 = invalid arguments),
+ * 256 B aligned, dominated by two fp32 tables of about L x L per map. */
+enum { RNAMSM_FOLD_MEA = 0, RNAMSM_FOLD_SCORE = 1 };
+size_t rnamsm_fold_workspace_bytes(int n, const int* L);
+int rnamsm_fold(int n, const float* const* maps, const int* L, const uint8_t* const* seqs, int mode, double gamma,
+                float threshold, int min_loop, int canonical, int* const* pairs_out, float* scores_out,
+                void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- one deep MSA sharded over the GPUs of a box (SURVEY.md 8e; rna-msm_b200/sharded.py) -----------
  * The reference has no multi-GPU forward; these entry points implement the partition its math allows:
  * rows for the tied row attention (sum of partial logits over ranks), columns for the column attention

@@ -16,10 +16,12 @@ from .inference import (extract_features, extract_features_batch, extract_featur
                         plan_batches, run_inference)
 from .ingest import ingest_msa  # noqa: F401
 from .coevolution import dca_contacts, sequence_weights  # noqa: F401
+from .structure import dot_bracket, fold_pairs, write_bpseq, write_ct  # noqa: F401
 
 __all__ = ["MSATransformer", "AxialTransformerLayer", "RowSelfAttention", "ColumnSelfAttention",
            "FeedForwardNetwork", "NormalizedResidualBlock", "LearnedPositionalEmbedding", "RobertaLMHead",
            "ContactPredictionHead", "Alphabet", "Vocab", "read_msa", "tokenize_msa", "extract_features",
            "run_inference", "ingest_msa", "pack_ss_input", "extract_features_streamed", "extract_features_batch",
            "extract_features_batch_streamed", "pack_rsa_input", "plan_batches", "plan_score_group", "parse_mutant",
-           "jacobian_entries", "extract_features_windowed", "sequence_weights", "dca_contacts"]
+           "jacobian_entries", "extract_features_windowed", "sequence_weights", "dca_contacts", "fold_pairs", "dot_bracket",
+           "write_ct", "write_bpseq"]

@@ -119,6 +119,9 @@ SIGNATURES = {
     "rnamsm_msa_seq_weights": (_i, [_vp, _i, _i, C.c_double, _vp, _vp, _vp, _sz, _vp]),
     "rnamsm_dca_workspace_bytes": (_sz, [_i, _i]),
     "rnamsm_msa_dca": (_i, [_vp, _i, _i, C.c_double, C.c_double, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "rnamsm_fold_workspace_bytes": (_sz, [_i, C.POINTER(_i)]),
+    "rnamsm_fold": (_i, [_i, C.POINTER(_vp), C.POINTER(_i), C.POINTER(_vp), _i, C.c_double, _f, _i, _i, C.POINTER(_vp),
+                         _vp, _vp, _sz, _vp]),
     "rnamsm_rsa_pack":(_i, [_vp, _i, _i, _i, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double), _vp, _vp, _vp, _vp]),
 }
 

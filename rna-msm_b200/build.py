@@ -17,7 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "librnamsm_b200.so")
-SOURCES = ["api.cu", "elementwise.cu", "simt_f32.cu", "umma_gemm.cu", "col_attn_umma.cu", "col_attn_fa.cu", "col_attn_probs.cu", "row_attn_short.cu", "peer.cu", "contact.cu", "ingest.cu", "score.cu", "sample.cu", "jacobian.cu", "windows.cu", "coevolution.cu"]
+SOURCES = ["api.cu", "elementwise.cu", "simt_f32.cu", "umma_gemm.cu", "col_attn_umma.cu", "col_attn_fa.cu", "col_attn_probs.cu", "row_attn_short.cu", "peer.cu", "contact.cu", "ingest.cu", "score.cu", "sample.cu", "jacobian.cu", "windows.cu", "coevolution.cu", "fold.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
