@@ -205,7 +205,8 @@ static int block_dtype(int requested, int dtype) {
 }
 
 // RNAMSM_FUSE_LN=1 routes every LayerNorm behind a residual GEMM through that GEMM's fused epilogue (umma_gemm.cu, kLN).
-// OFF by default: the fused kernel is exact (bit-identical rows, tests/test_gpu_ops.py) but SLOWER on a B200 -- measured
+// OFF by default: the fused kernel is exact (bit-identical rows, tests/test_gpu_ops.py; bit-identical whole forwards,
+// tests/test_gpu_forward_routes.py) but SLOWER on a B200 -- measured
 // at 131072 x 768: residual GEMM 176 us + LayerNorm 94 us = 270 us un-fused vs 804 us fused (K = 768), 598 vs 935 us
 // (K = 3072); the handshake itself is free (178 us with the row work skipped).  The 4 LayerNorm warps of a CTA keep only
 // 8 rows (24 KiB) in flight while the GEMM's own TMA traffic holds HBM at 85 % of its peak, so each dependent
