@@ -17,6 +17,28 @@
 
 namespace rnamsm {
 
+// Bio.SeqIO's FASTA parser (what MSA.from_fasta iterates) reads the file in text mode, so '\r\n' and a lone '\r' end a
+// line like '\n'.  It rstrip()s every line, joins them and removes ' ' and '\r' (SimpleFastaParser).  So a space and a
+// line end are always dropped, while the other blanks str.isspace() knows ('\t', '\v', '\f', 0x1c-0x1f) are dropped
+// only where nothing but blanks follows them up to the end of their line: a tab inside a line is kept.
+__device__ __forceinline__ bool is_soft_blank(uint8_t c) { return c == '\t' || c == '\v' || c == '\f' || (c >= 0x1c && c <= 0x1f); }
+__device__ __forceinline__ bool is_line_end(uint8_t c) { return c == '\n' || c == '\r'; }
+
+// append the soft blanks of raw[from, to) (all blanks, spaces among them) to the row: a run whose line went on
+__device__ int append_blank_run(const uint8_t* __restrict__ raw, long long from, long long to, uint8_t* __restrict__ row,
+                                int L, int written, int lane) {
+  for (long long p = from; p < to; p += 32) {
+    const long long q = p + lane;
+    const uint8_t ch = q < to ? raw[q] : (uint8_t)' ';
+    const bool keep = ch != ' ';
+    const unsigned m = __ballot_sync(0xffffffffu, keep);
+    const int pos = written + __popc(m & ((1u << lane) - 1u));
+    if (keep && pos < L) row[pos] = ch;
+    written += __popc(m);
+  }
+  return written;
+}
+
 // raw: concatenated record bodies; off[n] .. off[n+1]: bytes of record n.  out [N, L]; bad[0] != 0 if a
 // cleaned row is not exactly L long.
 __global__ void __launch_bounds__(256)
@@ -26,20 +48,35 @@ msa_clean_kernel(const uint8_t* __restrict__ raw, const long long* __restrict__ 
   const int n = blockIdx.x * 8 + warp;
   if (n >= N) return;
   const long long b = off[n], e = off[n + 1];
+  uint8_t* row = out + (size_t)n * L;
   int written = 0;
+  long long run = -1;          // start of a trailing blank run of earlier steps, kept only if text follows it
   for (long long p = b; p < e; p += 32) {
     const long long q = p + lane;
-    uint8_t ch = q < e ? raw[q] : (uint8_t)'.';
-    // Bio.SeqIO's FASTA parser (what MSA.from_fasta iterates) joins the record's lines and removes spaces, line
-    // ends and trailing blanks before from_fasta's own rules see the sequence
-    const bool keep = !((ch >= 'a' && ch <= 'z') || ch == '.' || ch == '*' || ch == '\n' || ch == '\r' || ch == ' ' ||
-                        ch == '\t');
+    uint8_t ch = q < e ? raw[q] : (uint8_t)'\n';             // the body ends where its last line ends
+    const bool soft = is_soft_blank(ch), solid = !soft && ch != ' ';
+    const unsigned solid_m = __ballot_sync(0xffffffffu, solid);
+    const unsigned text_m = __ballot_sync(0xffffffffu, solid && !is_line_end(ch));
+    if (run >= 0 && solid_m) {                               // the first solid byte decides the pending run
+      if ((text_m >> (__ffs(solid_m) - 1)) & 1u) written = append_blank_run(raw, run, p, row, L, written, lane);
+      run = -1;
+    }
+    // a soft blank is kept if the next solid byte of this step is text; none: the run stays pending
+    const unsigned later = lane == 31 ? 0u : solid_m & (0xffffffffu << (lane + 1));
+    const bool soft_kept = soft && later && ((text_m >> (__ffs(later) - 1)) & 1u);
+    if (solid_m == 0u) {
+      if (run < 0) run = p;
+    } else if (solid_m >> 31 == 0u) {
+      run = p + 32 - __clz(solid_m);
+    }
+    // then MSA.from_fasta's own rules: drop lowercase, '.', '*'; T -> U; IUPAC -> X
+    const bool keep = soft_kept || (solid && !is_line_end(ch) && !((ch >= 'a' && ch <= 'z') || ch == '.' || ch == '*'));
     if (ch == 'T') ch = 'U';
     else if (ch == 'R' || ch == 'Y' || ch == 'K' || ch == 'M' || ch == 'S' || ch == 'W' || ch == 'B' || ch == 'D' ||
              ch == 'H' || ch == 'V' || ch == 'N') ch = 'X';
     const unsigned m = __ballot_sync(0xffffffffu, keep);
     const int pos = written + __popc(m & ((1u << lane) - 1u));
-    if (keep && pos < L) out[(size_t)n * L + pos] = ch;
+    if (keep && pos < L) row[pos] = ch;
     written += __popc(m);
   }
   if (lane == 0 && written != L) atomicExch(bad, n + 1);
@@ -221,7 +258,8 @@ int rnamsm_msa_greedy_select(const uint8_t* chars, int N, int L, int num, int wa
   const int blocks_h = std::min(ceil_div(N, 8), 148 * 4);
   const int blocks_m = std::min(ceil_div(N, 256), 148 * 4);
   const size_t lut_bytes = (size_t)(L + 1) * sizeof(double);
-  if (lut_bytes > 48 * 1024)
+  // the LUT shares the 48 KiB default with greedy_mean_kernel's static sb[8]: 6128 <= L <= 6143 needs the opt-in too
+  if (lut_bytes + 8 * sizeof(Best) > 48 * 1024)
     RNAMSM_CHECK_CUDA(cudaFuncSetAttribute(greedy_mean_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lut_bytes));
   RNAMSM_CHECK_CUDA(cudaMemsetAsync(is_sel, 0, (size_t)N, st));
   const int zero = 0;

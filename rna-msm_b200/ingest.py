@@ -13,6 +13,7 @@ hhfilter returns beyond the limit, utils/align.py:172-173; the hhfilter binary i
 from __future__ import annotations
 
 import ctypes as C
+import re
 from typing import List, Tuple
 
 import numpy as np
@@ -28,9 +29,12 @@ def split_records(path: str) -> Tuple[List[str], bytes, np.ndarray]:
     bodies: List[bytes] = []
     with open(path, "rb") as f:
         data = f.read()
-    # a record starts at a '>' in the FIRST column of a line (Bio.SeqIO); a '>' inside a header ("a->b") is text
+    # a record starts at a '>' in the FIRST column of a line (Bio.SeqIO); a '>' inside a header ("a->b") is text.
+    # SeqIO reads in text mode, where a lone '\r' ends a line too
+    if b"\r>" in data:
+        data = data.replace(b"\r>", b"\n>")
     for rec in (b"\n" + data).split(b"\n>")[1:]:            # anything before the first record is ignored
-        nl = rec.find(b"\n")
+        nl = min((i for i in (rec.find(b"\n"), rec.find(b"\r")) if i >= 0), default=-1)
         headers.append(rec[:nl if nl >= 0 else len(rec)].decode(errors="replace").strip())
         bodies.append(rec[nl + 1:] if nl >= 0 else b"")
     offsets = np.zeros(len(bodies) + 1, dtype=np.int64)
@@ -38,9 +42,16 @@ def split_records(path: str) -> Tuple[List[str], bytes, np.ndarray]:
     return headers, b"".join(bodies), offsets
 
 
+# blanks at the end of a line: SeqIO rstrip()s every line (str.isspace() over ASCII), so these go; inside a line only
+# the spaces go (csrc/ingest.cu msa_clean_kernel)
+_TRAILING_BLANKS = re.compile(rb"[\t\x0b\x0c\x1c-\x1f ]+(?=[\r\n]|\Z)")
+
+
 def cleaned_length(body: bytes) -> int:
-    """Length of one record after the from_fasta rules (host: the first record only, to size the matrix)."""
-    return sum(1 for ch in body if not (97 <= ch <= 122 or ch in b".*\n\r \t"))
+    """Length of one record after SeqIO's line handling and the from_fasta rules (host: the first record only, to
+    size the matrix)."""
+    body = _TRAILING_BLANKS.sub(b"", body)
+    return sum(1 for ch in body if not (97 <= ch <= 122 or ch in b".*\n\r "))
 
 
 @torch.no_grad()
